@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the spectral encoding front end (BASELINE.json metric: scans/s encoded to 800-D).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the fused encode kernel over this rank's batch of synthetic scans
 (BASELINE.json configs[1]: 4541 HDL-64-shaped scans of ~120 k xyzi points, 8.7 GB, resident in
@@ -25,6 +25,11 @@ Prints ONE JSON line (rank 0):
                 git-ignored copy made by oracle/make_ref.py is present, else the oracle port)
 
 ``--impl reference`` times that same CPU encoder as the reference arm, honouring --steps/--warmup.
+
+``--dump-outputs DIR`` writes, after the timed steps, what the timed path returned in its last step
+as ``DIR/<name>.npy`` (float32 / float64; integer outputs converted exactly), so that two builds can
+be compared output for output: the inputs depend on the arguments only (seeded). Outputs above
+64 MB in all are cut to a fixed, seeded sample of rows, listed in ``DIR/rows.npy``.
 
 Secondary lines (not the BASELINE.json metric, same JSON shape): ``--workload retrieval`` (stage-1
 Wasserstein top-K over a 100 k x 800 database), ``--workload keyframe`` (voxel IoU of the keyframe
@@ -477,6 +482,9 @@ def run_gpu_arm(args):
     end.record(stream)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # one GPU: this batch's descriptors; N > 1: the gathered database, the same on every rank
+        dump_outputs(args.dump_outputs, {"descriptors": out if sharded is None else sharded.flush()})
     total_ms = ev[0].elapsed_time(end)
     step_ms = [ev[2 * k].elapsed_time(ev[2 * k + 1]) for k in range(args.steps)]
     if world > 1:
@@ -722,9 +730,11 @@ def run_retrieval(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        r.query_batch(q, top_k=k)
+        res = r.query_batch(q, top_k=k)
     e1.record()
     torch.cuda.synchronize()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("indices", "distances", "counts"), res)))
     ms = e0.elapsed_time(e1) / args.steps
     passes = -(-nq // 8)                                   # one pass over the CDF rows serves 8 queries
     alg_bytes = passes * n_db * 800 * 4
@@ -809,6 +819,8 @@ def run_keyframe(args):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"overlap": out, "voxel_counts": cnt})
     assert np.array_equal(out.cpu().numpy(), iou)
     peak, _ = hbm_peak()
     line = {"metric": "keyframe_overlap_pairs_per_sec", "value": n_pairs / (ms * 1e-3), "unit": "pairs/s", "n_gpus": 1,
@@ -869,6 +881,8 @@ def run_quantize(args):
     e3.record()
     torch.cuda.synchronize()
     ms_q, ms_d = e0.elapsed_time(e1) / args.steps, e2.elapsed_time(e3) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"quantized": q, "dequantized": d})
     peak, _ = hbm_peak()
     bytes_q = n * 800 * (4 + 2)
     line = {"metric": "descriptors_quantised_per_sec", "value": n / (ms_q * 1e-3), "unit": "descriptors/s", "n_gpus": 1,
@@ -893,6 +907,34 @@ def run_quantize(args):
                                           "is hard-wired to 50 bins)"}
         line["checks"]["equal_to_cpu"] = bool(np.array_equal(want, q[:2000].cpu().numpy()))
     emit(line)
+
+
+DUMP_BYTES = 64_000_000 - (64 << 10)     # 64 MB in all, less room for the .npy headers
+
+
+def dump_outputs(dump_dir, arrays):
+    """``arrays``: name -> torch tensor or numpy array, all with the same number of rows. Writes
+    ``dump_dir/<name>.npy``; floating arrays keep their type, integer ones become float32 (up to
+    16 bits) or float64, both exact. Above DUMP_BYTES in all, every array keeps the same seeded
+    sample of rows, in order, and ``rows.npy`` lists them."""
+    import numpy as np
+    import torch
+    arrays = {name: a if torch.is_tensor(a) else torch.from_numpy(np.asarray(a)) for name, a in arrays.items()}
+    out_type = {name: torch.float64 if a.element_size() > (4 if a.is_floating_point() else 2) else torch.float32
+                for name, a in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.numel() * out_type[name].itemsize for name, a in arrays.items()) / max(n, 1)
+    rows = None
+    if n * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, int(DUMP_BYTES // (row_bytes + 8)), replace=False))
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().to(out_type[name])           # where the array lives; only the kept rows reach the host
+        if rows is not None:
+            a = a[torch.from_numpy(rows).to(a.device)]
+        np.save(os.path.join(dump_dir, name + ".npy"), a.cpu().numpy())
+    if rows is not None:
+        np.save(os.path.join(dump_dir, "rows.npy"), rows.astype(np.float64))
 
 
 def emit(line: dict) -> None:
@@ -935,7 +977,13 @@ def main():
     ap.add_argument("--db", type=int, default=100000, help="retrieval: database rows")
     ap.add_argument("--queries", type=int, default=8, help="retrieval: queries per call")
     ap.add_argument("--topk", type=int, default=10, help="retrieval: K")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path returned in its last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the GPU path (--impl b200)")
     if args.impl == "reference":
         run_reference_arm(args)
         return

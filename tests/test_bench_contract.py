@@ -4,6 +4,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 from conftest import ROOT
 
 
@@ -44,3 +47,53 @@ def test_both_arms_describe_the_same_config():
     d = json.loads(r.stdout.strip().splitlines()[-1])
     a = argparse.Namespace(scans=bench.N_SCANS, shape="hdl64", shuffle=False, gather="fused", gather_lag=0, gpus=8)
     assert d["config"] == bench.make_config(a, 8) and d["n_gpus"] == 8
+
+
+def test_steps_below_one_are_refused():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr and r.stdout == ""
+
+
+def test_dump_outputs_converts_exactly_and_samples_rows_above_64_mb(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    bench.dump_outputs(str(tmp_path / "small"), {"q": np.arange(12, dtype=np.uint16).reshape(6, 2),
+                                                  "i": np.arange(6, dtype=np.int64) + 2 ** 40,
+                                                  "f": np.linspace(0, 1, 6)})
+    q, i, f = (np.load(tmp_path / "small" / f"{k}.npy") for k in ("q", "i", "f"))
+    assert q.dtype == np.float32 and q.tolist() == np.arange(12).reshape(6, 2).tolist()
+    assert i.dtype == np.float64 and i.tolist() == [2 ** 40 + k for k in range(6)]
+    assert f.dtype == np.float64 and not os.path.exists(tmp_path / "small" / "rows.npy")
+
+    n = 22000                                        # 22000 x 800 float32 = 70 MB
+    big = {"d": np.repeat(np.arange(n, dtype=np.float32)[:, None], 800, 1), "label": np.arange(n, dtype=np.int32)}
+    bench.dump_outputs(str(tmp_path / "big"), big)
+    bench.dump_outputs(str(tmp_path / "again"), big)
+    rows = np.load(tmp_path / "big" / "rows.npy")
+    np.testing.assert_array_equal(np.load(tmp_path / "again" / "rows.npy"), rows)     # the same sample every time
+    d, label = np.load(tmp_path / "big" / "d.npy"), np.load(tmp_path / "big" / "label.npy")
+    assert sum(os.path.getsize(tmp_path / "big" / f) for f in os.listdir(tmp_path / "big")) <= 64_000_000
+    assert len(rows) > n // 2 and np.all(np.diff(rows) > 0)
+    np.testing.assert_array_equal(d, big["d"][rows.astype(np.int64)])
+    np.testing.assert_array_equal(label, rows)
+
+
+@pytest.mark.gpu
+def test_dumped_descriptors_are_the_timed_output_for_the_seeded_scans(tmp_path):
+    from neural_spectral_codec_b200 import SpectralEncoder, synth
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "0",
+                        "--scans", "40", "--no-cpu", "--no-extras", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads(r.stdout.strip().splitlines()[-1])
+    assert d["steps"] == 2 and d["gpu_launches"] == 2 and d["checks"]["ok"]
+    assert os.listdir(tmp_path) == ["descriptors.npy"]
+    got = np.load(tmp_path / "descriptors.npy")
+    # plumbing only (the dump is the last timed step for the seeded scans): parity with the oracle is checks.ok
+    enc = SpectralEncoder(n_elevation=16, n_azimuth=360, n_bins=50, alpha=2.0, learnable_alpha=True,
+                          target_elevation_bins=16).to("cuda")
+    pts, offs = synth.make_batch(synth.HDL64, 0, 40, device="cuda")
+    want = enc.encode_points_batch(pts, offs).cpu().numpy()
+    assert got.dtype == np.float32 and got.shape == (40, 800)
+    np.testing.assert_array_equal(got, want)
