@@ -118,6 +118,19 @@ int nsc_encode_batch(const float* d_points, int point_stride, const int64_t* d_o
                      const int32_t* h_lut, float* d_out, void* d_workspace,
                      size_t workspace_bytes, void* stream);
 
+/* nsc_encode_batch straight to the descriptor wire format: each row is normalised as above and
+ * quantised in the same kernel's epilogue exactly as nsc_quantize_histograms (below) would quantise
+ * the float32 row nsc_encode_batch writes -- the same integers for every row, empty scans included --
+ * without the float32 round trip through device memory.
+ *   q_epsilon  the quantiser's epsilon (HistogramQuantizer default 1e-8; independent of p->epsilon)
+ *   d_out      uint16[n_scans * target_rows * n_bins], each row summing to 65535 (a row whose
+ *              rounded total is 0 stays all zero, as in the reference)
+ * Arguments are validated in the order of nsc_encode_batch, with the same status codes. */
+int nsc_encode_batch_u16(const float* d_points, int point_stride, const int64_t* d_offsets,
+                         int64_t point_origin, int n_scans, const nsc_params* p,
+                         const int32_t* h_lut, float q_epsilon, uint16_t* d_out, void* d_workspace,
+                         size_t workspace_bytes, void* stream);
+
 /* nsc_encode_batch fused with the all-gather that follows it in a multi-GPU encode
  * (SURVEY.md 8(e): the replicated descriptor database that
  * WassersteinRetriever.add_to_database, reference src/retrieval/wasserstein.py:300-326, would
@@ -221,6 +234,11 @@ void nsc_pipeline_destroy(nsc_pipeline* pl);
 int nsc_pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_stride,
                         int64_t n_points, const int64_t* h_offsets, int n_scans,
                         const nsc_params* p, const int32_t* h_lut, float* h_out);
+/* The same with the wire format of nsc_encode_batch_u16 in h_out (uint16[n_scans * target_rows *
+ * n_bins]): the rows a keyframe store keeps, in one call; 2 bytes per element cross PCIe instead of 4. */
+int nsc_pipeline_encode_u16(nsc_pipeline* pl, const float* h_points, int point_stride,
+                            int64_t n_points, const int64_t* h_offsets, int n_scans,
+                            const nsc_params* p, const int32_t* h_lut, float q_epsilon, uint16_t* h_out);
 
 /* ONE scan from pageable host memory to a descriptor on the DEVICE, on the caller's stream -- the
  * reference's own call shape: encoder.encode_points(numpy_scan) per scan (pipeline.py:245,
@@ -240,6 +258,10 @@ int nsc_pipeline_encode_scan(nsc_pipeline* pl, const float* h_points, int point_
 int nsc_pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, const int64_t* h_counts,
                               int point_stride, int n_scans, const nsc_params* p,
                               const int32_t* h_lut, float* h_out);
+/* ... and with uint16 rows of nsc_encode_batch_u16 in h_out (uint16[n_scans * target_rows * n_bins]). */
+int nsc_pipeline_encode_scans_u16(nsc_pipeline* pl, const float* const* h_scans, const int64_t* h_counts,
+                                  int point_stride, int n_scans, const nsc_params* p,
+                                  const int32_t* h_lut, float q_epsilon, uint16_t* h_out);
 
 /* ---- keyframe gate geometry (SURVEY.md 8(f), third "next" row) ------------------------------ */
 /* Voxel-set IoU of n_pairs cloud pairs in one launch: the geometric-novelty criterion of the

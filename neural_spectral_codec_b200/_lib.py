@@ -24,6 +24,7 @@ MAX_DESCRIPTOR = 4096
 MAX_PEERS = 8
 STAGE_PROJECTED = 0
 STAGE_INTERPOLATED = 1
+QUANT_EPSILON = 1e-8     # the reference HistogramQuantizer's default epsilon (the uint16 encode paths)
 
 
 class NscParams(C.Structure):
@@ -65,6 +66,7 @@ SYMBOLS = {
     "nsc_freq_to_bin": (_I, [C.c_float, _PP, _VP]),
     "nsc_workspace_bytes": (_SZ, [_I, _PP]),
     "nsc_encode_batch": (_I, [_VP, _I, _VP, _I64, _I, _PP, _VP, _VP, _VP, _SZ, _VP]),
+    "nsc_encode_batch_u16": (_I, [_VP, _I, _VP, _I64, _I, _PP, _VP, C.c_float, _VP, _VP, _SZ, _VP]),
     "nsc_encode_batch_peers": (_I, [_VP, _I, _VP, _I64, _I, _PP, _VP, _VP, _I, _I64, _VP, _SZ, _VP]),
     "nsc_peer_signal_wait": (_I, [_VP, _I, _I, C.c_uint32, C.c_uint32, _VP]),
     "nsc_project_batch": (_I, [_VP, _I, _VP, _I64, _I, _PP, _I, _VP, _VP, _SZ, _VP]),
@@ -77,8 +79,10 @@ SYMBOLS = {
     "nsc_pipeline_create": (_I, [_I64, _I, _I, C.POINTER(_VP)]),
     "nsc_pipeline_destroy": (None, [_VP]),
     "nsc_pipeline_encode": (_I, [_VP, _VP, _I, _I64, _VP, _I, _PP, _VP, _VP]),
+    "nsc_pipeline_encode_u16": (_I, [_VP, _VP, _I, _I64, _VP, _I, _PP, _VP, C.c_float, _VP]),
     "nsc_pipeline_encode_scan": (_I, [_VP, _VP, _I, _I64, _PP, _VP, _VP, _VP]),
     "nsc_pipeline_encode_scans": (_I, [_VP, _VP, _VP, _I, _I, _PP, _VP, _VP]),
+    "nsc_pipeline_encode_scans_u16": (_I, [_VP, _VP, _VP, _I, _I, _PP, _VP, C.c_float, _VP]),
     "nsc_voxel_overlap_workspace_bytes": (_SZ, [_I64, _I64, _I]),
     "nsc_voxel_overlap_batch": (_I, [_VP, _I, _I, _VP, _I64, _I64, _VP, _I, C.c_double, _VP, _VP, _VP, _SZ, _VP]),
     "nsc_wasserstein_cdf": (_I, [_VP, _I64, _I, C.c_float, _VP, _VP]),

@@ -41,20 +41,42 @@ size_t nsc_workspace_bytes(int n_scans, const nsc_params* p) {
     return workspace_bytes_for(n_scans, p->n_elevation);
 }
 
-int nsc_encode_batch(const float* d_points, int point_stride, const int64_t* d_offsets,
-                     int64_t point_origin, int n_scans, const nsc_params* p, const int32_t* h_lut,
-                     float* d_out, void* d_workspace, size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+namespace {
+// nsc_encode_batch (d_out_q null) and nsc_encode_batch_u16 (d_out null): one validation order
+int encode_batch(const float* d_points, int point_stride, const int64_t* d_offsets, int64_t point_origin,
+                 int n_scans, const nsc_params* p, const int32_t* h_lut, float* d_out, uint16_t* d_out_q,
+                 float q_epsilon, void* d_workspace, size_t workspace_bytes, void* stream) {
     DeviceParams dp;
     int st = make_device_params(p, h_lut, &dp);
     if (st != NSC_OK) return st;
     st = check_points(d_points, point_stride, d_offsets, n_scans);
     if (st != NSC_OK) return st;
     if (n_scans == 0) return NSC_OK;
-    if (!d_out) return NSC_ERR_NULL_POINTER;
+    if (!d_out && !d_out_q) return NSC_ERR_NULL_POINTER;
     if (!d_workspace || workspace_bytes < workspace_bytes_min()) return NSC_ERR_WORKSPACE;
     return launch_encode(d_points, point_stride, (const long long*)d_offsets, point_origin, n_scans,
                          dp, d_out, nullptr, 0, nullptr, 0, 0, (unsigned*)d_workspace, workspace_bytes,
-                         (cudaStream_t)stream);
+                         (cudaStream_t)stream, d_out_q, q_epsilon);
+}
+}  // namespace
+
+extern "C" {
+
+int nsc_encode_batch(const float* d_points, int point_stride, const int64_t* d_offsets,
+                     int64_t point_origin, int n_scans, const nsc_params* p, const int32_t* h_lut,
+                     float* d_out, void* d_workspace, size_t workspace_bytes, void* stream) {
+    return encode_batch(d_points, point_stride, d_offsets, point_origin, n_scans, p, h_lut, d_out, nullptr, 0.0f,
+                        d_workspace, workspace_bytes, stream);
+}
+
+int nsc_encode_batch_u16(const float* d_points, int point_stride, const int64_t* d_offsets,
+                         int64_t point_origin, int n_scans, const nsc_params* p, const int32_t* h_lut,
+                         float q_epsilon, uint16_t* d_out, void* d_workspace, size_t workspace_bytes,
+                         void* stream) {
+    return encode_batch(d_points, point_stride, d_offsets, point_origin, n_scans, p, h_lut, nullptr, d_out,
+                        q_epsilon, d_workspace, workspace_bytes, stream);
 }
 
 int nsc_encode_batch_peers(const float* d_points, int point_stride, const int64_t* d_offsets,
@@ -332,9 +354,21 @@ int nsc_pipeline_create(int64_t max_chunk_points, int n_buffers, int device, nsc
     return NSC_OK;
 }
 
-int nsc_pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_stride,
-                        int64_t n_points, const int64_t* h_offsets, int n_scans,
-                        const nsc_params* p, const int32_t* h_lut, float* h_out) {
+}  // extern "C"
+
+// Encodes a staged chunk into the slot's device descriptors: float32 (out_bytes 4), or uint16
+// (out_bytes 2) in the first half of the same buffer.
+static int launch_slot(nsc_pipeline::Slot& s, int stride, long long origin, int ns, const DeviceParams& dp,
+                       size_t out_bytes, float q_eps) {
+    return launch_encode(s.d_points, stride, s.d_offsets, origin, ns, dp, out_bytes == 4 ? s.d_out : nullptr, nullptr,
+                         0, nullptr, 0, 0, s.d_ws, 256, s.stream,
+                         out_bytes == 2 ? reinterpret_cast<unsigned short*>(s.d_out) : nullptr, q_eps);
+}
+
+// nsc_pipeline_encode / nsc_pipeline_encode_u16: descriptors of out_bytes (4 or 2) per element.
+static int pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_stride, int64_t n_points,
+                           const int64_t* h_offsets, int n_scans, const nsc_params* p, const int32_t* h_lut,
+                           void* h_out, size_t out_bytes, float q_eps) {
     if (!pl) return NSC_ERR_NULL_POINTER;
     DeviceParams dp;
     int st = make_device_params(p, h_lut, &dp);
@@ -377,10 +411,9 @@ int nsc_pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_strid
             st = record_cuda(e);
             break;
         }
-        st = launch_encode(s.d_points, point_stride, s.d_offsets, p0, ns, dp, s.d_out, nullptr, 0,
-                           nullptr, 0, 0, s.d_ws, 256, s.stream);
+        st = launch_slot(s, point_stride, p0, ns, dp, out_bytes, q_eps);
         if (st != NSC_OK) break;
-        if ((e = cudaMemcpyAsync(h_out + (size_t)first * D, s.d_out, (size_t)ns * D * 4,
+        if ((e = cudaMemcpyAsync((char*)h_out + (size_t)first * D * out_bytes, s.d_out, (size_t)ns * D * out_bytes,
                                  cudaMemcpyDeviceToHost, s.stream)) != cudaSuccess ||
             (e = cudaEventRecord(s.done, s.stream)) != cudaSuccess) {
             st = record_cuda(e);
@@ -429,9 +462,10 @@ static void stage_scans(float* dst, const float* const* h_scans, const int64_t* 
     for (auto& th : pool) th.join();
 }
 
-int nsc_pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, const int64_t* h_counts,
-                              int point_stride, int n_scans, const nsc_params* p,
-                              const int32_t* h_lut, float* h_out) {
+// nsc_pipeline_encode_scans / nsc_pipeline_encode_scans_u16: descriptors of out_bytes (4 or 2) per element.
+static int pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, const int64_t* h_counts,
+                                 int point_stride, int n_scans, const nsc_params* p, const int32_t* h_lut,
+                                 void* h_out, size_t out_bytes, float q_eps) {
     if (!pl) return NSC_ERR_NULL_POINTER;
     DeviceParams dp;
     int st = make_device_params(p, h_lut, &dp);
@@ -469,7 +503,7 @@ int nsc_pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, con
         if (!s.busy) return NSC_OK;
         cudaError_t er = cudaEventSynchronize(s.done);
         if (er != cudaSuccess) return record_cuda(er);
-        memcpy(h_out + (size_t)pending[k].first * D, s.h_out, (size_t)pending[k].count * D * 4);
+        memcpy((char*)h_out + (size_t)pending[k].first * D * out_bytes, s.h_out, (size_t)pending[k].count * D * out_bytes);
         s.busy = false;
         return NSC_OK;
     };
@@ -491,10 +525,9 @@ int nsc_pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, con
             st = record_cuda(e);
             break;
         }
-        st = launch_encode(s.d_points, point_stride, s.d_offsets, 0, ns, dp, s.d_out, nullptr, 0, nullptr, 0,
-                           0, s.d_ws, 256, s.stream);
+        st = launch_slot(s, point_stride, 0, ns, dp, out_bytes, q_eps);
         if (st != NSC_OK) break;
-        if ((e = cudaMemcpyAsync(s.h_out, s.d_out, (size_t)ns * D * 4, cudaMemcpyDeviceToHost, s.stream)) != cudaSuccess ||
+        if ((e = cudaMemcpyAsync(s.h_out, s.d_out, (size_t)ns * D * out_bytes, cudaMemcpyDeviceToHost, s.stream)) != cudaSuccess ||
             (e = cudaEventRecord(s.done, s.stream)) != cudaSuccess) {
             st = record_cuda(e);
             break;
@@ -511,6 +544,32 @@ int nsc_pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, con
     }
     cudaSetDevice(prev);
     return st;
+}
+
+extern "C" {
+
+int nsc_pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_stride,
+                        int64_t n_points, const int64_t* h_offsets, int n_scans,
+                        const nsc_params* p, const int32_t* h_lut, float* h_out) {
+    return pipeline_encode(pl, h_points, point_stride, n_points, h_offsets, n_scans, p, h_lut, h_out, 4, 0.0f);
+}
+
+int nsc_pipeline_encode_u16(nsc_pipeline* pl, const float* h_points, int point_stride,
+                            int64_t n_points, const int64_t* h_offsets, int n_scans,
+                            const nsc_params* p, const int32_t* h_lut, float q_epsilon, uint16_t* h_out) {
+    return pipeline_encode(pl, h_points, point_stride, n_points, h_offsets, n_scans, p, h_lut, h_out, 2, q_epsilon);
+}
+
+int nsc_pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, const int64_t* h_counts,
+                              int point_stride, int n_scans, const nsc_params* p,
+                              const int32_t* h_lut, float* h_out) {
+    return pipeline_encode_scans(pl, h_scans, h_counts, point_stride, n_scans, p, h_lut, h_out, 4, 0.0f);
+}
+
+int nsc_pipeline_encode_scans_u16(nsc_pipeline* pl, const float* const* h_scans, const int64_t* h_counts,
+                                  int point_stride, int n_scans, const nsc_params* p,
+                                  const int32_t* h_lut, float q_epsilon, uint16_t* h_out) {
+    return pipeline_encode_scans(pl, h_scans, h_counts, point_stride, n_scans, p, h_lut, h_out, 2, q_epsilon);
 }
 
 // One scan from pageable host memory to a descriptor ON THE DEVICE, on the caller's stream: the

@@ -42,6 +42,11 @@ struct EncodeArgs {
     long long origin;
     int n_scans;
     float* out;          // n_scans x D, may be null (projection only)
+    // n_scans x D uint16 wire format instead of `out` (never both): the quantiser's epsilon and the
+    // pairwise-sum plan for rows of D elements (nsc_quantize.cuh), built once per launch on the host
+    unsigned short* out_q;
+    float q_eps;
+    SumPlan q_plan;
     float* img_out;      // n_scans x E x 360, may be null
     int stage;
     unsigned* counter;
@@ -395,7 +400,7 @@ __device__ __forceinline__ void finish_scan(const EncodeArgs& a, const DevicePar
         }
     }
     NSC_PHASE(2);
-    if (a.out || a.peers.n > 0) {
+    if (a.out || a.out_q || a.peers.n > 0) {
 #ifdef NSC_PHASE_TIMING
         spectrum_and_bins(S, dp, dp.E, [&](int p) { NSC_PHASE(p); });
 #else
@@ -403,7 +408,8 @@ __device__ __forceinline__ void finish_scan(const EncodeArgs& a, const DevicePar
 #endif
         NSC_PHASE(3);
         normalise_and_store(S, dp, a.out ? a.out + (long long)scan * D : nullptr, a.peers,
-                            a.peers.row0 + scan);
+                            a.peers.row0 + scan, a.out_q ? a.out_q + (long long)scan * D : nullptr, a.q_eps,
+                            &a.q_plan);
         NSC_PHASE(4);
     }
     (void)phase_t0;
@@ -746,7 +752,8 @@ __device__ __forceinline__ void ws_tail_role(const EncodeArgs& a, const DevicePa
             }
             if (NSC_EXP_TAIL_PARTS & 8)
                 normalise_and_store(S, dp, a.out ? a.out + (long long)scan * D : nullptr, a.peers,
-                                    a.peers.row0 + scan, G());
+                                    a.peers.row0 + scan, a.out_q ? a.out_q + (long long)scan * D : nullptr,
+                                    a.q_eps, &a.q_plan, G());
         }
 #else
         float* stage0 = (a.img_out && a.stage == NSC_STAGE_PROJECTED)
@@ -760,10 +767,11 @@ __device__ __forceinline__ void ws_tail_role(const EncodeArgs& a, const DevicePa
                 a.img_out[(long long)scan * dp.E * kAz + i] = S.img[S.src[r] * kPitch + c];
             }
         }
-        if (a.out || a.peers.n > 0) {
+        if (a.out || a.out_q || a.peers.n > 0) {
             spectrum_and_bins(S, dp, dp.E, [&](int p) { if (p == 9) release(); }, G());
             normalise_and_store(S, dp, a.out ? a.out + (long long)scan * D : nullptr, a.peers,
-                                a.peers.row0 + scan, G());
+                                a.peers.row0 + scan, a.out_q ? a.out_q + (long long)scan * D : nullptr,
+                                a.q_eps, &a.q_plan, G());
         } else {
             G::sync();     // every thread is done reading the image
             release();
@@ -898,7 +906,7 @@ encode_images_kernel(const float* __restrict__ images, int n_images, int rows,
         }
         __syncthreads();
         spectrum_and_bins(S, dp, rows);
-        normalise_and_store(S, dp, out + (long long)im * D, none, 0);
+        normalise_and_store(S, dp, out + (long long)im * D, none, 0, nullptr, 0.0f, nullptr);
     }
     if (threadIdx.x == 0) wait_bulk_stores_done();
 }
@@ -1009,7 +1017,8 @@ size_t workspace_bytes_min() { return kMinWorkspace; }
 int launch_encode(const float* d_points, int stride, const long long* d_offsets, long long origin,
                   int n_scans, const DeviceParams& dp, float* d_out, float* d_img_out, int stage,
                   float* const* d_peer_out, int n_peers, long long peer_row0,
-                  unsigned* d_workspace, size_t workspace_bytes, cudaStream_t stream) {
+                  unsigned* d_workspace, size_t workspace_bytes, cudaStream_t stream,
+                  unsigned short* d_out_q, float q_eps) {
     if (n_scans == 0) return NSC_OK;
     DeviceInfo di;
     int st = device_info(&di);
@@ -1020,6 +1029,13 @@ int launch_encode(const float* d_points, int stride, const long long* d_offsets,
     a.origin = origin;
     a.n_scans = n_scans;
     a.out = d_out;
+    a.out_q = d_out_q;
+    a.q_eps = q_eps;
+    memset(&a.q_plan, 0, sizeof(a.q_plan));
+    if (d_out_q) {
+        st = build_plan(dp.T * dp.n_bins, &a.q_plan);    // D <= NSC_MAX_DESCRIPTOR: always fits
+        if (st != NSC_OK) return st;
+    }
     a.img_out = d_img_out;
     a.stage = stage;
     a.counter = d_workspace;

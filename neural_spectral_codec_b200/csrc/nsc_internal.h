@@ -47,7 +47,8 @@ int record_cuda(cudaError_t e);
 int launch_encode(const float* d_points, int stride, const long long* d_offsets, long long origin,
                   int n_scans, const DeviceParams& dp, float* d_out, float* d_img_out, int stage,
                   float* const* d_peer_out, int n_peers, long long peer_row0,
-                  unsigned* d_workspace, size_t workspace_bytes, cudaStream_t stream);
+                  unsigned* d_workspace, size_t workspace_bytes, cudaStream_t stream,
+                  unsigned short* d_out_q = nullptr, float q_eps = 0.0f);   // d_out_q: uint16 rows instead of d_out
 int launch_encode_images(const float* d_images, int n_images, int rows, const DeviceParams& dp,
                          float* d_out, cudaStream_t stream);
 int launch_interpolate(const float* d_in, int n_images, int rows, int nearest, float* d_out, cudaStream_t stream);

@@ -2,11 +2,13 @@
 //   validity masks -> circular linear hole interpolation + empty-row fill
 //   (reference src/encoding/range_image.py:15-89) -> optional row pooling
 //   (spectral_encoder.py:171-176) -> 360-point FFT magnitude per row (:180-186) ->
-//   contiguous-frequency bin sums (:118-158) -> L1 normalisation (:197-202).
+//   contiguous-frequency bin sums (:118-158) -> L1 normalisation (:197-202) -> optionally the
+//   uint16 wire format (HistogramQuantizer.quantize, quantization.py:131-167).
 // All functions are CTA-collective: every thread of the block must call them.
 #pragma once
 #include "nsc_fft.cuh"
 #include "nsc_internal.h"
+#include "nsc_quantize.cuh"
 
 namespace nsc {
 
@@ -314,16 +316,107 @@ __device__ __forceinline__ void spectrum_and_bins(const TailSmem& S, const P& dp
     }
 }
 
-// h / (sum h + eps), or the uniform descriptor when sum h <= eps (spectral_encoder.py:197-202).
 struct PeerOut {
     float* ptr[NSC_MAX_PEERS];
     int n;
     long long row0;
 };
 
+// The uint16 epilogue of normalise_and_store: the normalised row -- the float32 values the float
+// path stores -- goes through HistogramQuantizer.quantize as nsc_quantize_histograms would take it
+// from global memory (NumPy-order row sum, one division, half-to-even rounding, the rounding error
+// added to the first largest bin) and leaves as 2 D bytes. Shared memory: the row stays in S.hist
+// (integers in place, then packed to uint16 at its front), the pairwise-sum slots use S.fa (dead
+// once the bin sums are in S.hist; the next scan writes it only after a group barrier), the
+// per-warp partials and the row sum use S.red.
+template <typename G>
+__device__ __forceinline__ void quantise_and_store(const TailSmem& S, int D, bool ok, float denom, float uniform,
+                                                   unsigned short* out_q, float q_eps, const SumPlan& plan) {
+    const int warp = G::tid() >> 5, lane = G::tid() & 31;
+    unsigned* part = reinterpret_cast<unsigned*>(S.red);          // [0, 2 warps): integer sums, first maxima
+    float* sum_s = reinterpret_cast<float*>(S.red) + 2 * G::kGroupWarps;
+    static_assert(4 * (2 * G::kGroupWarps + 1) <= kWarps * 8 + 16, "S.red holds the partials");
+    for (int i = G::tid(); i < D; i += G::kSize) S.hist[i] = ok ? __fdiv_rn(S.hist[i], denom) : uniform;
+    G::sync();                     // also: every thread has read the float path's partials in S.red
+    if (warp == 0) {
+        const float s = numpy_sum(S.hist, plan, reinterpret_cast<float*>(S.fa), lane);
+        if (lane == 0) *sum_s = s;
+    }
+    G::sync();
+    const float sum = *sum_s;
+    const bool norm = sum > q_eps;                                 // quantization.py:144-146
+    const float qden = __fadd_rn(sum, q_eps);
+    // the hoisted division gives __fdiv_rn's bits for a denominator of moderate size (RowDivisor)
+    const bool hoisted = norm && moderate(qden);
+    const RowDivisor div(hoisted ? qden : 1.0f);
+    unsigned qsum = 0, best = 0;                                   // best: (q << 16) | (0xffff - index)
+    for (int i = G::tid(); i < D; i += G::kSize) {
+        const float h = S.hist[i];
+        const int q = quantise_value(norm ? (hoisted ? div(h) : __fdiv_rn(h, qden)) : h);
+        S.hist[i] = __int_as_float(q);                             // own entry: no barrier needed
+        qsum += (unsigned)q;
+        best = max(best, ((unsigned)q << 16) | (0xffffu - (unsigned)i));
+    }
+    qsum = __reduce_add_sync(0xffffffffu, qsum);
+    best = __reduce_max_sync(0xffffffffu, best);
+    if (lane == 0) {
+        part[warp] = qsum;
+        part[G::kGroupWarps + warp] = best;
+    }
+    G::sync();
+    qsum = 0;
+    best = 0;
+    for (int w = 0; w < G::kGroupWarps; ++w) {
+        qsum += part[w];
+        best = max(best, part[G::kGroupWarps + w]);
+    }
+    // quantization.py:154-167: the rounding error goes into the first largest bin
+    int fix_idx = -1, fix_val = 0;
+    if ((int)qsum > 0 && qsum != 65535u) {
+        fix_idx = 0xffff - (int)(best & 0xffffu);
+        const int v = (int)(best >> 16) + (65535 - (int)qsum);
+        fix_val = v < 0 ? 0 : (v > 65535 ? 65535 : v);
+    }
+    const int* qs = reinterpret_cast<const int*>(S.hist);
+    if ((D & 7) == 0 && (reinterpret_cast<uintptr_t>(out_q) & 15) == 0) {
+        // pack in place, 8 integers (32 bytes) -> 16 bytes: unit u lands on bytes [16 u, 16 u + 16).
+        // A pass writes below everything later passes read; its barrier orders its own reads (and
+        // those of every earlier pass) before its writes.
+        const int n_units = D >> 3;
+        for (int u0 = 0; u0 < n_units; u0 += G::kSize) {
+            const int u = u0 + G::tid();
+            uint4 w = make_uint4(0u, 0u, 0u, 0u);
+            if (u < n_units) {
+                const int4 a = reinterpret_cast<const int4*>(qs)[2 * u];
+                const int4 b = reinterpret_cast<const int4*>(qs)[2 * u + 1];
+                const int e = 8 * u;
+                auto f = [&](int q, int k) { return (unsigned)(e + k == fix_idx ? fix_val : q); };
+                w = make_uint4(f(a.x, 0) | (f(a.y, 1) << 16), f(a.z, 2) | (f(a.w, 3) << 16),
+                               f(b.x, 4) | (f(b.y, 5) << 16), f(b.z, 6) | (f(b.w, 7) << 16));
+            }
+            G::sync();
+            if (u < n_units) reinterpret_cast<uint4*>(S.hist)[u] = w;
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic writes -> async-proxy reads
+        G::sync();
+        if (G::tid() == 0) {
+            bulk_store_s2g(out_q, S.hist, (uint32_t)D * 2u);
+            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        }
+        return;
+    }
+    for (int i = G::tid(); i < D; i += G::kSize) out_q[i] = (unsigned short)(i == fix_idx ? fix_val : qs[i]);
+    // S.red / S.hist / S.fa are next written after the barriers at the top of the next scan
+}
+
+// h / (sum h + eps), or the uniform descriptor when sum h <= eps (spectral_encoder.py:197-202), to
+// `out` and every peer as float32 or, with out_q set (out null, no peers), to out_q in the uint16
+// wire format of quantise_and_store (q_eps, plan: the quantiser's epsilon and sum plan for D).
 template <typename P, typename G = CtaGroup>
 __device__ __forceinline__ void normalise_and_store(const TailSmem& S, const P& dp, float* out,
-                                                    const PeerOut& peers, long long peer_row, G = G()) {
+                                                    const PeerOut& peers, long long peer_row,
+                                                    unsigned short* out_q, float q_eps, const SumPlan* plan,
+                                                    G = G()) {
     const int D = dp.T * dp.n_bins;
     const int warp = G::tid() >> 5, lane = G::tid() & 31;
     double acc = 0.0;
@@ -338,6 +431,10 @@ __device__ __forceinline__ void normalise_and_store(const TailSmem& S, const P& 
     const float total = (float)tot;
     const bool ok = total > dp.eps;
     const float denom = __fadd_rn(total, dp.eps);
+    if (out_q) {
+        quantise_and_store<G>(S, D, ok, denom, dp.uniform, out_q, q_eps, *plan);
+        return;
+    }
     // bulk path: 16-byte granularity of size and of every destination row
     bool bulk = ((D * 4) & 15) == 0 && (out == nullptr || (reinterpret_cast<uintptr_t>(out) & 15) == 0);
     for (int p = 0; p < peers.n; ++p) bulk = bulk && (reinterpret_cast<uintptr_t>(peers.ptr[p]) & 15) == 0;

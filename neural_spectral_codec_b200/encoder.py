@@ -17,7 +17,9 @@ Beyond the reference surface:
   * ``encode_points_batch(points, offsets)`` -- device-resident concatenated scans in, one
     fused kernel launch, ``(B, 800)`` out (the batched entry of ``BASELINE.json``);
   * ``encode_scans(scans)`` -- host buffers in, host descriptors out, H2D / encode / D2H
-    overlapped on rotating streams inside the library (the end-to-end path).
+    overlapped on rotating streams inside the library (the end-to-end path);
+  * ``dtype=torch.uint16`` / ``dtype=np.uint16`` on both -- the descriptors in the wire format of
+    ``HistogramQuantizer.quantize`` (the same integers), quantised in the encode kernel's epilogue.
 """
 from __future__ import annotations
 
@@ -187,6 +189,15 @@ def _anywidth_images(x, p, lut, method, out, images_out):
     _lib.check(st, "nsc_anywidth_images")
 
 
+def _quantize_rows(rows: torch.Tensor, out: torch.Tensor) -> None:
+    """float32 descriptor rows -> ``out`` in the wire format (``nsc_quantize_histograms``, the
+    reference quantiser's default epsilon): the second launch of widths without a fused kernel."""
+    with torch.cuda.device(rows.device):
+        st = _lib.load().nsc_quantize_histograms(rows.data_ptr(), rows.shape[0], rows.shape[1], _lib.QUANT_EPSILON,
+                                                 out.data_ptr(), torch.cuda.current_stream(rows.device).cuda_stream)
+    _lib.check(st, "nsc_quantize_histograms")
+
+
 def _check_batch(points: torch.Tensor, offsets: torch.Tensor):
     if not isinstance(points, torch.Tensor) or not points.is_cuda:
         raise _no_cpu("points must be a CUDA tensor")
@@ -300,29 +311,46 @@ class SpectralEncoder(nn.Module):
 
     # ------------------------------------------------------------------ points in
     def encode_points_batch(self, points: torch.Tensor, offsets: torch.Tensor,
-                            out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                            out: Optional[torch.Tensor] = None, dtype: torch.dtype = torch.float32) -> torch.Tensor:
         """``B`` scans concatenated on the device -> ``(B, output_dim)`` float32 on the device.
 
         points: float32 ``(sum N, 3|4)`` CUDA tensor, rows xyz[i] as the reference loaders give
         them; offsets: int64 ``(B+1,)`` point offsets. One fused kernel launch on the current
         stream; nothing synchronises.
+
+        ``dtype=torch.uint16`` returns the rows in the wire format instead: the integers
+        ``HistogramQuantizer(output_dim).quantize`` gives for the float32 rows (epsilon 1e-8, each
+        row summing to 65535), quantised in the same kernel launch. ``out``, if given, has ``dtype``.
+        Image widths other than 360 have no fused kernel: there the general kernel writes float32
+        rows and ``nsc_quantize_histograms`` quantises them -- the same integers, two launches.
         """
         lib = _lib.load()
+        if dtype not in (torch.float32, torch.uint16):
+            raise ValueError("dtype must be torch.float32 or torch.uint16")
         points, offsets, n_scans, stride = _check_batch(points, offsets)
         dev = points.device
         if out is None:
-            out = torch.empty((n_scans, self.output_dim), dtype=torch.float32, device=dev)
-        elif (out.shape != (n_scans, self.output_dim) or out.dtype != torch.float32
+            out = torch.empty((n_scans, self.output_dim), dtype=dtype, device=dev)
+        elif (out.shape != (n_scans, self.output_dim) or out.dtype != dtype
               or not out.is_contiguous() or out.device != dev):
-            raise ValueError("out must be a contiguous float32 (B, output_dim) tensor on the same device")
+            raise ValueError(f"out must be a contiguous {str(dtype)[6:]} (B, output_dim) tensor on the same device")
         p = self._params()
         lut = self.freq_to_bin()
         if self.n_azimuth != _lib.N_AZIMUTH:
-            _anywidth_points(points, offsets, n_scans, stride, p, lut, out, None, _lib.STAGE_INTERPOLATED)
+            rows = out if dtype == torch.float32 else torch.empty(out.shape, dtype=torch.float32, device=dev)
+            _anywidth_points(points, offsets, n_scans, stride, p, lut, rows, None, _lib.STAGE_INTERPOLATED)
+            if dtype == torch.uint16 and n_scans:
+                _quantize_rows(rows, out)
             return out
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
             ws = _workspace(dev, stream, p, n_scans)
+            if dtype == torch.uint16:
+                st = lib.nsc_encode_batch_u16(points.data_ptr(), stride, offsets.data_ptr(), 0, n_scans,
+                                              C.byref(p), lut.ctypes.data, _lib.QUANT_EPSILON, out.data_ptr(),
+                                              ws.data_ptr(), ws.numel() * 4, stream)
+                _lib.check(st, "nsc_encode_batch_u16")
+                return out
             st = lib.nsc_encode_batch(points.data_ptr(), stride, offsets.data_ptr(), 0, n_scans,
                                       C.byref(p), lut.ctypes.data, out.data_ptr(), ws.data_ptr(),
                                       ws.numel() * 4, stream)
@@ -369,15 +397,23 @@ class SpectralEncoder(nn.Module):
 
     def encode_scans(self, scans: Union[Sequence[np.ndarray], Tuple[np.ndarray, np.ndarray]],
                      out: Optional[np.ndarray] = None, max_chunk_points: int = 4_000_000,
-                     n_buffers: int = 3) -> np.ndarray:
+                     n_buffers: int = 3, dtype=np.float32) -> np.ndarray:
         """Host scans in, host descriptors out: ``(B, output_dim)`` float32 numpy.
 
         ``scans`` is a list of ``(N_i, 4)`` (or all ``(N_i, 3)``) float32 arrays, or a tuple
         ``(points, offsets)`` of an already concatenated host buffer (pinned memory gives the
         full PCIe rate). Copies and the fused kernel overlap on ``n_buffers`` streams inside
         ``nsc_pipeline_encode``; the call returns when ``out`` is complete.
+
+        ``dtype=np.uint16`` returns the wire format of ``encode_points_batch(..., dtype=torch.uint16)``
+        (``*_u16`` pipeline entry points: half the bytes cross PCIe, no float32 rows on the host);
+        ``out``, if given, has ``dtype``.
         """
         lib = _lib.load()
+        dtype = np.dtype(dtype)
+        if dtype not in (np.float32, np.uint16):
+            raise ValueError("dtype must be np.float32 or np.uint16")
+        u16 = dtype == np.uint16
         dev = self._cuda_device("encode_scans")
         arrs = None
         if isinstance(scans, tuple) and len(scans) == 2 and np.ndim(scans[1]) == 1:
@@ -401,14 +437,15 @@ class SpectralEncoder(nn.Module):
             np.cumsum([a.shape[0] for a in arrs], out=offs[1:])
         n_scans = offs.shape[0] - 1
         if out is None:
-            out = np.empty((n_scans, self.output_dim), np.float32)
-        elif out.shape != (n_scans, self.output_dim) or out.dtype != np.float32 or not out.flags.c_contiguous:
-            raise ValueError("out must be contiguous float32 (B, output_dim)")
+            out = np.empty((n_scans, self.output_dim), dtype)
+        elif out.shape != (n_scans, self.output_dim) or out.dtype != dtype or not out.flags.c_contiguous:
+            raise ValueError(f"out must be contiguous {dtype.name} (B, output_dim)")
         if n_scans == 0:
             return out
         if self.n_azimuth != _lib.N_AZIMUTH:     # other widths: the general kernel, one device batch
             host = pts if arrs is None else (np.concatenate(arrs) if len(arrs) else np.zeros((0, 4), np.float32))
-            d = self.encode_points_batch(torch.from_numpy(np.ascontiguousarray(host)).to(dev), torch.from_numpy(offs))
+            d = self.encode_points_batch(torch.from_numpy(np.ascontiguousarray(host)).to(dev), torch.from_numpy(offs),
+                                         dtype=torch.uint16 if u16 else torch.float32)
             out[...] = d.cpu().numpy()
             return out
         biggest = int(np.diff(offs).max())
@@ -424,12 +461,21 @@ class SpectralEncoder(nn.Module):
         if arrs is not None:   # separate host arrays: gathered into pinned staging inside the library
             ptrs = (C.c_void_p * n_scans)(*[a.ctypes.data for a in arrs])
             counts = np.diff(offs)
-            st = lib.nsc_pipeline_encode_scans(self._pipeline, ptrs, counts.ctypes.data, arrs[0].shape[1],
-                                               n_scans, C.byref(p), lut.ctypes.data, out.ctypes.data)
-            _lib.check(st, "nsc_pipeline_encode_scans")
+            args = (self._pipeline, ptrs, counts.ctypes.data, arrs[0].shape[1], n_scans, C.byref(p), lut.ctypes.data)
+            if u16:
+                st = lib.nsc_pipeline_encode_scans_u16(*args, _lib.QUANT_EPSILON, out.ctypes.data)
+                _lib.check(st, "nsc_pipeline_encode_scans_u16")
+            else:
+                st = lib.nsc_pipeline_encode_scans(*args, out.ctypes.data)
+                _lib.check(st, "nsc_pipeline_encode_scans")
             return out
-        st = lib.nsc_pipeline_encode(self._pipeline, pts.ctypes.data, pts.shape[1], pts.shape[0],
-                                     offs.ctypes.data, n_scans, C.byref(p), lut.ctypes.data, out.ctypes.data)
+        args = (self._pipeline, pts.ctypes.data, pts.shape[1], pts.shape[0], offs.ctypes.data, n_scans, C.byref(p),
+                lut.ctypes.data)
+        if u16:
+            st = lib.nsc_pipeline_encode_u16(*args, _lib.QUANT_EPSILON, out.ctypes.data)
+            _lib.check(st, "nsc_pipeline_encode_u16")
+            return out
+        st = lib.nsc_pipeline_encode(*args, out.ctypes.data)
         _lib.check(st, "nsc_pipeline_encode")
         return out
 
