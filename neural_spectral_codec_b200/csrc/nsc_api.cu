@@ -56,9 +56,12 @@ int encode_batch(const float* d_points, int point_stride, const int64_t* d_offse
     if (n_scans == 0) return NSC_OK;
     if (!d_out && !d_out_q) return NSC_ERR_NULL_POINTER;
     if (!d_workspace || workspace_bytes < workspace_bytes_min()) return NSC_ERR_WORKSPACE;
-    return launch_encode(d_points, point_stride, (const long long*)d_offsets, point_origin, n_scans,
-                         dp, d_out, nullptr, 0, nullptr, 0, 0, (unsigned*)d_workspace, workspace_bytes,
-                         (cudaStream_t)stream, d_out_q, q_epsilon);
+    EncodeOutputs out;
+    out.rows = d_out;
+    out.rows_q = d_out_q;
+    out.q_eps = q_epsilon;
+    return launch_encode({d_points, point_stride, (const long long*)d_offsets, point_origin, n_scans}, dp, out,
+                         (unsigned*)d_workspace, workspace_bytes, (cudaStream_t)stream);
 }
 }  // namespace
 
@@ -94,8 +97,11 @@ int nsc_encode_batch_peers(const float* d_points, int point_stride, const int64_
         if (!h_peer_db[i]) return NSC_ERR_NULL_POINTER;
     if (n_scans == 0) return NSC_OK;
     if (!d_workspace || workspace_bytes < workspace_bytes_min()) return NSC_ERR_WORKSPACE;
-    return launch_encode(d_points, point_stride, (const long long*)d_offsets, point_origin, n_scans,
-                         dp, nullptr, nullptr, 0, h_peer_db, n_peers, db_row0,
+    EncodeOutputs out;
+    out.peers = h_peer_db;
+    out.n_peers = n_peers;
+    out.peer_row0 = db_row0;
+    return launch_encode({d_points, point_stride, (const long long*)d_offsets, point_origin, n_scans}, dp, out,
                          (unsigned*)d_workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
@@ -160,9 +166,11 @@ int nsc_project_batch(const float* d_points, int point_stride, const int64_t* d_
     if (n_scans == 0) return NSC_OK;
     if (!d_images) return NSC_ERR_NULL_POINTER;
     if (!d_workspace || workspace_bytes < workspace_bytes_min()) return NSC_ERR_WORKSPACE;
-    return launch_encode(d_points, point_stride, (const long long*)d_offsets, point_origin, n_scans,
-                         dp, nullptr, d_images, stage, nullptr, 0, 0, (unsigned*)d_workspace, workspace_bytes,
-                         (cudaStream_t)stream);
+    EncodeOutputs out;
+    out.images = d_images;
+    out.stage = stage;
+    return launch_encode({d_points, point_stride, (const long long*)d_offsets, point_origin, n_scans}, dp, out,
+                         (unsigned*)d_workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int nsc_encode_range_images(const float* d_images, int n_images, int rows, const nsc_params* p,
@@ -356,16 +364,8 @@ int nsc_pipeline_create(int64_t max_chunk_points, int n_buffers, int device, nsc
 
 }  // extern "C"
 
-// Encodes a staged chunk into the slot's device descriptors: float32 (out_bytes 4), or uint16
-// (out_bytes 2) in the first half of the same buffer.
-static int launch_slot(nsc_pipeline::Slot& s, int stride, long long origin, int ns, const DeviceParams& dp,
-                       size_t out_bytes, float q_eps) {
-    return launch_encode(s.d_points, stride, s.d_offsets, origin, ns, dp, out_bytes == 4 ? s.d_out : nullptr, nullptr,
-                         0, nullptr, 0, 0, s.d_ws, 256, s.stream,
-                         out_bytes == 2 ? reinterpret_cast<unsigned short*>(s.d_out) : nullptr, q_eps);
-}
-
-// nsc_pipeline_encode / nsc_pipeline_encode_u16: descriptors of out_bytes (4 or 2) per element.
+// nsc_pipeline_encode / nsc_pipeline_encode_u16: descriptors of out_bytes (4 or 2) per element,
+// the uint16 ones in the first half of the slot's float32 descriptor buffer.
 static int pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_stride, int64_t n_points,
                            const int64_t* h_offsets, int n_scans, const nsc_params* p, const int32_t* h_lut,
                            void* h_out, size_t out_bytes, float q_eps) {
@@ -387,6 +387,8 @@ static int pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_st
     if (e != cudaSuccess) return record_cuda(e);
     e = cudaSetDevice(pl->device);
     if (e != cudaSuccess) return record_cuda(e);
+    EncodeOutputs out;
+    out.q_eps = q_eps;
 
     int first = 0, k = 0;
     while (first < n_scans && st == NSC_OK) {
@@ -411,7 +413,9 @@ static int pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_st
             st = record_cuda(e);
             break;
         }
-        st = launch_slot(s, point_stride, p0, ns, dp, out_bytes, q_eps);
+        if (out_bytes == 4) out.rows = s.d_out;
+        else out.rows_q = reinterpret_cast<unsigned short*>(s.d_out);
+        st = launch_encode({s.d_points, point_stride, s.d_offsets, p0, ns}, dp, out, s.d_ws, 256, s.stream);
         if (st != NSC_OK) break;
         if ((e = cudaMemcpyAsync((char*)h_out + (size_t)first * D * out_bytes, s.d_out, (size_t)ns * D * out_bytes,
                                  cudaMemcpyDeviceToHost, s.stream)) != cudaSuccess ||
@@ -462,7 +466,7 @@ static void stage_scans(float* dst, const float* const* h_scans, const int64_t* 
     for (auto& th : pool) th.join();
 }
 
-// nsc_pipeline_encode_scans / nsc_pipeline_encode_scans_u16: descriptors of out_bytes (4 or 2) per element.
+// nsc_pipeline_encode_scans / nsc_pipeline_encode_scans_u16: descriptors as in pipeline_encode.
 static int pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, const int64_t* h_counts,
                                  int point_stride, int n_scans, const nsc_params* p, const int32_t* h_lut,
                                  void* h_out, size_t out_bytes, float q_eps) {
@@ -486,6 +490,8 @@ static int pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, 
     e = cudaSetDevice(pl->device);
     if (e != cudaSuccess) return record_cuda(e);
 
+    EncodeOutputs out;
+    out.q_eps = q_eps;
     // pinned staging for every slot, allocated on the first call of this entry point
     for (int i = 0; i < pl->n_buffers; ++i) {
         nsc_pipeline::Slot& s = pl->slot[i];
@@ -525,7 +531,9 @@ static int pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, 
             st = record_cuda(e);
             break;
         }
-        st = launch_slot(s, point_stride, 0, ns, dp, out_bytes, q_eps);
+        if (out_bytes == 4) out.rows = s.d_out;
+        else out.rows_q = reinterpret_cast<unsigned short*>(s.d_out);
+        st = launch_encode({s.d_points, point_stride, s.d_offsets, 0, ns}, dp, out, s.d_ws, 256, s.stream);
         if (st != NSC_OK) break;
         if ((e = cudaMemcpyAsync(s.h_out, s.d_out, (size_t)ns * D * out_bytes, cudaMemcpyDeviceToHost, s.stream)) != cudaSuccess ||
             (e = cudaEventRecord(s.done, s.stream)) != cudaSuccess) {
@@ -613,7 +621,9 @@ int nsc_pipeline_encode_scan(nsc_pipeline* pl, const float* h_points, int point_
     }
     const size_t bytes = (size_t)n_points * point_stride * 4;
     if (bytes && (e = pl->pool->run(h_points, s.h_stage, s.d_points, bytes, 256 << 10, cs)) != cudaSuccess) return fail(e);
-    st = launch_encode(s.d_points, point_stride, s.d_offsets, 0, 1, dp, d_out, nullptr, 0, nullptr, 0, 0, s.d_ws, 256, cs);
+    EncodeOutputs out;
+    out.rows = d_out;
+    st = launch_encode({s.d_points, point_stride, s.d_offsets, 0, 1}, dp, out, s.d_ws, 256, cs);
     if (st == NSC_OK) {
         if ((e = cudaEventRecord(s.done, cs)) != cudaSuccess) return fail(e);
         s.busy = true;

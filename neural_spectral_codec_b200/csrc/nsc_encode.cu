@@ -36,21 +36,36 @@ namespace {
 #endif
 constexpr int kUnroll = 4;   // independent 16-byte loads in flight per thread (LDG feed)
 
+// EncodeOutputs as the kernels read it: the peer pointers by value, and with rows_q the quantiser's
+// pairwise-sum plan for rows of D elements (nsc_quantize.cuh), built once per launch on the host.
+struct KernelOutputs {
+    float* rows;
+    unsigned short* rows_q;
+    float q_eps;
+    SumPlan q_plan;
+    float* images;
+    int stage;
+    PeerOut peers;
+    __device__ bool descriptors() const { return rows || rows_q || peers.n > 0; }
+    __device__ RowDest row(int scan, int D) const {
+        RowDest d;
+        d.out = rows ? rows + (long long)scan * D : nullptr;
+        d.peers = &peers;
+        d.peer_row = peers.row0 + scan;
+        d.out_q = rows_q ? rows_q + (long long)scan * D : nullptr;
+        d.q_eps = q_eps;
+        d.plan = &q_plan;
+        return d;
+    }
+};
+
 struct EncodeArgs {
     const float* points;
     const long long* offsets;
     long long origin;
     int n_scans;
-    float* out;          // n_scans x D, may be null (projection only)
-    // n_scans x D uint16 wire format instead of `out` (never both): the quantiser's epsilon and the
-    // pairwise-sum plan for rows of D elements (nsc_quantize.cuh), built once per launch on the host
-    unsigned short* out_q;
-    float q_eps;
-    SumPlan q_plan;
-    float* img_out;      // n_scans x E x 360, may be null
-    int stage;
+    KernelOutputs out;
     unsigned* counter;
-    PeerOut peers;
     // warp-specialised kernel: the last n_scans - n_whole scans are handed out in `parts` pieces
     // each, so that the final, partial wave of the grid is spread over all CTAs (see launch_encode)
     int n_whole, parts, n_units;
@@ -363,12 +378,11 @@ __device__ __forceinline__ void point_pass(const float* __restrict__ points, lon
     }
 }
 
-// Everything after the scatter for one scan: keys -> ranges, interpolation, (optional) image
-// output, spectrum, bins, normalisation, descriptor store. CTA-collective.
 #ifdef NSC_PHASE_TIMING
 // Tuning build: thread 0 of every CTA accumulates the cycles it spends in each phase of a scan
 // into counter[4 + 2*phase] (64-bit), phases: 0 init, 1 point pass, 2 rows_to_filled,
-// 3 spectrum_and_bins, 4 normalise. Read back by tools/phase_timing.py.
+// 3 spectrum_and_bins, 4 normalise, 5..9 the sub-phases of spectrum_and_bins. Read back by
+// tools/phase_timing.py.
 #define NSC_PHASE(p)                                                                         \
     do {                                                                                     \
         if (threadIdx.x == 0) {                                                              \
@@ -379,40 +393,38 @@ __device__ __forceinline__ void point_pass(const float* __restrict__ points, lon
         }                                                                                    \
     } while (0)
 #else
-#define NSC_PHASE(p) do { } while (0)
+#define NSC_PHASE(p) do { (void)phase_t0; } while (0)
 #endif
 
-__device__ __forceinline__ void finish_scan(const EncodeArgs& a, const DeviceParams& dp,
-                                            const TailSmem& S, int scan, long long& phase_t0) {
-    const int tid = threadIdx.x;
+// Everything after the scatter for one scan, run by the thread group G: keys -> ranges,
+// interpolation, (optional) image output, spectrum, bins, normalisation, descriptor store.
+// `mark(p)` is called between the phases: 2, 3 and 4 here, 5..9 inside spectrum_and_bins (9: the
+// image is read for the last time). Returns false, right after the image output, when the launch
+// writes no descriptors.
+template <typename G, typename Mark>
+__device__ __forceinline__ bool finish_scan(const EncodeArgs& a, const DeviceParams& dp,
+                                            const TailSmem& S, int scan, Mark mark) {
+    const KernelOutputs& o = a.out;
     const int D = dp.T * dp.n_bins;
     // bits of min s -> range = sqrt_rn(s); empty -> 0 (range_image.py:162,:214); masks; hole
     // interpolation; empty-row indirection
-    float* stage0 = (a.img_out && a.stage == NSC_STAGE_PROJECTED)
-                        ? a.img_out + (long long)scan * dp.E * kAz : nullptr;
-    rows_to_filled<true>(S, dp.E, dp.interpolate != 0, stage0, [&dp](uint32_t key) {
+    float* stage0 = (o.images && o.stage == NSC_STAGE_PROJECTED) ? o.images + (long long)scan * dp.E * kAz : nullptr;
+    rows_to_filled<true, G>(S, dp.E, dp.interpolate != 0, stage0, [&dp](uint32_t key) {
         return key_is_empty(key, dp) ? 0.0f : __fsqrt_rn(__uint_as_float(key));
     });
-    if (a.img_out && a.stage == NSC_STAGE_INTERPOLATED) {
-        for (int i = tid; i < dp.E * kAz; i += kThreads) {
+    if (o.images && o.stage == NSC_STAGE_INTERPOLATED) {
+        for (int i = G::tid(); i < dp.E * kAz; i += G::kSize) {
             const int r = i / kAz, c = i - r * kAz;
-            a.img_out[(long long)scan * dp.E * kAz + i] = S.img[S.src[r] * kPitch + c];
+            o.images[(long long)scan * dp.E * kAz + i] = S.img[S.src[r] * kPitch + c];
         }
     }
-    NSC_PHASE(2);
-    if (a.out || a.out_q || a.peers.n > 0) {
-#ifdef NSC_PHASE_TIMING
-        spectrum_and_bins(S, dp, dp.E, [&](int p) { NSC_PHASE(p); });
-#else
-        spectrum_and_bins(S, dp, dp.E);
-#endif
-        NSC_PHASE(3);
-        normalise_and_store(S, dp, a.out ? a.out + (long long)scan * D : nullptr, a.peers,
-                            a.peers.row0 + scan, a.out_q ? a.out_q + (long long)scan * D : nullptr, a.q_eps,
-                            &a.q_plan);
-        NSC_PHASE(4);
-    }
-    (void)phase_t0;
+    mark(2);
+    if (!o.descriptors()) return false;
+    spectrum_and_bins(S, dp, dp.E, mark, G());
+    mark(3);
+    normalise_and_store(S, dp, o.row(scan, D), G());
+    mark(4);
+    return true;
 }
 
 template <int STRIDE, int ROWMODE, int FEED>
@@ -454,7 +466,7 @@ encode_points_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant
         point_pass<STRIDE, ROWMODE, FEED>(a.points, beg, n, dp, img_biased, smem_raw + L.ring_off, g_stage);
         __syncthreads();
         NSC_PHASE(1);
-        finish_scan(a, dp, S, scan, phase_t0);
+        finish_scan<CtaGroup>(a, dp, S, scan, [&](int p) { NSC_PHASE(p); });
     }
     if (tid == 0) wait_bulk_stores_done();      // descriptors leave shared memory before the CTA does
 }
@@ -564,7 +576,7 @@ __device__ __forceinline__ void ws_producer_role(const EncodeArgs& a, unsigned c
     int unit = blockIdx.x;
     int next = (int)gridDim.x + (int)atomicAdd(a.counter, 1u);
     const uint64_t pol = l2_policy_evict_first();
-    const bool hint = NSC_L2_HINTS != 0 && a.peers.n == 0;
+    const bool hint = NSC_L2_HINTS != 0 && a.out.peers.n == 0;
     uint32_t slot = 0, phase = 0;                     // phase = (stage counter / kWsDepth) & 1
     bool wrapped = false;
     for (int k = 0;; ++k) {
@@ -666,7 +678,6 @@ __device__ __forceinline__ void ws_tail_role(const EncodeArgs& a, const DevicePa
     S.src = (int*)(smem + L.src_off);
     S.red = (double*)(smem + L.red_off);
     S.bin_start = smem + L.bins_off;
-    [[maybe_unused]] const int D = dp.T * dp.n_bins;
     for (int k = 0;; ++k) {
         const int b = k & 1;
         int scan, n_unused;
@@ -703,80 +714,10 @@ __device__ __forceinline__ void ws_tail_role(const EncodeArgs& a, const DevicePa
             for (int i = gt; i < L.img_words; i += G::kSize) img[i] = __ldcg(g + i);
             G::sync();
         }
-#ifdef NSC_EXP_SKIP_TAIL
-        release();      // measurement-only build: no tail at all (descriptors are not written)
-#elif defined(NSC_EXP_TAIL_PARTS)
-        // measurement-only builds: run only the parts of the tail selected by the bit mask
-        // (1 = ranges + interpolation, 2 = signal load + FFT, 4 = magnitudes + bins, 8 = normalise + store)
-        if (NSC_EXP_TAIL_PARTS & 1)
-            rows_to_filled<true, G>(S, dp.E, dp.interpolate != 0, nullptr, [&dp](uint32_t key) {
-                return key_is_empty(key, dp) ? 0.0f : __fsqrt_rn(__uint_as_float(key));
-            });
-        else if (gt < dp.E) S.src[gt] = gt;
-        G::sync();
-        {
-            const int n_sig = (dp.T + 1) / 2;
-            float* mag = reinterpret_cast<float*>(S.fa);
-            if (NSC_EXP_TAIL_PARTS & 2) {
-                for (int t = gt; t < n_sig * kAz; t += G::kSize) {
-                    const int g = t / kAz, n = t - g * kAz;
-                    S.fa[t] = make_float2(pooled_value(S, dp.E, dp.T, 2 * g, n), pooled_value(S, dp.E, dp.T, 2 * g + 1, n));
-                }
-                G::sync();
-                fft_pass<8, 1, G>(S.fa, S.fb, S.tw, n_sig);
-                G::sync();
-                fft_pass<9, 8, G>(S.fb, S.fa, S.tw, n_sig);
-                G::sync();
-                fft_pass<5, 72, G>(S.fa, S.fb, S.tw, n_sig);
-                G::sync();
-            }
-            if (NSC_EXP_TAIL_PARTS & 4) {
-                for (int t = gt; t < n_sig * kFreqs; t += G::kSize) {
-                    const int g = t / kFreqs, k = t - g * kFreqs;
-                    const float2* z = S.fb + g * kAz;
-                    const float2 p = z[k], m = z[k == 0 ? 0 : kAz - k];
-                    const float ar = p.x + m.x, ai = p.y - m.y, br = p.y + m.y, bi = p.x - m.x;
-                    mag[(2 * g) * kFreqs + k] = 0.5f * __fsqrt_rn(fmaf(ar, ar, ai * ai));
-                    mag[(2 * g + 1) * kFreqs + k] = 0.5f * __fsqrt_rn(fmaf(br, br, bi * bi));
-                }
-                G::sync();
-            }
-            release();
-            if (NSC_EXP_TAIL_PARTS & 4) {
-                for (int i = gt; i < dp.T * dp.n_bins; i += G::kSize) {
-                    const int r = i / dp.n_bins, bb = i - r * dp.n_bins;
-                    float h = 0.0f;
-                    for (int k = S.bin_start[bb], k1 = S.bin_start[bb + 1]; k < k1; ++k) h += mag[r * kFreqs + k];
-                    S.hist[i] = h;
-                }
-            }
-            if (NSC_EXP_TAIL_PARTS & 8)
-                normalise_and_store(S, dp, a.out ? a.out + (long long)scan * D : nullptr, a.peers,
-                                    a.peers.row0 + scan, a.out_q ? a.out_q + (long long)scan * D : nullptr,
-                                    a.q_eps, &a.q_plan, G());
-        }
-#else
-        float* stage0 = (a.img_out && a.stage == NSC_STAGE_PROJECTED)
-                            ? a.img_out + (long long)scan * dp.E * kAz : nullptr;
-        rows_to_filled<true, G>(S, dp.E, dp.interpolate != 0, stage0, [&dp](uint32_t key) {
-            return key_is_empty(key, dp) ? 0.0f : __fsqrt_rn(__uint_as_float(key));
-        });
-        if (a.img_out && a.stage == NSC_STAGE_INTERPOLATED) {
-            for (int i = gt; i < dp.E * kAz; i += G::kSize) {
-                const int r = i / kAz, c = i - r * kAz;
-                a.img_out[(long long)scan * dp.E * kAz + i] = S.img[S.src[r] * kPitch + c];
-            }
-        }
-        if (a.out || a.out_q || a.peers.n > 0) {
-            spectrum_and_bins(S, dp, dp.E, [&](int p) { if (p == 9) release(); }, G());
-            normalise_and_store(S, dp, a.out ? a.out + (long long)scan * D : nullptr, a.peers,
-                                a.peers.row0 + scan, a.out_q ? a.out_q + (long long)scan * D : nullptr,
-                                a.q_eps, &a.q_plan, G());
-        } else {
-            G::sync();     // every thread is done reading the image
+        if (!finish_scan<G>(a, dp, S, scan, [&](int p) { if (p == 9) release(); })) {
+            G::sync();     // projection only: every thread is done reading the image
             release();
         }
-#endif
         G::sync();         // S.red / S.hist / S.src are rewritten by the next scan's tail
         if (gt == 0) mail[16] = k + 1;                    // tail_done
     }
@@ -878,7 +819,7 @@ encode_points_split_kernel(const __grid_constant__ EncodeArgs a, const __grid_co
     if (rank == 0) {
         __syncthreads();
         long long phase_t0 = 0;
-        finish_scan(a, dp, S, scan, phase_t0);
+        finish_scan<CtaGroup>(a, dp, S, scan, [&](int p) { NSC_PHASE(p); });
         if (tid == 0) wait_bulk_stores_done();
     }
 }
@@ -894,9 +835,6 @@ encode_images_kernel(const float* __restrict__ images, int n_images, int rows,
     const int D = dp.T * dp.n_bins;
     init_tail_tables(S, dp);
     if (threadIdx.x < rows) S.src[threadIdx.x] = threadIdx.x;
-    PeerOut none;
-    none.n = 0;
-    none.row0 = 0;
     for (int im = blockIdx.x; im < n_images; im += gridDim.x) {
         __syncthreads();
         const float* src = images + (long long)im * rows * kAz;
@@ -906,7 +844,9 @@ encode_images_kernel(const float* __restrict__ images, int n_images, int rows,
         }
         __syncthreads();
         spectrum_and_bins(S, dp, rows);
-        normalise_and_store(S, dp, out + (long long)im * D, none, 0, nullptr, 0.0f, nullptr);
+        RowDest dst;
+        dst.out = out + (long long)im * D;
+        normalise_and_store(S, dp, dst);
     }
     if (threadIdx.x == 0) wait_bulk_stores_done();
 }
@@ -998,6 +938,23 @@ int configure(K kernel, int smem, const DeviceInfo& di, int* blocks_per_sm) {
     return NSC_OK;
 }
 
+using PointKernel = void (*)(const EncodeArgs, const DeviceParams);
+
+// The instantiation of the cluster (split) or the generic point kernel for a feed, a point stride
+// and a row mode; only the LDG feed reads 3-float points.
+#define NSC_POINT_KERNELS(K)                                                                     \
+    {{K<3, kRowPoly, kFeedLdg>, K<3, kRowSearch, kFeedLdg>},                                    \
+     {K<4, kRowPoly, kFeedLdg>, K<4, kRowSearch, kFeedLdg>},                                    \
+     {K<4, kRowPoly, kFeedCpAsync>, K<4, kRowSearch, kFeedCpAsync>},                            \
+     {K<4, kRowPoly, kFeedTma>, K<4, kRowSearch, kFeedTma>}}
+PointKernel point_kernel(bool split, int feed, int stride, int row_mode) {
+    static const PointKernel generic[4][2] = NSC_POINT_KERNELS(encode_points_kernel);
+    static const PointKernel cluster[4][2] = NSC_POINT_KERNELS(encode_points_split_kernel);
+    const int f = feed == kFeedTma ? 3 : feed == kFeedCpAsync ? 2 : stride == 4 ? 1 : 0;
+    return (split ? cluster : generic)[f][row_mode == kRowPoly ? 0 : 1];
+}
+#undef NSC_POINT_KERNELS
+
 }  // namespace
 
 // Workspace: [0, 256) work counter; [256, 256 + 4 * kMaxSplitScans) arrival counters and then one
@@ -1014,39 +971,37 @@ size_t workspace_bytes_for(int n_scans, int E) {
 }
 size_t workspace_bytes_min() { return kMinWorkspace; }
 
-int launch_encode(const float* d_points, int stride, const long long* d_offsets, long long origin,
-                  int n_scans, const DeviceParams& dp, float* d_out, float* d_img_out, int stage,
-                  float* const* d_peer_out, int n_peers, long long peer_row0,
-                  unsigned* d_workspace, size_t workspace_bytes, cudaStream_t stream,
-                  unsigned short* d_out_q, float q_eps) {
+int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutputs& out,
+                  unsigned* d_workspace, size_t workspace_bytes, cudaStream_t stream) {
+    const int n_scans = in.n_scans;
     if (n_scans == 0) return NSC_OK;
+    if (out.n_peers < 0 || out.n_peers > NSC_MAX_PEERS) return NSC_ERR_BAD_COUNT;
+    // uint16 rows are packed over the float32 row in shared memory: they are written alone
+    if (out.rows_q && (out.rows || out.n_peers > 0)) return NSC_ERR_BAD_PARAMS;
     DeviceInfo di;
     int st = device_info(&di);
     if (st != NSC_OK) return st;
-    EncodeArgs a;
-    a.points = d_points;
-    a.offsets = d_offsets;
-    a.origin = origin;
+    EncodeArgs a = {};
+    a.points = in.points;
+    a.offsets = in.offsets;
+    a.origin = in.origin;
     a.n_scans = n_scans;
-    a.out = d_out;
-    a.out_q = d_out_q;
-    a.q_eps = q_eps;
-    memset(&a.q_plan, 0, sizeof(a.q_plan));
-    if (d_out_q) {
-        st = build_plan(dp.T * dp.n_bins, &a.q_plan);    // D <= NSC_MAX_DESCRIPTOR: always fits
+    a.out.rows = out.rows;
+    a.out.rows_q = out.rows_q;
+    a.out.q_eps = out.q_eps;
+    if (out.rows_q) {
+        st = build_plan(dp.T * dp.n_bins, &a.out.q_plan);    // D <= NSC_MAX_DESCRIPTOR: always fits
         if (st != NSC_OK) return st;
     }
-    a.img_out = d_img_out;
-    a.stage = stage;
+    a.out.images = out.images;
+    a.out.stage = out.stage;
+    for (int i = 0; i < out.n_peers; ++i) a.out.peers.ptr[i] = out.peers[i];
+    a.out.peers.n = out.n_peers;
+    a.out.peers.row0 = out.peer_row0;
     a.counter = d_workspace;
-    a.peers.n = n_peers;
-    a.peers.row0 = peer_row0;
-    for (int i = 0; i < NSC_MAX_PEERS; ++i) a.peers.ptr[i] = i < n_peers ? d_peer_out[i] : nullptr;
     a.n_whole = n_scans;
     a.parts = 1;
     a.n_units = n_scans;
-    a.part_arrive = nullptr;
-    a.part_image = nullptr;
 
     // Feed of the point pass (see enum Feed) and kernel choice. Product builds take no switches;
     // tuning builds (-DNSC_TUNING, csrc/Makefile VARIANT=tune) read NSC_FEED=ldg|cpasync|tma,
@@ -1068,7 +1023,7 @@ int launch_encode(const float* d_points, int stride, const long long* d_offsets,
     split_allowed = env_split;
     ws_allowed = env_ws && feed_override < 0;
 #endif
-    if (stride != 4) feed = kFeedLdg;
+    if (in.stride != 4) feed = kFeedLdg;
     const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes_of(feed));
     int csize = 1;
     if (split_allowed) {
@@ -1076,21 +1031,9 @@ int launch_encode(const float* d_points, int stride, const long long* d_offsets,
         else if (n_scans * 4 <= di.sms) csize = 4;
         else if (n_scans * 2 <= di.sms) csize = 2;
     }
-    void (*kernel)(const EncodeArgs, const DeviceParams) = nullptr;
-    const bool poly = dp.row_mode == kRowPoly;
+    PointKernel kernel = nullptr;
     if (csize > 1) {
-        if (feed == kFeedTma)
-            kernel = poly ? encode_points_split_kernel<4, kRowPoly, kFeedTma>
-                          : encode_points_split_kernel<4, kRowSearch, kFeedTma>;
-        else if (feed == kFeedCpAsync)
-            kernel = poly ? encode_points_split_kernel<4, kRowPoly, kFeedCpAsync>
-                          : encode_points_split_kernel<4, kRowSearch, kFeedCpAsync>;
-        else if (stride == 4)
-            kernel = poly ? encode_points_split_kernel<4, kRowPoly, kFeedLdg>
-                          : encode_points_split_kernel<4, kRowSearch, kFeedLdg>;
-        else
-            kernel = poly ? encode_points_split_kernel<3, kRowPoly, kFeedLdg>
-                          : encode_points_split_kernel<3, kRowSearch, kFeedLdg>;
+        kernel = point_kernel(true, feed, in.stride, dp.row_mode);
         st = configure(kernel, L.total, di, nullptr);
         if (st != NSC_OK) return st;
         cudaLaunchConfig_t cfg = {};
@@ -1110,8 +1053,8 @@ int launch_encode(const float* d_points, int stride, const long long* d_offsets,
     // Large batches of 16-byte points: the warp-specialised kernel, when two images, the FFT
     // scratch and the ring fit one SM's shared memory; other geometries take the generic kernel.
     const WsLayout W(dp.E, dp.T, dp.n_bins);
-    if (ws_allowed && stride == 4 && W.ok && W.total <= di.max_smem_optin) {
-        kernel = poly ? encode_points_ws_kernel<kRowPoly> : encode_points_ws_kernel<kRowSearch>;
+    if (ws_allowed && in.stride == 4 && W.ok && W.total <= di.max_smem_optin) {
+        kernel = dp.row_mode == kRowPoly ? encode_points_ws_kernel<kRowPoly> : encode_points_ws_kernel<kRowSearch>;
         st = configure(kernel, W.total, di, nullptr);
         if (st != NSC_OK) return st;
         const int grid = di.sms < n_scans ? di.sms : n_scans;
@@ -1143,19 +1086,7 @@ int launch_encode(const float* d_points, int stride, const long long* d_offsets,
         kernel<<<grid, kWsThreads, W.total, stream>>>(a, dp);
         return record_cuda(cudaGetLastError());
     }
-    if (feed == kFeedTma) {
-        kernel = poly ? encode_points_kernel<4, kRowPoly, kFeedTma>
-                      : encode_points_kernel<4, kRowSearch, kFeedTma>;
-    } else if (feed == kFeedCpAsync) {
-        kernel = poly ? encode_points_kernel<4, kRowPoly, kFeedCpAsync>
-                      : encode_points_kernel<4, kRowSearch, kFeedCpAsync>;
-    } else if (stride == 4) {
-        kernel = poly ? encode_points_kernel<4, kRowPoly, kFeedLdg>
-                      : encode_points_kernel<4, kRowSearch, kFeedLdg>;
-    } else {
-        kernel = poly ? encode_points_kernel<3, kRowPoly, kFeedLdg>
-                      : encode_points_kernel<3, kRowSearch, kFeedLdg>;
-    }
+    kernel = point_kernel(false, feed, in.stride, dp.row_mode);
     int per_sm = 0;
     st = configure(kernel, L.total, di, &per_sm);
     if (st != NSC_OK) return st;

@@ -43,12 +43,35 @@ int validate_params(const nsc_params* p);
 // thread-local CUDA error text for nsc_last_cuda_error().
 int record_cuda(cudaError_t e);
 
+// The points of an encode launch: scan i is points [offsets[i] - origin, offsets[i + 1] - origin)
+// of `points`, `stride` floats (3 or 4) per point.
+struct PointBatch {
+    const float* points;
+    int stride;
+    const long long* offsets;    // n_scans + 1 entries, device memory
+    long long origin;
+    int n_scans;
+};
+
+// What an encode launch writes; every output left null is not written. Descriptor rows are
+// n_scans x D (D = T * n_bins): float32 to `rows` and to rows peer_row0 + scan of the n_peers
+// databases in `peers` (a host array of device pointers), or the uint16 wire format alone to
+// `rows_q` (HistogramQuantizer.quantize with epsilon q_eps). Range images are n_scans x E x 360,
+// taken at `stage` (NSC_STAGE_*).
+struct EncodeOutputs {
+    float* rows = nullptr;
+    unsigned short* rows_q = nullptr;
+    float q_eps = 0.0f;
+    float* images = nullptr;
+    int stage = NSC_STAGE_PROJECTED;
+    float* const* peers = nullptr;
+    int n_peers = 0;
+    long long peer_row0 = 0;
+};
+
 // Launchers (nsc_encode.cu)
-int launch_encode(const float* d_points, int stride, const long long* d_offsets, long long origin,
-                  int n_scans, const DeviceParams& dp, float* d_out, float* d_img_out, int stage,
-                  float* const* d_peer_out, int n_peers, long long peer_row0,
-                  unsigned* d_workspace, size_t workspace_bytes, cudaStream_t stream,
-                  unsigned short* d_out_q = nullptr, float q_eps = 0.0f);   // d_out_q: uint16 rows instead of d_out
+int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutputs& out,
+                  unsigned* d_workspace, size_t workspace_bytes, cudaStream_t stream);
 int launch_encode_images(const float* d_images, int n_images, int rows, const DeviceParams& dp,
                          float* d_out, cudaStream_t stream);
 int launch_interpolate(const float* d_in, int n_images, int rows, int nearest, float* d_out, cudaStream_t stream);

@@ -316,10 +316,25 @@ __device__ __forceinline__ void spectrum_and_bins(const TailSmem& S, const P& dp
     }
 }
 
+// The peer databases a launch copies every float32 descriptor row to (row row0 + scan).
 struct PeerOut {
     float* ptr[NSC_MAX_PEERS];
     int n;
     long long row0;
+};
+
+// Where normalise_and_store sends one descriptor row: float32 to `out` (if set) and to row
+// `peer_row` of every database in `peers` (if set), or, with out_q set (nothing else), the uint16
+// wire format of quantise_and_store to out_q (q_eps, plan: the quantiser's epsilon and the
+// pairwise-sum plan for D).
+struct RowDest {
+    float* out = nullptr;
+    const PeerOut* peers = nullptr;
+    long long peer_row = 0;
+    unsigned short* out_q = nullptr;
+    float q_eps = 0.0f;
+    const SumPlan* plan = nullptr;
+    __device__ int n_peers() const { return peers ? peers->n : 0; }
 };
 
 // The uint16 epilogue of normalise_and_store: the normalised row -- the float32 values the float
@@ -410,12 +425,9 @@ __device__ __forceinline__ void quantise_and_store(const TailSmem& S, int D, boo
 }
 
 // h / (sum h + eps), or the uniform descriptor when sum h <= eps (spectral_encoder.py:197-202), to
-// `out` and every peer as float32 or, with out_q set (out null, no peers), to out_q in the uint16
-// wire format of quantise_and_store (q_eps, plan: the quantiser's epsilon and sum plan for D).
+// the destinations of `dst`.
 template <typename P, typename G = CtaGroup>
-__device__ __forceinline__ void normalise_and_store(const TailSmem& S, const P& dp, float* out,
-                                                    const PeerOut& peers, long long peer_row,
-                                                    unsigned short* out_q, float q_eps, const SumPlan* plan,
+__device__ __forceinline__ void normalise_and_store(const TailSmem& S, const P& dp, RowDest dst,
                                                     G = G()) {
     const int D = dp.T * dp.n_bins;
     const int warp = G::tid() >> 5, lane = G::tid() & 31;
@@ -431,28 +443,29 @@ __device__ __forceinline__ void normalise_and_store(const TailSmem& S, const P& 
     const float total = (float)tot;
     const bool ok = total > dp.eps;
     const float denom = __fadd_rn(total, dp.eps);
-    if (out_q) {
-        quantise_and_store<G>(S, D, ok, denom, dp.uniform, out_q, q_eps, *plan);
+    if (dst.out_q) {
+        quantise_and_store<G>(S, D, ok, denom, dp.uniform, dst.out_q, dst.q_eps, *dst.plan);
         return;
     }
     // bulk path: 16-byte granularity of size and of every destination row
-    bool bulk = ((D * 4) & 15) == 0 && (out == nullptr || (reinterpret_cast<uintptr_t>(out) & 15) == 0);
-    for (int p = 0; p < peers.n; ++p) bulk = bulk && (reinterpret_cast<uintptr_t>(peers.ptr[p]) & 15) == 0;
+    bool bulk = ((D * 4) & 15) == 0 && (dst.out == nullptr || (reinterpret_cast<uintptr_t>(dst.out) & 15) == 0);
+    for (int p = 0; p < dst.n_peers(); ++p) bulk = bulk && (reinterpret_cast<uintptr_t>(dst.peers->ptr[p]) & 15) == 0;
     if (bulk) {
         for (int i = G::tid(); i < D; i += G::kSize) S.hist[i] = ok ? __fdiv_rn(S.hist[i], denom) : dp.uniform;
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic writes -> async-proxy reads
         G::sync();
         if (G::tid() == 0) {
-            if (out) bulk_store_s2g(out, S.hist, (uint32_t)D * 4u);
-            for (int p = 0; p < peers.n; ++p) bulk_store_s2g(peers.ptr[p] + peer_row * D, S.hist, (uint32_t)D * 4u);
+            if (dst.out) bulk_store_s2g(dst.out, S.hist, (uint32_t)D * 4u);
+            for (int p = 0; p < dst.n_peers(); ++p)
+                bulk_store_s2g(dst.peers->ptr[p] + dst.peer_row * D, S.hist, (uint32_t)D * 4u);
             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
         }
         return;
     }
     for (int i = G::tid(); i < D; i += G::kSize) {
         const float v = ok ? __fdiv_rn(S.hist[i], denom) : dp.uniform;
-        if (out) out[i] = v;
-        for (int p = 0; p < peers.n; ++p) peers.ptr[p][peer_row * D + i] = v;
+        if (dst.out) dst.out[i] = v;
+        for (int p = 0; p < dst.n_peers(); ++p) dst.peers->ptr[p][dst.peer_row * D + i] = v;
     }
     // S.red / S.hist are next written after the barriers at the top of the next scan
 }
