@@ -220,7 +220,10 @@ int nsc_anywidth_images(const float* d_images_in, int n_images, int rows, const 
 typedef struct nsc_pipeline nsc_pipeline;
 
 /* Creates a pipeline that stages at most max_chunk_points points per chunk through
- * n_buffers (2..4) device staging buffers with one stream each. */
+ * n_buffers (1..4) device staging buffers with one stream each. A pipeline serves one call at a
+ * time (calls from several threads must not overlap on it). Its encode entry points may be mixed on
+ * one pipeline: a buffer is reused only after the work that last used it, on whichever stream
+ * (nsc_pipeline_encode_scan's included), has finished. */
 int nsc_pipeline_create(int64_t max_chunk_points, int n_buffers, int device, nsc_pipeline** out);
 void nsc_pipeline_destroy(nsc_pipeline* pl);
 
@@ -228,9 +231,9 @@ void nsc_pipeline_destroy(nsc_pipeline* pl);
  * PCIe rate; pageable works), h_offsets int64[n_scans+1] starting at 0, h_out
  * float32[n_scans * target_rows * n_bins]. Chunks of whole scans are copied H2D, encoded
  * and copied back D2H on rotating streams so copies overlap compute. Synchronous: returns
- * when h_out is complete. A scan larger than max_chunk_points returns NSC_ERR_WORKSPACE;
- * offsets that decrease, start below 0 or end beyond n_points (the length of h_points in
- * points) return NSC_ERR_BAD_OFFSETS before anything is copied. */
+ * when h_out is complete. Offsets that decrease, start below 0 or end beyond n_points (the
+ * length of h_points in points) return NSC_ERR_BAD_OFFSETS, and a scan larger than
+ * max_chunk_points returns NSC_ERR_WORKSPACE, both before anything is copied. */
 int nsc_pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_stride,
                         int64_t n_points, const int64_t* h_offsets, int n_scans,
                         const nsc_params* p, const int32_t* h_lut, float* h_out);

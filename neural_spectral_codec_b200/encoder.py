@@ -261,10 +261,7 @@ class SpectralEncoder(nn.Module):
         self.output_dim = target_elevation_bins * n_bins
         self._lut_key = None
         self._lut = None
-        self._pipeline = None
-        self._pipeline_key = None
-        self._scan_pipeline = None
-        self._scan_pipeline_key = None
+        self._pipelines = {}    # name -> (nsc_pipeline handle, (device, chunk, n_buffers))
 
     # ------------------------------------------------------------------ constants
     def _compute_bin_edges(self, alpha: torch.Tensor) -> torch.Tensor:
@@ -377,21 +374,15 @@ class SpectralEncoder(nn.Module):
     def _encode_host_scan(self, a: np.ndarray, dev: torch.device) -> torch.Tensor:
         """One pageable numpy scan -> descriptor on the device through ``nsc_pipeline_encode_scan``
         (pinned staging in pieces overlapped with their DMA, kernel on the current stream)."""
-        lib = _lib.load()
+        index = dev.index if dev.index is not None else torch.cuda.current_device()
         cap = max(1 << 18, int(a.shape[0]))
-        key = (dev.index if dev.index is not None else torch.cuda.current_device(), cap)
-        if self._scan_pipeline is None or self._scan_pipeline_key[0] != key[0] or self._scan_pipeline_key[1] < cap:
-            if self._scan_pipeline is not None:
-                lib.nsc_pipeline_destroy(self._scan_pipeline)
-                self._scan_pipeline = None
-            h = C.c_void_p()
-            _lib.check(lib.nsc_pipeline_create(cap, 3, key[0], C.byref(h)), "nsc_pipeline_create")
-            self._scan_pipeline, self._scan_pipeline_key = h, key
+        pl = self._cached_pipeline("scan", (index, cap, 3), lambda k: k[0] == index and k[1] >= cap)
         out = torch.empty((self.output_dim,), dtype=torch.float32, device=dev)
         p = self._params()
         lut = self.freq_to_bin()
-        st = lib.nsc_pipeline_encode_scan(self._scan_pipeline, a.ctypes.data, a.shape[1], a.shape[0], C.byref(p),
-                                          lut.ctypes.data, out.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+        st = _lib.load().nsc_pipeline_encode_scan(pl, a.ctypes.data, a.shape[1], a.shape[0], C.byref(p),
+                                                  lut.ctypes.data, out.data_ptr(),
+                                                  torch.cuda.current_stream(dev).cuda_stream)
         _lib.check(st, "nsc_pipeline_encode_scan")
         return out
 
@@ -451,41 +442,43 @@ class SpectralEncoder(nn.Module):
         biggest = int(np.diff(offs).max())
         chunk = max(int(max_chunk_points), biggest)
         key = (dev.index if dev.index is not None else torch.cuda.current_device(), chunk, n_buffers)
-        if self._pipeline_key != key:
-            self._close_pipeline()
-            h = C.c_void_p()
-            _lib.check(lib.nsc_pipeline_create(chunk, n_buffers, key[0], C.byref(h)), "nsc_pipeline_create")
-            self._pipeline, self._pipeline_key = h, key
+        pl = self._cached_pipeline("batch", key, key.__eq__)
         p = self._params()
         lut = self.freq_to_bin()
         if arrs is not None:   # separate host arrays: gathered into pinned staging inside the library
             ptrs = (C.c_void_p * n_scans)(*[a.ctypes.data for a in arrs])
             counts = np.diff(offs)
-            args = (self._pipeline, ptrs, counts.ctypes.data, arrs[0].shape[1], n_scans, C.byref(p), lut.ctypes.data)
-            if u16:
-                st = lib.nsc_pipeline_encode_scans_u16(*args, _lib.QUANT_EPSILON, out.ctypes.data)
-                _lib.check(st, "nsc_pipeline_encode_scans_u16")
-            else:
-                st = lib.nsc_pipeline_encode_scans(*args, out.ctypes.data)
-                _lib.check(st, "nsc_pipeline_encode_scans")
-            return out
-        args = (self._pipeline, pts.ctypes.data, pts.shape[1], pts.shape[0], offs.ctypes.data, n_scans, C.byref(p),
-                lut.ctypes.data)
+            name = "nsc_pipeline_encode_scans"
+            args = (pl, ptrs, counts.ctypes.data, arrs[0].shape[1], n_scans, C.byref(p), lut.ctypes.data)
+        else:
+            name = "nsc_pipeline_encode"
+            args = (pl, pts.ctypes.data, pts.shape[1], pts.shape[0], offs.ctypes.data, n_scans, C.byref(p),
+                    lut.ctypes.data)
         if u16:
-            st = lib.nsc_pipeline_encode_u16(*args, _lib.QUANT_EPSILON, out.ctypes.data)
-            _lib.check(st, "nsc_pipeline_encode_u16")
-            return out
-        st = lib.nsc_pipeline_encode(*args, out.ctypes.data)
-        _lib.check(st, "nsc_pipeline_encode")
+            name += "_u16"
+            args += (_lib.QUANT_EPSILON,)
+        _lib.check(getattr(lib, name)(*args, out.ctypes.data), name)
         return out
 
+    def _cached_pipeline(self, name: str, key: Tuple[int, int, int], keep) -> C.c_void_p:
+        """The pipeline cached as ``name``, kept while ``keep(its key)`` holds and otherwise replaced
+        by ``nsc_pipeline_create(chunk, n_buffers, device)`` for ``key = (device, chunk, n_buffers)``."""
+        cached = self._pipelines.get(name)
+        if cached is not None and keep(cached[1]):
+            return cached[0]
+        lib = _lib.load()
+        if cached is not None:
+            del self._pipelines[name]
+            lib.nsc_pipeline_destroy(cached[0])
+        h = C.c_void_p()
+        _lib.check(lib.nsc_pipeline_create(key[1], key[2], key[0], C.byref(h)), "nsc_pipeline_create")
+        self._pipelines[name] = (h, key)
+        return h
+
     def _close_pipeline(self) -> None:
-        if getattr(self, "_pipeline", None) is not None:
-            _lib.load().nsc_pipeline_destroy(self._pipeline)
-            self._pipeline, self._pipeline_key = None, None
-        if getattr(self, "_scan_pipeline", None) is not None:
-            _lib.load().nsc_pipeline_destroy(self._scan_pipeline)
-            self._scan_pipeline, self._scan_pipeline_key = None, None
+        pipelines = getattr(self, "_pipelines", {})
+        while pipelines:
+            _lib.load().nsc_pipeline_destroy(pipelines.popitem()[1][0])
 
     def __del__(self):
         try:
