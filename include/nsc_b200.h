@@ -322,6 +322,30 @@ int nsc_wasserstein_query(const float* d_query_hists, int n_queries, const float
                           float* d_distances, int top_k, int64_t* d_top_idx, float* d_top_dist,
                           int32_t* d_top_count, void* d_workspace, size_t workspace_bytes, void* stream);
 
+/* The same database kept as uint16 rows: a quarter of the float32 database's bytes, and half the
+ * bytes the distance pass streams per row.
+ * nsc_wasserstein_cdf_u16 turns uint16 histogram rows (the wire format of nsc_quantize_histograms /
+ * nsc_encode_batch_u16) into uint16 CDF rows in units of 1/65535. With S_i the integer prefix sums of
+ * a row and T = S_{n_bins-1}:
+ *   T = 65535 (every row the quantiser or the encoder writes): the stored row is S_i, exact.
+ *   T = 0 (an empty scan's row): the stored row is all zero. The query reads a stored row whose last
+ *         element is 0 as the uniform CDF (i + 1) / n_bins -- what dequantize yields for a zero row --
+ *         computed in the kernel, not rounded into storage.
+ *   any other T: round-half-even(65535 * S_i / T) in 64-bit integers, at most 0.5 / 65535 per CDF
+ *         element from the CDF of the dequantised float row.
+ * d_rows, d_cdf16: uint16[n_rows * n_bins]; n_bins <= 1024. Status codes and their order are those of
+ * nsc_wasserstein_cdf.
+ * nsc_wasserstein_query_u16 is nsc_wasserstein_query over d_db_cdf16 from nsc_wasserstein_cdf_u16
+ * (queries stay float32 histograms): the same validation order and codes, the same workspace, top-K
+ * selection and spatial filter. Its distances equal those of the float32 database of the dequantised
+ * rows to float32 rounding (the sums run in counts and are scaled by 1/65535 once per row). */
+int nsc_wasserstein_cdf_u16(const uint16_t* d_rows, int64_t n_rows, int n_bins, uint16_t* d_cdf16, void* stream);
+int nsc_wasserstein_query_u16(const float* d_query_hists, int n_queries, const uint16_t* d_db_cdf16,
+                              int64_t n_db, int n_bins, float epsilon, const double* d_db_xyz,
+                              const double* d_query_xyz, double min_spatial_distance,
+                              float* d_distances, int top_k, int64_t* d_top_idx, float* d_top_dist,
+                              int32_t* d_top_count, void* d_workspace, size_t workspace_bytes, void* stream);
+
 /* ---- descriptor wire format (SURVEY.md 8(f), fourth "next" row) --------------------------- */
 /* Replaces HistogramQuantizer.quantize / dequantize (reference src/encoding/quantization.py
  * :131-167, :169-192) for n_rows rows at once and any row length <= 4096 (the reference class is

@@ -99,9 +99,64 @@ cdf_rows_kernel(const float* __restrict__ hists, long long n, int n_bins, float 
     }
 }
 
+// uint16 rows -> uint16 CDF rows in units of 1/65535, one warp per row: an integer prefix scan S
+// (lane l owns the contiguous elements [l*per, (l+1)*per), like row_cdf) and the total T = S[n-1].
+// T = 65535 (every quantised row): S itself, exact. T = 0: zeros (the distance pass reads them as
+// the uniform CDF). Any other T: round-half-even(65535 S / T) in 64-bit integers.
+__global__ void __launch_bounds__(kRThreads)
+cdf16_rows_kernel(const unsigned short* __restrict__ rows, long long n, int n_bins,
+                  unsigned short* __restrict__ cdfs) {
+    extern __shared__ unsigned short smem16[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int per = (n_bins + 31) / 32;
+    unsigned short* row_s = smem16 + warp * (per * 32);
+    const long long n_warps = (long long)gridDim.x * kRWarps;
+    for (long long r = (long long)blockIdx.x * kRWarps + warp; r < n; r += n_warps) {
+        const unsigned short* src = rows + r * n_bins;
+        for (int e = lane; e < per * 32; e += 32) row_s[e] = e < n_bins ? __ldcs(src + e) : 0;
+        __syncwarp();
+        unsigned s[kMaxPerLane];
+        unsigned run = 0;
+#pragma unroll
+        for (int i = 0; i < kMaxPerLane; ++i)
+            if (i < per) {
+                run += row_s[lane * per + i];
+                s[i] = run;
+            }
+        unsigned incl = run;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const unsigned o = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= d) incl += o;
+        }
+        const unsigned offset = incl - run;
+        const unsigned total = __shfl_sync(0xffffffffu, incl, 31);
+        __syncwarp();
+#pragma unroll
+        for (int i = 0; i < kMaxPerLane; ++i)
+            if (i < per) {
+                unsigned v = s[i] + offset;
+                if (total == 0) {
+                    v = 0;
+                } else if (total != 65535u) {
+                    const unsigned long long num = 65535ull * v;
+                    unsigned long long qt = num / total;
+                    const unsigned long long rem = num - qt * total;
+                    if (2 * rem > total || (2 * rem == total && (qt & 1))) ++qt;
+                    v = (unsigned)qt;
+                }
+                row_s[lane * per + i] = (unsigned short)v;
+            }
+        __syncwarp();
+        unsigned short* dst = cdfs + r * n_bins;
+        for (int e = lane; e < n_bins; e += 32) dst[e] = row_s[e];
+        __syncwarp();
+    }
+}
+
 struct QueryArgs {
     const float* queries;     // Q x n_bins histograms
-    const float* db_cdfs;     // N x n_bins
+    const void* db_cdfs;      // N x n_bins: float32 CDF rows, or uint16 rows in units of 1/65535
     const double* db_xyz;     // N x 3 or null
     const double* query_xyz;  // Q x 3 or null
     double min_dist;
@@ -114,40 +169,55 @@ struct QueryArgs {
 
 // CDF rows per warp ring (one fewer in flight): 4 when two CTAs per SM still fit, else 3
 
-__device__ __forceinline__ void cp_async4(float* dst, const float* src) {
+__device__ __forceinline__ void cp_async4(void* dst, const void* src) {
     const unsigned d = (unsigned)__cvta_generic_to_shared(dst);
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(d), "l"(src) : "memory");
 }
-__device__ __forceinline__ void cp_async16(float* dst, const float* src) {
+__device__ __forceinline__ void cp_async16(void* dst, const void* src) {
     const unsigned d = (unsigned)__cvta_generic_to_shared(dst);
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(src) : "memory");
 }
 
 // PER = elements per lane (n_bins <= 32 * PER); PER = 25 is the 800-D descriptor.
-template <int PER, int kRowStages>
+// T = float: CDF rows of nsc_wasserstein_cdf. T = unsigned short: rows of nsc_wasserstein_cdf_u16 in
+// units of 1/65535 (counts). The uint16 instantiation works in counts: each query CDF is scaled by
+// 65535 once when it is staged, each database element converts to float exactly, and the sum of a
+// row is scaled back by 1/65535 once.
+template <typename T, int PER, int kRowStages>
 __global__ void __launch_bounds__(kRThreads)
 wasserstein_kernel(const __grid_constant__ QueryArgs a) {
+    constexpr bool kCounts = sizeof(T) == 2;
     extern __shared__ __align__(16) float smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     constexpr int padded = PER * 32;
     float* qcdf = smem;                                           // Q x padded
-    float* ring = smem + a.n_queries * padded + warp * (kRowStages * padded);
+    T* ring = reinterpret_cast<T*>(smem + a.n_queries * padded) + warp * (kRowStages * padded);
     const long long n_warps = (long long)gridDim.x * kRWarps;
     const long long r0 = (long long)blockIdx.x * kRWarps + warp;
-    const bool vec = (a.n_bins & 3) == 0;
+    // 16-byte copies where every row starts on a 16-byte boundary. uint16 rows: 4-byte copies of
+    // element pairs where rows start on 4-byte boundaries; an odd n_bins (or an unaligned base) has
+    // no cp.async size, so those rows go through plain loads (synchronous, still in ring order).
+    const bool vec = kCounts ? (a.n_bins & 7) == 0 && (reinterpret_cast<uintptr_t>(a.db_cdfs) & 15) == 0
+                             : (a.n_bins & 3) == 0;
+    const bool pairs = kCounts && (a.n_bins & 1) == 0 && (reinterpret_cast<uintptr_t>(a.db_cdfs) & 3) == 0;
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // the selection may become resident now
     if (a.n_bins < padded)
         for (int s = 0; s < kRowStages; ++s)
-            for (int e = a.n_bins + lane; e < padded; e += 32) ring[s * padded + e] = 0.0f;
+            for (int e = a.n_bins + lane; e < padded; e += 32) ring[s * padded + e] = T(0);
     __syncwarp();
     auto issue = [&](long long r, int slot) {
         if (r < a.n_db) {
-            const float* src = a.db_cdfs + r * a.n_bins;
-            float* dst = ring + slot * padded;
+            const T* src = static_cast<const T*>(a.db_cdfs) + r * a.n_bins;
+            T* dst = ring + slot * padded;
+            constexpr int kVec = 16 / sizeof(T);
             if (vec) {
-                for (int e = lane * 4; e < a.n_bins; e += 128) cp_async16(dst + e, src + e);
-            } else {
+                for (int e = lane * kVec; e < a.n_bins; e += 32 * kVec) cp_async16(dst + e, src + e);
+            } else if (!kCounts) {
                 for (int e = lane; e < a.n_bins; e += 32) cp_async4(dst + e, src + e);
+            } else if (pairs) {
+                for (int e = lane * 2; e < a.n_bins; e += 64) cp_async4(dst + e, src + e);
+            } else {
+                for (int e = lane; e < a.n_bins; e += 32) dst[e] = src[e];
             }
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
@@ -156,20 +226,27 @@ wasserstein_kernel(const __grid_constant__ QueryArgs a) {
 #pragma unroll
     for (int s = 0; s < kRowStages - 1; ++s) issue(r0 + s * n_warps, s);
     // query CDFs (wasserstein.py:152-154,165), one warp per query, staged through the ring slot
-    // the prologue above left free (its padding lanes stay zero)
+    // the prologue above left free (its padding lanes stay zero). A uint16 ring slot is too small
+    // for a float row, so there the query is staged in its own qcdf row: row_cdf reads the whole row
+    // into registers before the warp overwrites it.
     {
-        float* stage = ring + (kRowStages - 1) * padded;
+        float* stage = reinterpret_cast<float*>(ring + (kRowStages - 1) * padded);
         for (int q = warp; q < a.n_queries; q += kRWarps) {
+            if (kCounts) stage = qcdf + q * padded;
             for (int e = lane; e < padded; e += 32) stage[e] = e < a.n_bins ? a.queries[(long long)q * a.n_bins + e] : 0.0f;
             __syncwarp();
             float c[kMaxPerLane];
             row_cdf<1>(stage, a.n_bins, PER, a.eps, lane, c);
+            if (kCounts) __syncwarp();
 #pragma unroll
             for (int i = 0; i < PER; ++i)      // padding lanes hold 0, like the padding of the database rows
-                qcdf[q * padded + lane * PER + i] = lane * PER + i < a.n_bins ? c[i] : 0.0f;
+                qcdf[q * padded + lane * PER + i] = lane * PER + i < a.n_bins ? (kCounts ? c[i] * 65535.0f : c[i]) : 0.0f;
             __syncwarp();
         }
     }
+    // an all-zero uint16 row (an empty scan's wire row) stands for the uniform CDF (i + 1) / n_bins,
+    // which dequantize yields for it: 65535 (i + 1) / n_bins counts, rounded once
+    const double uniform_step = kCounts ? 65535.0 / a.n_bins : 0.0;
     __syncthreads();
     const bool spatial = a.db_xyz != nullptr && a.query_xyz != nullptr;
     int slot = 0;
@@ -180,10 +257,22 @@ wasserstein_kernel(const __grid_constant__ QueryArgs a) {
         issue(r + (kRowStages - 1) * n_warps, (slot + kRowStages - 1) % kRowStages);
         asm volatile("cp.async.wait_group %0;" ::"n"(kRowStages - 1) : "memory");
         __syncwarp();
-        const float* row_s = ring + slot * padded + lane * PER;
+        const T* row_s = ring + slot * padded + lane * PER;
         float c[PER];
 #pragma unroll
-        for (int i = 0; i < PER; ++i) c[i] = row_s[i];
+        for (int i = 0; i < PER; ++i) {
+            if (kCounts)      // 2^23 + c as float bits, minus 2^23: exact for 0 <= c <= 65535
+                c[i] = __uint_as_float(0x4B000000u | (unsigned)row_s[i]) - 8388608.0f;
+            else
+                c[i] = row_s[i];
+        }
+        if (kCounts && ring[slot * padded + a.n_bins - 1] == T(0)) {   // CDF rows end on 0 only when all zero
+#pragma unroll
+            for (int i = 0; i < PER; ++i) {
+                const int e = lane * PER + i;
+                c[i] = e < a.n_bins ? (float)((e + 1) * uniform_step) : 0.0f;
+            }
+        }
         double px = 0, py = 0, pz = 0;
         if (spatial && lane == 0) { px = a.db_xyz[3 * r]; py = a.db_xyz[3 * r + 1]; pz = a.db_xyz[3 * r + 2]; }
 #pragma unroll
@@ -198,6 +287,7 @@ wasserstein_kernel(const __grid_constant__ QueryArgs a) {
             }
             if (PER & 1) d0 += fabsf(c[PER - 1] - qc[PER - 1]);
             float d = warp_sum(d0 + d1);
+            if (kCounts) d *= 1.0f / 65535.0f;
             if (lane == 0) {
                 if (spatial) {   // two_stage_retrieval.py:160-164: skip keyframes closer than the threshold
                     const double dx = px - a.query_xyz[3 * q], dy = py - a.query_xyz[3 * q + 1],
@@ -623,6 +713,23 @@ int nsc_wasserstein_cdf(const float* d_hists, int64_t n_rows, int n_bins, float 
     return record_cuda(cudaGetLastError());
 }
 
+int nsc_wasserstein_cdf_u16(const uint16_t* d_rows, int64_t n_rows, int n_bins, uint16_t* d_cdf16, void* stream) {
+    if (n_rows < 0) return NSC_ERR_BAD_COUNT;
+    if (n_bins < 1 || n_bins > 32 * kMaxPerLane) return NSC_ERR_BAD_PARAMS;
+    if (n_rows == 0) return NSC_OK;
+    if (!d_rows || !d_cdf16) return NSC_ERR_NULL_POINTER;
+    int sms = 0;
+    int st = sm_count(&sms);
+    if (st != NSC_OK) return st;
+    const int padded = ((n_bins + 31) / 32) * 32;
+    const size_t smem = (size_t)kRWarps * padded * 2;
+    long long grid = (n_rows + kRWarps - 1) / kRWarps;
+    if (grid > (long long)sms * 8) grid = (long long)sms * 8;
+    cdf16_rows_kernel<<<(int)grid, kRThreads, smem, (cudaStream_t)stream>>>(
+        reinterpret_cast<const unsigned short*>(d_rows), n_rows, n_bins, reinterpret_cast<unsigned short*>(d_cdf16));
+    return record_cuda(cudaGetLastError());
+}
+
 constexpr int kMaxDistGrid = 1024;     // CTAs of the distance pass (bounds the warp-minima rows of the workspace)
 
 size_t nsc_wasserstein_workspace_bytes(int n_queries) {
@@ -631,11 +738,17 @@ size_t nsc_wasserstein_workspace_bytes(int n_queries) {
     return (size_t)n_queries * per_query + 256;
 }
 
-int nsc_wasserstein_query(const float* d_query_hists, int n_queries, const float* d_db_cdfs,
-                          int64_t n_db, int n_bins, float epsilon, const double* d_db_xyz,
-                          const double* d_query_xyz, double min_spatial_distance,
-                          float* d_distances, int top_k, int64_t* d_top_idx, float* d_top_dist,
-                          int32_t* d_top_count, void* d_workspace, size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+namespace {
+
+// nsc_wasserstein_query and nsc_wasserstein_query_u16: T is the element type of the database rows
+template <typename T>
+int wasserstein_query(const float* d_query_hists, int n_queries, const T* d_db_cdfs,
+                      int64_t n_db, int n_bins, float epsilon, const double* d_db_xyz,
+                      const double* d_query_xyz, double min_spatial_distance,
+                      float* d_distances, int top_k, int64_t* d_top_idx, float* d_top_dist,
+                      int32_t* d_top_count, void* d_workspace, size_t workspace_bytes, void* stream) {
     if (n_queries < 0 || n_db < 0 || top_k < 0) return NSC_ERR_BAD_COUNT;
     if (n_bins < 1 || n_bins > 32 * kMaxPerLane || top_k > kTopThreads) return NSC_ERR_BAD_PARAMS;
     if (n_db >= (1ll << 32)) return NSC_ERR_BAD_COUNT;
@@ -666,14 +779,16 @@ int nsc_wasserstein_query(const float* d_query_hists, int n_queries, const float
         cudaError_t e = cudaGetDevice(&dev);
         if (e == cudaSuccess) e = cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
         if (e != cudaSuccess) return record_cuda(e);
-        auto smem_for = [&](int nq, int stages) { return (size_t)(nq + kRWarps * stages) * per * 32 * 4; };
+        auto smem_for = [&](int nq, int stages) {
+            return (size_t)nq * per * 32 * 4 + (size_t)kRWarps * stages * per * 32 * sizeof(T);
+        };
         const int stages = 2 * (smem_for(q_max, 4) + 1024) <= (size_t)smem_optin ? 4 : 3;   // keep two CTAs per SM
         if (stages == 4)
-            kern = per == 8 ? wasserstein_kernel<8, 4> : per == 16 ? wasserstein_kernel<16, 4>
-                   : per == 25 ? wasserstein_kernel<25, 4> : wasserstein_kernel<32, 4>;
+            kern = per == 8 ? wasserstein_kernel<T, 8, 4> : per == 16 ? wasserstein_kernel<T, 16, 4>
+                   : per == 25 ? wasserstein_kernel<T, 25, 4> : wasserstein_kernel<T, 32, 4>;
         else
-            kern = per == 8 ? wasserstein_kernel<8, 3> : per == 16 ? wasserstein_kernel<16, 3>
-                   : per == 25 ? wasserstein_kernel<25, 3> : wasserstein_kernel<32, 3>;
+            kern = per == 8 ? wasserstein_kernel<T, 8, 3> : per == 16 ? wasserstein_kernel<T, 16, 3>
+                   : per == 25 ? wasserstein_kernel<T, 25, 3> : wasserstein_kernel<T, 32, 3>;
         const size_t smem_max = smem_for(q_max, stages);
         e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
         if (e != cudaSuccess) return record_cuda(e);
@@ -742,6 +857,30 @@ int nsc_wasserstein_query(const float* d_query_hists, int n_queries, const float
         return record_cuda(cudaGetLastError());
     }
     return NSC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int nsc_wasserstein_query(const float* d_query_hists, int n_queries, const float* d_db_cdfs,
+                          int64_t n_db, int n_bins, float epsilon, const double* d_db_xyz,
+                          const double* d_query_xyz, double min_spatial_distance,
+                          float* d_distances, int top_k, int64_t* d_top_idx, float* d_top_dist,
+                          int32_t* d_top_count, void* d_workspace, size_t workspace_bytes, void* stream) {
+    return wasserstein_query(d_query_hists, n_queries, d_db_cdfs, n_db, n_bins, epsilon, d_db_xyz, d_query_xyz,
+                             min_spatial_distance, d_distances, top_k, d_top_idx, d_top_dist, d_top_count,
+                             d_workspace, workspace_bytes, stream);
+}
+
+int nsc_wasserstein_query_u16(const float* d_query_hists, int n_queries, const uint16_t* d_db_cdf16,
+                              int64_t n_db, int n_bins, float epsilon, const double* d_db_xyz,
+                              const double* d_query_xyz, double min_spatial_distance,
+                              float* d_distances, int top_k, int64_t* d_top_idx, float* d_top_dist,
+                              int32_t* d_top_count, void* d_workspace, size_t workspace_bytes, void* stream) {
+    return wasserstein_query(d_query_hists, n_queries, reinterpret_cast<const unsigned short*>(d_db_cdf16), n_db,
+                             n_bins, epsilon, d_db_xyz, d_query_xyz, min_spatial_distance, d_distances, top_k,
+                             d_top_idx, d_top_dist, d_top_count, d_workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

@@ -9,6 +9,14 @@ of by one ``torch.cat`` per keyframe. ``query_batch`` answers many queries in on
 the database and takes the spatial exclusion of ``TwoStageRetrieval._global_retrieval``
 (``src/retrieval/two_stage_retrieval.py:145-202``) as optional positions.
 
+``database_dtype=torch.uint16`` keeps the database in the ``HistogramQuantizer`` wire format
+instead: the rows as uint16 and their CDFs as uint16 in units of 1/65535
+(``nsc_wasserstein_cdf_u16`` / ``nsc_wasserstein_query_u16``), a quarter of the float32
+database's memory. Its distances are those of the float32 database of the dequantised rows. The
+default stays float32, which keeps the unquantised distances. Rows and queries of either dtype go
+into either database: uint16 rows are dequantised on the device, float rows going into a uint16
+database are quantised on the device, both with the retriever's ``epsilon``.
+
 All arithmetic runs in ``libnsc_b200.so`` (``nsc_wasserstein_cdf`` / ``nsc_wasserstein_query``);
 there is no CPU path.
 """
@@ -25,7 +33,10 @@ MAX_TOP_K = 1024
 
 
 class WassersteinRetriever:
-    def __init__(self, use_torch: bool = True, device: str = "cuda", epsilon: float = 1e-8):
+    def __init__(self, use_torch: bool = True, device: str = "cuda", epsilon: float = 1e-8,
+                 database_dtype: torch.dtype = torch.float32):
+        if database_dtype not in (torch.float32, torch.uint16):
+            raise ValueError("database_dtype must be torch.float32 or torch.uint16")
         dev = torch.device(device)
         if dev.type != "cuda":
             raise RuntimeError("WassersteinRetriever: no CPU implementation; pass a CUDA device")
@@ -33,6 +44,7 @@ class WassersteinRetriever:
         self.use_torch = use_torch      # kept for signature compatibility; always the CUDA path
         self.device = dev
         self.epsilon = float(epsilon)
+        self.database_dtype = database_dtype
         self._hists: Optional[torch.Tensor] = None      # capacity x n_bins
         self._cdfs: Optional[torch.Tensor] = None
         self._xyz: Optional[torch.Tensor] = None        # capacity x 3 float64 (NaN = unknown)
@@ -55,8 +67,8 @@ class WassersteinRetriever:
         if rows <= cap:
             return
         new_cap = max(rows, 2 * cap, 1024)
-        hists = torch.empty((new_cap, n_bins), dtype=torch.float32, device=self.device)
-        cdfs = torch.empty((new_cap, n_bins), dtype=torch.float32, device=self.device)
+        hists = torch.empty((new_cap, n_bins), dtype=self.database_dtype, device=self.device)
+        cdfs = torch.empty((new_cap, n_bins), dtype=self.database_dtype, device=self.device)
         xyz = torch.full((new_cap, 3), float("nan"), dtype=torch.float64, device=self.device)
         if self.database_size:
             hists[: self.database_size] = self._hists[: self.database_size]
@@ -64,32 +76,60 @@ class WassersteinRetriever:
             xyz[: self.database_size] = self._xyz[: self.database_size]
         self._hists, self._cdfs, self._xyz = hists, cdfs, xyz
 
-    def add_to_database(self, histograms: Union[np.ndarray, torch.Tensor],
-                        positions: Union[np.ndarray, torch.Tensor, None] = None) -> None:
-        """Append ``(n, n_bins)`` histograms (reference :300-326); ``positions`` are optional
-        ``(n, 3)`` keyframe positions (``pose[:3, 3]``) for the spatial filter of ``query_batch``."""
-        lib = _lib.load()
-        if isinstance(histograms, np.ndarray):
-            histograms = torch.from_numpy(np.ascontiguousarray(histograms, np.float32))
-        h = histograms.detach().to(self.device, torch.float32)
+    def _rows(self, x: Union[np.ndarray, torch.Tensor], what: str) -> torch.Tensor:
+        """``(n, n_bins)`` rows on the device: uint16 rows stay uint16, anything else is float32."""
+        if isinstance(x, np.ndarray):
+            x = torch.from_numpy(np.ascontiguousarray(x, np.uint16 if x.dtype == np.uint16 else np.float32))
+        h = x.detach().to(self.device, torch.uint16 if x.dtype == torch.uint16 else torch.float32)
         if h.dim() == 1:
             h = h.unsqueeze(0)
         if h.dim() != 2:
-            raise ValueError("histograms must have shape (n, n_bins)")
+            raise ValueError(f"{what} must have shape (n, n_bins)")
+        return h
+
+    def _convert(self, rows: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+        """float32 rows -> uint16 ``out`` (quantise) or uint16 rows -> float32 ``out`` (dequantise)."""
+        lib = _lib.load()
+        rows = rows.contiguous()
+        name = "nsc_quantize_histograms" if out.dtype == torch.uint16 else "nsc_dequantize_histograms"
+        with torch.cuda.device(self.device):
+            st = getattr(lib, name)(rows.data_ptr(), rows.shape[0], rows.shape[1], self.epsilon, out.data_ptr(),
+                                    torch.cuda.current_stream(self.device).cuda_stream)
+        _lib.check(st, name)
+        return out
+
+    def add_to_database(self, histograms: Union[np.ndarray, torch.Tensor],
+                        positions: Union[np.ndarray, torch.Tensor, None] = None) -> None:
+        """Append ``(n, n_bins)`` histograms (reference :300-326); ``positions`` are optional
+        ``(n, 3)`` keyframe positions (``pose[:3, 3]``) for the spatial filter of ``query_batch``.
+        float rows or uint16 wire rows; they are converted to the database's dtype."""
+        lib = _lib.load()
+        h = self._rows(histograms, "histograms")
         n, n_bins = h.shape
         if n == 0:
             return
         lo = self.database_size
         self._reserve(lo + n, n_bins)
-        self._hists[lo: lo + n] = h
+        if h.dtype == self.database_dtype:
+            self._hists[lo: lo + n] = h
+        elif h.dtype == torch.uint16:
+            self._hists[lo: lo + n] = self._convert(h, torch.empty(h.shape, dtype=torch.float32, device=self.device))
+        else:
+            self._convert(h, self._hists[lo: lo + n])
         if positions is not None:
             p = torch.as_tensor(positions, dtype=torch.float64).reshape(n, 3)
             self._xyz[lo: lo + n] = p.to(self.device)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
         with torch.cuda.device(self.device):
-            st = lib.nsc_wasserstein_cdf(self._hists[lo: lo + n].data_ptr(), n, n_bins, self.epsilon,
-                                         self._cdfs[lo: lo + n].data_ptr(),
-                                         torch.cuda.current_stream(self.device).cuda_stream)
-        _lib.check(st, "nsc_wasserstein_cdf")
+            if self.database_dtype == torch.uint16:
+                name = "nsc_wasserstein_cdf_u16"
+                st = lib.nsc_wasserstein_cdf_u16(self._hists[lo: lo + n].data_ptr(), n, n_bins,
+                                                 self._cdfs[lo: lo + n].data_ptr(), stream)
+            else:
+                name = "nsc_wasserstein_cdf"
+                st = lib.nsc_wasserstein_cdf(self._hists[lo: lo + n].data_ptr(), n, n_bins, self.epsilon,
+                                             self._cdfs[lo: lo + n].data_ptr(), stream)
+        _lib.check(st, name)
         self.database_size = lo + n
 
     def clear_database(self) -> None:
@@ -104,18 +144,17 @@ class WassersteinRetriever:
         counts (Q,) int32)`` on the device, ``k = min(top_k, database_size)``; rows are sorted by
         ascending distance and padded with -1 / +inf beyond ``counts[q]`` (only when the spatial
         filter leaves fewer than ``k`` candidates). With ``return_distances`` the full
-        ``(Q, database_size)`` distance matrix is returned as a fourth element."""
+        ``(Q, database_size)`` distance matrix is returned as a fourth element. Queries are float
+        rows or uint16 wire rows (dequantised on the device first)."""
         lib = _lib.load()
-        if isinstance(query_hists, np.ndarray):
-            query_hists = torch.from_numpy(np.ascontiguousarray(query_hists, np.float32))
-        q = query_hists.detach().to(self.device, torch.float32)
-        if q.dim() == 1:
-            q = q.unsqueeze(0)
-        q = q.contiguous()
+        q = self._rows(query_hists, "queries")
         nq = q.shape[0]
         n = self.database_size
         if n and q.shape[1] != self._hists.shape[1]:
             raise ValueError("query and database bin counts differ")
+        if q.dtype == torch.uint16:
+            q = self._convert(q, torch.empty(q.shape, dtype=torch.float32, device=self.device))
+        q = q.contiguous()
         k = min(int(top_k), n)
         # The select kernel holds its candidates in one CTA (k <= 1024). Larger k -- the reference's
         # TwoStageRetrieval._global_retrieval asks for every keyframe, top_k = len(keyframes) -- takes
@@ -135,15 +174,16 @@ class WassersteinRetriever:
             need = int(lib.nsc_wasserstein_workspace_bytes(nq))
             if self._ws is None or self._ws.numel() < need:
                 self._ws = torch.zeros(need, dtype=torch.uint8, device=self.device)
+            name = "nsc_wasserstein_query_u16" if self.database_dtype == torch.uint16 else "nsc_wasserstein_query"
             with torch.cuda.device(self.device):
-                st = lib.nsc_wasserstein_query(
+                st = getattr(lib, name)(
                     q.data_ptr(), nq, self._cdfs.data_ptr(), n, q.shape[1], self.epsilon,
                     self._xyz.data_ptr() if use_xyz else None, qp.data_ptr() if use_xyz else None,
                     float(spatial_filter_distance), dist.data_ptr(), k_kernel,
                     idx.data_ptr() if k_kernel else None, top.data_ptr() if k_kernel else None,
                     cnt.data_ptr() if k_kernel else None, self._ws.data_ptr(), self._ws.numel(),
                     torch.cuda.current_stream(self.device).cuda_stream)
-            _lib.check(st, "nsc_wasserstein_query")
+            _lib.check(st, name)
             if k > MAX_TOP_K:
                 sd, si = torch.sort(dist, dim=1, stable=True)
                 top, idx = sd[:, :k].contiguous(), si[:, :k].contiguous()
