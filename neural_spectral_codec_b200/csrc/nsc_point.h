@@ -13,7 +13,11 @@
 //                sqrt is taken once per pixel after the scatter.
 //   column  = floor(((atan2(y,x) + pi) mod 2pi) / 2pi * 360)                       (:166-167,:194)
 //             -> octant-reduced odd polynomial of atan in column units, error 3e-7 rad; the
-//                north star excuses points within 1e-5 rad of a column edge.
+//                north star excuses points within 1e-5 rad of a column edge. The reduction is
+//                scale-invariant for every x, y with |x|, |y| < 2^64 -- signed zeros and
+//                subnormals included, so points on or next to the vertical axis get the
+//                reference's column -- which covers every point whose s is finite, i.e. every
+//                point that can be kept. Larger or non-finite x, y still land in [0, 360].
 //   row     = floor((atan2(z, sqrt(x*x+y*y)) - el_min) / (el_max - el_min) * E), clipped (:170,:186)
 //             -> u = z / rho clamped to the field of view, odd polynomial of atan scaled to
 //                row units (kRowPoly), or a binary search of z|z| against tan^2 thresholds
@@ -103,11 +107,37 @@ NSC_HD uint32_t floor_biased(float v, float add) {
 #endif
 }
 
+// Octant reduction t = min(|x|,|y|) / max(|x|,|y|) with x and y first scaled by 2^32, which is
+// exact: a nonzero magnitude below 2^64 (every x, y of a point whose s is finite) becomes a normal
+// number in [2^-117, 2^96), where rcp.approx.ftz flushes neither its input nor its result, so t is
+// the same for (x, y) and (2^k x, 2^k y), subnormals included. The floor only turns x = y = 0 into
+// t = 0 (instead of 0 * Inf); it is below every scaled nonzero magnitude.
+constexpr float kOctScale = 0x1p32f;
+constexpr float kOctFloor = 0x1p-126f;
+
+// |x| * 2^32 and |y| * 2^32; on the device one packed multiply (x and y of a loaded point sit in
+// an aligned register pair).
+NSC_HD void scaled_abs(float x, float y, float& ax, float& ay) {
+#if defined(__CUDA_ARCH__)
+    uint64_t v, k;
+    asm("mov.b64 %0, {%1, %2};" : "=l"(v) : "f"(x), "f"(y));
+    asm("mov.b64 %0, {%1, %1};" : "=l"(k) : "f"(kOctScale));
+    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(v) : "l"(v), "l"(k));
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(ax), "=f"(ay) : "l"(v));
+    ax = fabsf(ax);
+    ay = fabsf(ay);
+#else
+    ax = fabsf(x * kOctScale);
+    ay = fabsf(y * kOctScale);
+#endif
+}
+
 // Column + kFloorBias, column in [0, 360]; 360 only for azimuth == 2*pi exactly, which the
 // reference wraps to 0 (the kernels keep a 361st column and fold it).
 NSC_HD uint32_t column_biased(float x, float y) {
-    const float ax = fabsf(x), ay = fabsf(y);
-    const float mx = fmaxf(fmaxf(ax, ay), 1e-30f);
+    float ax, ay;
+    scaled_abs(x, y, ax, ay);
+    const float mx = fmaxf(fmaxf(ax, ay), kOctFloor);
     const float mn = fminf(ax, ay);
     const float t = mn * rcp_fast(mx);
     const float t2 = t * t;
@@ -202,9 +232,11 @@ __device__ __forceinline__ void classify2(float xa, float ya, float za, float xb
     const float sb = __fadd_rn(rho2b, __fmul_rn(zb, zb));
     key_a = (sa >= dp.s_lo) ? __float_as_uint(sa) : 0xffffffffu;
     key_b = (sb >= dp.s_lo) ? __float_as_uint(sb) : 0xffffffffu;
-    // column: octant reduction scalar, polynomial packed
-    const float axa = fabsf(xa), aya = fabsf(ya), axb = fabsf(xb), ayb = fabsf(yb);
-    const float ra = rcp_fast(fmaxf(fmaxf(axa, aya), 1e-30f)), rb = rcp_fast(fmaxf(fmaxf(axb, ayb), 1e-30f));
+    // column: octant reduction (scaled as in column_biased) scalar, polynomial packed
+    float axa, aya, axb, ayb;
+    scaled_abs(xa, ya, axa, aya);
+    scaled_abs(xb, yb, axb, ayb);
+    const float ra = rcp_fast(fmaxf(fmaxf(axa, aya), kOctFloor)), rb = rcp_fast(fmaxf(fmaxf(axb, ayb), kOctFloor));
     const uint64_t t = mul2(pack2(fminf(axa, aya), fminf(axb, ayb)), pack2(ra, rb));
     const uint64_t t2 = mul2(t, t);
     uint64_t p = pack2(NSC_COL_C6, NSC_COL_C6);

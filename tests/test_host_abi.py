@@ -184,6 +184,77 @@ def test_row_rules_on_other_fields_of_view(lib, er, rows, mode):
     np.testing.assert_array_equal(col[clear], ocol[clear])
 
 
+def host_classify_cfg(lib, pts, cfg):
+    return host_classify(lib, pts, n_elevation=cfg.n_elevation, el_min_rad=float(cfg.el_min),
+                         el_max_rad=float(cfg.el_max), min_range=cfg.min_range, max_range=cfg.max_range)
+
+
+# (elevation range, rows, min_range, max_range, row rule): both row rules, E = 1 and E = 2
+HOST_CONFIGS = [((-24.8, 2.0), 16, 1.0, 80.0, 0), ((-15.0, 15.0), 16, 1.0, 80.0, 0), ((-60.0, 60.0), 32, 1.0, 80.0, 1),
+                ((-89.0, 89.0), 64, 0.5, 120.0, 1), ((-30.0, 30.0), 1, 2.0, 50.0, 0), ((-30.0, 30.0), 2, 1.0, 80.0, 0)]
+
+
+def host_config(lib, er, rows, lo, hi, mode):
+    cfg = orc.OracleConfig(n_elevation=rows, elevation_range=er, min_range=lo, max_range=hi)
+    p = default_params(lib, n_elevation=rows, el_min_rad=float(cfg.el_min), el_max_rad=float(cfg.el_max))
+    assert lib.nsc_test_row_mode(C.byref(p)) == mode
+    return cfg
+
+
+@pytest.mark.parametrize("er,rows,lo,hi,mode", HOST_CONFIGS)
+def test_near_axis_points_get_the_oracle_pixel(lib, er, rows, lo, hi, mode):
+    """|x|, |y| in [1e-45, 1e-20] with z inside the range limits: points on the vertical axis's
+    doorstep, kept, with the row clamped and the column of atan2(y, x). The octant reduction
+    min(|x|,|y|) / max(|x|,|y|) must not depend on the scale of x and y (a floor of 1e-30 on the
+    denominator once sent these points to arbitrary columns). No row edge is near; points within
+    1e-5 rad of a column edge may take the column across it, every other one the oracle's."""
+    from point_sets import across_edges, near_axis, oracle_pixels
+    cfg = host_config(lib, er, rows, lo, hi, mode)
+    pts = near_axis(np.random.default_rng(rows), 40000, cfg)
+    row, col, keep = host_classify_cfg(lib, pts, cfg)
+    okeep, orow, ocol, _, d_az, d_el = oracle_pixels(pts, cfg)
+    assert okeep.all() and keep.all()
+    assert (d_el > 1e-5).all()
+    np.testing.assert_array_equal(row, orow)
+    clear = d_az > 1e-5
+    assert clear.sum() > 0.5 * len(pts)
+    np.testing.assert_array_equal(col[clear], ocol[clear])
+    _, col_x = across_edges(pts, cfg, orow, ocol)
+    assert ((col == ocol) | (col == col_x))[~clear].all()
+
+
+@pytest.mark.parametrize("er,rows,lo,hi,mode", HOST_CONFIGS)
+def test_axes_and_signed_zeros_match_the_oracle_exactly(lib, er, rows, lo, hi, mode):
+    """Points on the x, y and z axes with +0 and -0 in every coordinate, and the azimuth wrap
+    (x < 0, y = +-0: atan2 = +-pi, the reference's column 0). They sit exactly on column edges,
+    yet the pixel must be the oracle's with no excuse."""
+    from point_sets import oracle_pixels, signed_zeros
+    cfg = host_config(lib, er, rows, lo, hi, mode)
+    pts = signed_zeros(cfg)
+    row, col, keep = host_classify_cfg(lib, pts, cfg)
+    okeep, orow, ocol, _, _, _ = oracle_pixels(pts, cfg)
+    np.testing.assert_array_equal(keep, okeep)
+    assert okeep.sum() >= len(pts) // 2
+    np.testing.assert_array_equal(row[keep], orow[keep])
+    np.testing.assert_array_equal(col[keep], ocol[keep])
+
+
+@pytest.mark.parametrize("er,rows,lo,hi,mode", HOST_CONFIGS)
+def test_adversarial_coordinates_keep_like_the_oracle_and_stay_in_the_image(lib, er, rows, lo, hi, mode):
+    """NaN, +-Inf, subnormals, +-1e38 and coordinates whose squares overflow, alone in one
+    coordinate of in-range points and in every triple: the keep/drop decision is the oracle's and
+    every kept point gets 0 <= row < E, 0 <= column < 360."""
+    from point_sets import adversarial, oracle_pixels
+    cfg = host_config(lib, er, rows, lo, hi, mode)
+    pts = adversarial(np.random.default_rng(7), 200, cfg)
+    row, col, keep = host_classify_cfg(lib, pts, cfg)
+    okeep = oracle_pixels(pts, cfg)[0]
+    np.testing.assert_array_equal(keep, okeep)
+    assert 0 < keep.sum() < len(pts)
+    assert ((row[keep] >= 0) & (row[keep] < rows)).all()
+    assert ((col[keep] >= 0) & (col[keep] < 360)).all()
+
+
 @pytest.mark.parametrize("lo,hi", [(0.5, 120.0), (2.0, 50.0), (0.0, 30.0), (1.0, 80.0)])
 def test_keep_drop_is_exact_for_other_range_limits(lib, lo, hi):
     """The float32 thresholds on s are derived per (min_range, max_range); the keep/drop decision
