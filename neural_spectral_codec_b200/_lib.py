@@ -109,7 +109,7 @@ TUNE_LIB_PATH = os.path.join(_HERE, "libnsc_b200_tune.so")
 def build(verbose: bool = False, tuning: bool = True) -> str:
     """Compile the CUDA sources for sm_100a into ``libnsc_b200.so`` (in-tree), and -- for the
     A/B tools and the bit-identity tests -- the tuning build ``libnsc_b200_tune.so``
-    (``-DNSC_TUNING``: the only build that reads NSC_FEED / NSC_SPLIT / NSC_WS from the
+    (``-DNSC_TUNING``: the only build that reads NSC_SPLIT / NSC_WS / NSC_TAILSPLIT from the
     environment; ``-DNSC_SEL_CAP=128``: a small candidate list, so that tests reach the overflow
     path of the retrieval selection; selected with ``NSC_LIB=<path>``)."""
     cmds = [["make", "-C", CSRC, "-j4"]]

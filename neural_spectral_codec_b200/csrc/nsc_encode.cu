@@ -6,10 +6,9 @@
 //                               per SM, a TMA producer thread, 24 stream warps, 7 tail warps, two
 //                               images; see the comment above it
 //   encode_points_kernel        generic: 2 x 512-thread CTAs per SM, every warp streams and then runs
-//                               the tail (12-byte points, images too large to keep twice, A/B feeds)
+//                               the tail (12-byte points, images too large to keep twice)
 //   encode_points_split_kernel  small batches: one thread-block cluster per scan
 #include <stdlib.h>
-#include <string.h>
 
 #include <mutex>
 #include <utility>
@@ -24,17 +23,7 @@ namespace nsc {
 
 namespace {
 
-#ifndef NSC_PRECHECK
-#define NSC_PRECHECK 1
-#endif
-// L2 policy of the point stream: 1 = evict-first when the kernel has no peers (single-GPU
-// encode: +1 %, the points no longer push the descriptor lines out of L2), plain when descriptors
-// of 7 peers are landing in this GPU's memory (evict-first costs 3.5 % there, profiles/r2o_*);
-// 0 = never (tuning builds).
-#ifndef NSC_L2_HINTS
-#define NSC_L2_HINTS 1
-#endif
-constexpr int kUnroll = 4;   // independent 16-byte loads in flight per thread (LDG feed)
+constexpr int kUnroll = 4;   // points in flight per thread (12-byte points, plain loads)
 
 // EncodeOutputs as the kernels read it: the peer pointers by value, and with rows_q the quantiser's
 // pairwise-sum plan for rows of D elements (nsc_quantize.cuh), built once per launch on the host.
@@ -73,21 +62,10 @@ struct EncodeArgs {
     unsigned* part_image;        // one E x 361 key image per split scan (0xffffffff before the launch)
 };
 
-// How the point pass of the GENERIC kernel is fed from HBM (the warp-specialised kernel has its own
-// whole-stage TMA ring).
-//   kFeedCpAsync  per-thread ring of 16-byte cp.async copies (SASS LDGSTS): kCpDepth-1 stages in
-//                 flight per thread without holding registers; needs 16-byte points.
-//   kFeedLdg      plain vector loads into registers (3-float points; A/B with NSC_FEED=ldg).
-// (An earlier per-WARP bulk-copy ring, 1.5 KB per copy, reached only 0.47 of the HBM roofline,
-// profiles/r1b_ncu_full_tma.txt; kFeedTma below copies whole 16 KB stages per CTA instead.)
-//   kFeedTma      the same ring filled by ONE elected thread with cp.async.bulk (SASS UBLKCP), a
-//                 whole 16 KB stage per copy, full/empty mbarriers per slot (NSC_FEED=tma).
-enum Feed { kFeedLdg = 0, kFeedCpAsync = 2, kFeedTma = 3 };
-constexpr int kDefaultFeed = kFeedCpAsync;
-constexpr int kTmaBarBytes = 128;   // 2 * kCpDepth mbarriers behind the ring
-__host__ __device__ constexpr int ring_bytes_of(int feed) {
-    return feed == kFeedCpAsync ? kCpRingBytes : feed == kFeedTma ? kCpRingBytes + kTmaBarBytes : 0;
-}
+// The point layout picks the feed of the generic and cluster kernels: 16-byte points stream through
+// the per-thread cp.async ring, 12-byte points take plain loads (cp.async needs 16-byte sources).
+// The warp-specialised kernel has its own whole-stage TMA ring. Feeds measured and dropped: DESIGN.md §4.
+__host__ __device__ constexpr int ring_bytes(int stride) { return stride == 4 ? kCpRingBytes : 0; }
 
 // ---- mbarrier / bulk-copy (TMA) primitives ------------------------------------------------
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
@@ -136,20 +114,6 @@ __device__ __forceinline__ void bulk_copy_g2s(uint32_t dst, const void* src, uin
         ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
         : "memory");
 }
-// full[s] at bars + 8 s (1 arrival: the producer's expect_tx), empty[s] at bars + 8 (kCpDepth + s)
-// (one arrival per consumer warp).
-__device__ __forceinline__ void tma_ring_init(unsigned char* ring) {
-    if (threadIdx.x == 0) {
-        const uint32_t bars = (uint32_t)__cvta_generic_to_shared(ring) + kCpRingBytes;
-        for (int s = 0; s < kCpDepth; ++s) {
-            mbar_init(bars + 8 * s, 1);
-            mbar_init(bars + 8 * (kCpDepth + s), kWarps - 1);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-}
-
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return (uint32_t)__cvta_generic_to_shared(p);
 }
@@ -189,7 +153,6 @@ __device__ __forceinline__ void scatter_min(uint32_t img_biased, uint32_t row_b,
             __trap();
     }
 #endif
-#if NSC_PRECHECK
     uint32_t cur;
     asm("ld.shared.u32 %0, [%1];" : "=r"(cur) : "r"(addr));
     asm volatile(
@@ -199,96 +162,37 @@ __device__ __forceinline__ void scatter_min(uint32_t img_biased, uint32_t row_b,
         "@p red.shared.min.u32 [%0], %1;\n"
         "}\n" ::"r"(addr), "r"(key), "r"(cur)
         : "memory");
-#else
-    asm volatile("red.shared.min.u32 [%0], %1;" ::"r"(addr), "r"(key) : "memory");
-#endif
 }
 
 template <int ROWMODE>
 __device__ __forceinline__ void project_point(float x, float y, float z, const DeviceParams& dp,
                                               uint32_t img_biased, bool in_range = true) {
-#ifdef NSC_EXP_NO_COMPUTE
-    // measurement-only build: keeps the loads alive, does no arithmetic and (in practice) no scatter
-    if (x == 12345.678f && in_range) scatter_min(img_biased, kFloorBias, kFloorBias, __float_as_uint(y + z));
-#else
     uint32_t row_b, col_b;
     uint32_t key = classify(x, y, z, dp, ROWMODE, row_b, col_b);
     if (!in_range) key = 0xffffffffu;
     scatter_min(img_biased, row_b, col_b, key);
-#endif
 }
 
 // Two points through the packed FP32 pipe (classify2, nsc_point.h); same bits as two project_point calls.
 template <int ROWMODE>
 __device__ __forceinline__ void project_pair(const float4& a, const float4& b, const DeviceParams& dp,
                                              uint32_t img_biased, bool in_a = true, bool in_b = true) {
-#if defined(NSC_EXP_NO_COMPUTE) || defined(NSC_NO_PACKED)
-    project_point<ROWMODE>(a.x, a.y, a.z, dp, img_biased, in_a);
-    project_point<ROWMODE>(b.x, b.y, b.z, dp, img_biased, in_b);
-#else
     uint32_t ka, ra, ca, kb, rb, cb;
     classify2(a.x, a.y, a.z, b.x, b.y, b.z, dp, ROWMODE, ka, ra, ca, kb, rb, cb);
     if (!in_a) ka = 0xffffffffu;
     if (!in_b) kb = 0xffffffffu;
     scatter_min(img_biased, ra, ca, ka);
     scatter_min(img_biased, rb, cb, kb);
-#endif
 }
 
 // Point pass over points [beg, beg + n) of the concatenated buffer: every kept point lowers the
 // key of its pixel in the shared-memory min image. CTA-collective (no barrier inside).
-template <int STRIDE, int ROWMODE, int FEED>
+template <int STRIDE, int ROWMODE>
 __device__ __forceinline__ void point_pass(const float* __restrict__ points, long long beg, int n,
                                            const DeviceParams& dp, uint32_t img_biased,
-                                           unsigned char* ring, uint32_t& g_stage) {
+                                           unsigned char* ring) {
     const int tid = threadIdx.x;
-    if (FEED == kFeedTma) {
-        // The last warp is the producer: its lane 0 keeps kCpDepth - 1 whole-stage bulk copies in
-        // flight; the other kWarps - 1 warps consume. Stage g of this CTA (counted across scans)
-        // lives in slot g % kCpDepth, full-barrier parity (g / kCpDepth) & 1; a slot is refilled
-        // once every consumer warp has arrived on its empty barrier.
-        constexpr int kConsumers = kThreads - 32;
-        constexpr int kStagePoints = kCpPts * kConsumers;
-        constexpr int kSlotBytes = kCpPts * kThreads * 16;
-        const float4* p4 = reinterpret_cast<const float4*>(points) + beg;
-        const uint32_t ring_u = smem_u32(ring), bars = ring_u + kCpRingBytes;
-        const int n_iter = (n + kStagePoints - 1) / kStagePoints;
-        const uint32_t g0 = g_stage;
-        if (tid >= kConsumers) {
-            if (tid == kConsumers) {
-                for (int it = 0; it < n_iter; ++it) {
-                    const uint32_t g = g0 + it, slot = g % kCpDepth;
-                    if (g >= kCpDepth) mbar_wait(bars + 8 * (kCpDepth + slot), ((g / kCpDepth) + 1) & 1);
-                    const uint32_t bytes = (uint32_t)min(kStagePoints, n - it * kStagePoints) * 16u;
-                    mbar_expect_tx(bars + 8 * slot, bytes);
-                    bulk_copy_g2s(ring_u + slot * kSlotBytes, p4 + (long long)it * kStagePoints, bytes,
-                                  bars + 8 * slot);
-                }
-            }
-        } else {
-            for (int it = 0; it < n_iter; ++it) {
-                const uint32_t g = g0 + it, slot = g % kCpDepth;
-                mbar_wait(bars + 8 * slot, (g / kCpDepth) & 1);
-                float4 v[kCpPts];
-#pragma unroll
-                for (int u = 0; u < kCpPts; ++u)
-                    v[u] = lds128(ring_u + slot * kSlotBytes + (u * kConsumers + tid) * 16);
-                if ((it + 1) * kStagePoints <= n) {
-#pragma unroll
-                    for (int u = 0; u < kCpPts; ++u)
-                        project_point<ROWMODE>(v[u].x, v[u].y, v[u].z, dp, img_biased);
-                } else {
-#pragma unroll
-                    for (int u = 0; u < kCpPts; ++u)
-                        project_point<ROWMODE>(v[u].x, v[u].y, v[u].z, dp, img_biased,
-                                               it * kStagePoints + u * kConsumers + tid < n);
-                }
-                __syncwarp();
-                if ((tid & 31) == 0) mbar_arrive(bars + 8 * (kCpDepth + slot));
-            }
-        }
-        g_stage = g0 + (uint32_t)n_iter;
-    } else if (FEED == kFeedCpAsync) {
+    if (STRIDE == 4) {
         // Each thread streams its own points through a private kCpDepth-deep shared-memory
         // ring of 16-byte cp.async copies. No cross-thread barrier is needed: a thread only
         // reads what it copied itself. Stage `it` holds points it*kStagePoints +
@@ -346,19 +250,6 @@ __device__ __forceinline__ void point_pass(const float* __restrict__ points, lon
             }
         }
         cp_async_wait<0>();
-    } else if (STRIDE == 4) {
-        const float4* p4 = reinterpret_cast<const float4*>(points) + beg;
-        for (int base = 0; base < n; base += kThreads * kUnroll) {
-            float4 v[kUnroll];
-#pragma unroll
-            for (int u = 0; u < kUnroll; ++u) {
-                const int i = base + u * kThreads + tid;
-                v[u] = i < n ? __ldcs(p4 + i) : make_float4(NAN, NAN, NAN, 0.0f);
-            }
-#pragma unroll
-            for (int u = 0; u < kUnroll; ++u)
-                project_point<ROWMODE>(v[u].x, v[u].y, v[u].z, dp, img_biased);
-        }
     } else {
         const float* p = points + beg * 3;
         for (int base = 0; base < n; base += kThreads * kUnroll) {
@@ -427,12 +318,12 @@ __device__ __forceinline__ bool finish_scan(const EncodeArgs& a, const DevicePar
     return true;
 }
 
-template <int STRIDE, int ROWMODE, int FEED>
+template <int STRIDE, int ROWMODE>
 __global__ void __launch_bounds__(kThreads, kMinBlocks)
 encode_points_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant__ DeviceParams dp) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ int s_scan;
-    const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes_of(FEED));
+    const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes(STRIDE));
     const TailSmem S(smem_raw, L);
     uint32_t* img = reinterpret_cast<uint32_t*>(S.img);
     const uint32_t img_biased = smem_u32(img) - kFloorBias * (uint32_t)(kPitch * 4 + 4);
@@ -440,8 +331,6 @@ encode_points_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant
     const int n_pix = dp.E * kPitch;
 
     init_tail_tables(S, dp);
-    uint32_t g_stage = 0;
-    if (FEED == kFeedTma) tma_ring_init(smem_raw + L.ring_off);
     long long phase_t0 = clock64();
     // Thread 0 always holds the NEXT scan index: the atomic's round trip (~1 us) is issued at the
     // top of a scan and only consumed at the top of the following one.
@@ -454,16 +343,13 @@ encode_points_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant
             if (next_scan < a.n_scans) next_scan = (int)atomicAdd(a.counter, 1u);
         }
         for (int i = tid; i < n_pix; i += kThreads) img[i] = kInfBits;
-        // The ring doubles as FFT scratch in the tail: every thread orders its generic-proxy
-        // writes before the barrier, the bulk copies (async proxy) are issued after it.
-        if (FEED == kFeedTma) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncthreads();
         const int scan = s_scan;
         if (scan >= a.n_scans) break;
         const long long beg = a.offsets[scan] - a.origin;
         const int n = (int)(a.offsets[scan + 1] - a.offsets[scan]);
         NSC_PHASE(0);
-        point_pass<STRIDE, ROWMODE, FEED>(a.points, beg, n, dp, img_biased, smem_raw + L.ring_off, g_stage);
+        point_pass<STRIDE, ROWMODE>(a.points, beg, n, dp, img_biased, smem_raw + L.ring_off);
         __syncthreads();
         NSC_PHASE(1);
         finish_scan<CtaGroup>(a, dp, S, scan, [&](int p) { NSC_PHASE(p); });
@@ -576,7 +462,10 @@ __device__ __forceinline__ void ws_producer_role(const EncodeArgs& a, unsigned c
     int unit = blockIdx.x;
     int next = (int)gridDim.x + (int)atomicAdd(a.counter, 1u);
     const uint64_t pol = l2_policy_evict_first();
-    const bool hint = NSC_L2_HINTS != 0 && a.out.peers.n == 0;
+    // Evict-first only when the kernel has no peers (single-GPU encode: +1 %, the points no longer
+    // push the descriptor lines out of L2); when descriptors of 7 peers are landing in this GPU's
+    // memory it costs 3.5 % (profiles/r2o_*), so the copies stay plain there.
+    const bool hint = a.out.peers.n == 0;
     uint32_t slot = 0, phase = 0;                     // phase = (stage counter / kWsDepth) & 1
     bool wrapped = false;
     for (int k = 0;; ++k) {
@@ -782,14 +671,14 @@ encode_points_ws_kernel(const __grid_constant__ EncodeArgs a, const __grid_const
 // image; after a cluster barrier the leader min-reduces the other images through distributed
 // shared memory and runs the tail. Cuts the latency of a single 120 k-point scan from one SM's
 // worth of time to roughly 1/cluster_size of it plus the tail.
-template <int STRIDE, int ROWMODE, int FEED>
+template <int STRIDE, int ROWMODE>
 __global__ void __launch_bounds__(kThreads, 1)
 encode_points_split_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant__ DeviceParams dp) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     const unsigned rank = cluster.block_rank(), csize = cluster.num_blocks();
-    const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes_of(FEED));
+    const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes(STRIDE));
     const TailSmem S(smem_raw, L);
     uint32_t* img = reinterpret_cast<uint32_t*>(S.img);
     const uint32_t img_biased = smem_u32(img) - kFloorBias * (uint32_t)(kPitch * 4 + 4);
@@ -798,15 +687,13 @@ encode_points_split_kernel(const __grid_constant__ EncodeArgs a, const __grid_co
     const int scan = blockIdx.x / csize;      // grid = n_scans * cluster size
 
     if (rank == 0) init_tail_tables(S, dp);
-    uint32_t g_stage = 0;
-    if (FEED == kFeedTma) tma_ring_init(smem_raw + L.ring_off);
     for (int i = tid; i < n_pix; i += kThreads) img[i] = kInfBits;
     __syncthreads();
     const long long beg = a.offsets[scan] - a.origin;
     const int n = (int)(a.offsets[scan + 1] - a.offsets[scan]);
     const int per = (n + (int)csize - 1) / (int)csize;
     const int lo = min(n, (int)rank * per), hi = min(n, lo + per);
-    point_pass<STRIDE, ROWMODE, FEED>(a.points, beg + lo, hi - lo, dp, img_biased, smem_raw + L.ring_off, g_stage);
+    point_pass<STRIDE, ROWMODE>(a.points, beg + lo, hi - lo, dp, img_biased, smem_raw + L.ring_off);
     cluster.sync();                           // every partial image is complete
     if (rank == 0) {
         for (int i = tid; i < n_pix; i += kThreads) {
@@ -940,18 +827,13 @@ int configure(K kernel, int smem, const DeviceInfo& di, int* blocks_per_sm) {
 
 using PointKernel = void (*)(const EncodeArgs, const DeviceParams);
 
-// The instantiation of the cluster (split) or the generic point kernel for a feed, a point stride
-// and a row mode; only the LDG feed reads 3-float points.
-#define NSC_POINT_KERNELS(K)                                                                     \
-    {{K<3, kRowPoly, kFeedLdg>, K<3, kRowSearch, kFeedLdg>},                                    \
-     {K<4, kRowPoly, kFeedLdg>, K<4, kRowSearch, kFeedLdg>},                                    \
-     {K<4, kRowPoly, kFeedCpAsync>, K<4, kRowSearch, kFeedCpAsync>},                            \
-     {K<4, kRowPoly, kFeedTma>, K<4, kRowSearch, kFeedTma>}}
-PointKernel point_kernel(bool split, int feed, int stride, int row_mode) {
-    static const PointKernel generic[4][2] = NSC_POINT_KERNELS(encode_points_kernel);
-    static const PointKernel cluster[4][2] = NSC_POINT_KERNELS(encode_points_split_kernel);
-    const int f = feed == kFeedTma ? 3 : feed == kFeedCpAsync ? 2 : stride == 4 ? 1 : 0;
-    return (split ? cluster : generic)[f][row_mode == kRowPoly ? 0 : 1];
+// The instantiation of the cluster (split) or the generic point kernel for a point stride and a
+// row mode.
+#define NSC_POINT_KERNELS(K) {{K<3, kRowPoly>, K<3, kRowSearch>}, {K<4, kRowPoly>, K<4, kRowSearch>}}
+PointKernel point_kernel(bool split, int stride, int row_mode) {
+    static const PointKernel generic[2][2] = NSC_POINT_KERNELS(encode_points_kernel);
+    static const PointKernel cluster[2][2] = NSC_POINT_KERNELS(encode_points_split_kernel);
+    return (split ? cluster : generic)[stride == 4 ? 1 : 0][row_mode == kRowPoly ? 0 : 1];
 }
 #undef NSC_POINT_KERNELS
 
@@ -1003,37 +885,27 @@ int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutp
     a.parts = 1;
     a.n_units = n_scans;
 
-    // Feed of the point pass (see enum Feed) and kernel choice. Product builds take no switches;
-    // tuning builds (-DNSC_TUNING, csrc/Makefile VARIANT=tune) read NSC_FEED=ldg|cpasync|tma,
-    // NSC_SPLIT=0 and NSC_WS=0 from the environment, once, for A/B runs and the bit-identity tests.
-    int feed = kDefaultFeed;
-    bool split_allowed = true, ws_allowed = true, tail_split_allowed = true;
+    // Kernel choice. Product builds take no switches; tuning builds (-DNSC_TUNING, csrc/Makefile
+    // VARIANT=tune) read NSC_SPLIT=0, NSC_WS=0 and NSC_TAILSPLIT=0 from the environment, once, so
+    // that A/B runs and the bit-identity tests can route a batch around the cluster kernel, the
+    // warp-specialised kernel or the split of its last wave.
 #ifdef NSC_TUNING
-    static const int feed_override = [] {
-        const char* e = getenv("NSC_FEED");
-        if (!e) return -1;
-        return strcmp(e, "ldg") == 0 ? (int)kFeedLdg : strcmp(e, "cpasync") == 0 ? (int)kFeedCpAsync
-               : strcmp(e, "tma") == 0 ? (int)kFeedTma : -1;
-    }();
     static const bool env_split = [] { const char* e = getenv("NSC_SPLIT"); return !(e && e[0] == '0'); }();
     static const bool env_ws = [] { const char* e = getenv("NSC_WS"); return !(e && e[0] == '0'); }();
     static const bool env_ts = [] { const char* e = getenv("NSC_TAILSPLIT"); return !(e && e[0] == '0'); }();
-    tail_split_allowed = env_ts;
-    if (feed_override >= 0) feed = feed_override;
-    split_allowed = env_split;
-    ws_allowed = env_ws && feed_override < 0;
+#else
+    constexpr bool env_split = true, env_ws = true, env_ts = true;
 #endif
-    if (in.stride != 4) feed = kFeedLdg;
-    const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes_of(feed));
+    const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes(in.stride));
     int csize = 1;
-    if (split_allowed) {
+    if (env_split) {
         if (n_scans * 8 <= di.sms) csize = 8;
         else if (n_scans * 4 <= di.sms) csize = 4;
         else if (n_scans * 2 <= di.sms) csize = 2;
     }
     PointKernel kernel = nullptr;
     if (csize > 1) {
-        kernel = point_kernel(true, feed, in.stride, dp.row_mode);
+        kernel = point_kernel(true, in.stride, dp.row_mode);
         st = configure(kernel, L.total, di, nullptr);
         if (st != NSC_OK) return st;
         cudaLaunchConfig_t cfg = {};
@@ -1053,7 +925,7 @@ int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutp
     // Large batches of 16-byte points: the warp-specialised kernel, when two images, the FFT
     // scratch and the ring fit one SM's shared memory; other geometries take the generic kernel.
     const WsLayout W(dp.E, dp.T, dp.n_bins);
-    if (ws_allowed && in.stride == 4 && W.ok && W.total <= di.max_smem_optin) {
+    if (env_ws && in.stride == 4 && W.ok && W.total <= di.max_smem_optin) {
         kernel = dp.row_mode == kRowPoly ? encode_points_ws_kernel<kRowPoly> : encode_points_ws_kernel<kRowSearch>;
         st = configure(kernel, W.total, di, nullptr);
         if (st != NSC_OK) return st;
@@ -1066,7 +938,7 @@ int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutp
         // piece streams faster than its tail -- the merge, and for the last piece the whole FFT --
         // runs, and the tail warps become the bottleneck (4541 scans as 4 pieces each: -3 %).
         const int R = n_scans > grid ? n_scans % grid : 0;
-        if (tail_split_allowed && R > 0 && 2 * R <= grid) {
+        if (env_ts && R > 0 && 2 * R <= grid) {
             int P = grid / R;
             if (P > 8) P = 8;
             if (workspace_bytes >= split_workspace(R, dp.E)) {
@@ -1086,7 +958,7 @@ int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutp
         kernel<<<grid, kWsThreads, W.total, stream>>>(a, dp);
         return record_cuda(cudaGetLastError());
     }
-    kernel = point_kernel(false, feed, in.stride, dp.row_mode);
+    kernel = point_kernel(false, in.stride, dp.row_mode);
     int per_sm = 0;
     st = configure(kernel, L.total, di, &per_sm);
     if (st != NSC_OK) return st;

@@ -419,12 +419,11 @@ def test_plain_c_caller_runs():
         assert r.stdout.count("descriptor sum 1.0000") + r.stdout.count("descriptor sum 0.9999") == 2, r.stdout
 
 
-@pytest.mark.parametrize("feed", ["tma", "ldg", "cpasync", "ws0"])
-def test_alternative_feeds_give_the_same_bits(feed, tmp_path):
+def test_generic_and_cluster_kernels_give_the_same_bits(tmp_path):
     """Large batches run the warp-specialised kernel (stream warps + tail warps, two images).
-    The tuning build (libnsc_b200_tune.so, the only one that reads the environment) can instead
-    run the generic persistent kernel fed by cp.async, by whole-stage TMA bulk copies with a
-    producer warp, or by plain vector loads: same descriptors, bit for bit."""
+    The tuning build (libnsc_b200_tune.so, the only one that reads the environment) with
+    NSC_WS=0 runs the generic persistent kernel instead, and the cluster kernel for 2 scans:
+    same descriptors as the product library, bit for bit."""
     import subprocess
     import sys
     from conftest import ROOT
@@ -449,8 +448,7 @@ for n in (2, 170):
 print("same")
 """
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True,
-                       env=dict(os.environ, NSC_LIB=_lib.TUNE_LIB_PATH,
-                                **({"NSC_WS": "0"} if feed == "ws0" else {"NSC_FEED": feed})), timeout=600)
+                       env=dict(os.environ, NSC_LIB=_lib.TUNE_LIB_PATH, NSC_WS="0"), timeout=600)
     assert r.returncode == 0 and "same" in r.stdout, r.stderr[-2000:]
 
 
