@@ -38,7 +38,16 @@ extern "C" {
 #define NSC_ABI_VERSION 2
 #define NSC_N_AZIMUTH 360        /* the in-kernel FFT is a 360-point transform            */
 #define NSC_N_FREQS 181          /* n_azimuth/2 + 1, spectral_encoder.py:88               */
-#define NSC_MAX_ELEVATION 64     /* rows of the projected image held in shared memory     */
+/* Rows of the projected image, held whole in one CTA's shared memory: up to 64 rows for every
+ * parameter block, up to 128 (one row per beam of a 128-beam sensor) for one that sets
+ * NSC_FLAG_TALL_IMAGES in nsc_params.flags. Images of more than 64 rows take their own kernels (one
+ * image per SM) and are pooled to target_rows <= 64 before the spectrum. A parameter block without
+ * the flag -- e.g. one filled for a library that stopped at 64 rows -- is refused above 64 rows with
+ * NSC_ERR_BAD_PARAMS, as before; libraries older than the flag ignore it and refuse 65..128 rows the
+ * same way. */
+#define NSC_MAX_ELEVATION 128
+#define NSC_MAX_ELEVATION_SHORT 64
+#define NSC_FLAG_TALL_IMAGES 1   /* nsc_params.flags: accept rows up to NSC_MAX_ELEVATION */
 #define NSC_MAX_TARGET_ROWS 64
 #define NSC_MAX_BINS 181
 #define NSC_MAX_DESCRIPTOR 4096  /* target_rows * n_bins held in shared memory             */
@@ -63,7 +72,8 @@ typedef enum nsc_status {
  * (range_image.py:102-109). POD; set struct_size = sizeof(nsc_params). */
 typedef struct nsc_params {
     int32_t struct_size;
-    int32_t n_elevation;        /* rows of the projected image, 1..NSC_MAX_ELEVATION       */
+    int32_t n_elevation;        /* rows of the projected image, 1..NSC_MAX_ELEVATION_SHORT,
+                                   1..NSC_MAX_ELEVATION with NSC_FLAG_TALL_IMAGES               */
     int32_t n_azimuth;          /* NSC_N_AZIMUTH for the fused kernels; nsc_anywidth_* take others */
     int32_t n_bins;             /* histogram bins per row, 1..NSC_MAX_BINS                  */
     int32_t target_rows;        /* target_elevation_bins; rows are average-pooled to this   */
@@ -73,7 +83,7 @@ typedef struct nsc_params {
     double el_min_rad;          /* np.deg2rad(elevation_range[0]) (range_image.py:126)      */
     double el_max_rad;          /* np.deg2rad(elevation_range[1]) (range_image.py:127)      */
     float epsilon;              /* 1e-8 (spectral_encoder.py:42)                            */
-    int32_t reserved;
+    int32_t flags;              /* NSC_FLAG_*; 0 from nsc_default_params (formerly reserved) */
 } nsc_params;
 
 /* Which image nsc_project_batch writes out. */
@@ -98,8 +108,8 @@ int nsc_freq_to_bin(float alpha, const nsc_params* p, int32_t* h_lut);
  * work counter) are enough for every call and smaller workspaces are refused; the RECOMMENDED size
  * returned here (a few MB) also holds one key image per scan of the grid's last, partial wave,
  * which lets a batch whose last wave fills at most half of the SMs split those scans over all
- * of them (+5 % on 600 scans). The result does not depend on the workspace size. Contents need
- * no initialisation. */
+ * of them (+5 % on 600 scans); images of more than 64 rows split no scan and get the 256 bytes.
+ * The result does not depend on the workspace size. Contents need no initialisation. */
 size_t nsc_workspace_bytes(int n_scans, const nsc_params* p);
 
 /* Replaces a loop of SpectralEncoder.encode_points (spectral_encoder.py:206-229; callers

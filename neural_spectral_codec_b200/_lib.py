@@ -19,7 +19,9 @@ CSRC = os.path.join(_HERE, "csrc")
 NSC_ABI_VERSION = 2
 N_AZIMUTH = 360
 N_FREQS = 181
-MAX_ELEVATION = 64
+MAX_ELEVATION = 128
+MAX_ELEVATION_SHORT = 64    # without FLAG_TALL_IMAGES
+FLAG_TALL_IMAGES = 1
 MAX_DESCRIPTOR = 4096
 MAX_PEERS = 8
 STAGE_PROJECTED = 0
@@ -41,7 +43,7 @@ class NscParams(C.Structure):
         ("el_min_rad", C.c_double),
         ("el_max_rad", C.c_double),
         ("epsilon", C.c_float),
-        ("reserved", C.c_int32),
+        ("flags", C.c_int32),
     ]
 
 

@@ -15,7 +15,7 @@ int validate_params(const nsc_params* p) {
     if (!p) return NSC_ERR_NULL_POINTER;
     if (p->struct_size != (int32_t)sizeof(nsc_params)) return NSC_ERR_BAD_STRUCT;
     if (p->n_azimuth != NSC_N_AZIMUTH) return NSC_ERR_BAD_PARAMS;
-    if (p->n_elevation < 1 || p->n_elevation > NSC_MAX_ELEVATION) return NSC_ERR_BAD_PARAMS;
+    if (p->n_elevation < 1 || p->n_elevation > max_rows(p)) return NSC_ERR_BAD_PARAMS;
     if (p->target_rows < 1 || p->target_rows > NSC_MAX_TARGET_ROWS) return NSC_ERR_BAD_PARAMS;
     if (p->n_bins < 1 || p->n_bins > NSC_MAX_BINS) return NSC_ERR_BAD_PARAMS;
     if ((long long)p->target_rows * p->n_bins > NSC_MAX_DESCRIPTOR) return NSC_ERR_BAD_PARAMS;

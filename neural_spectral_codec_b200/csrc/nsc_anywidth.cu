@@ -99,11 +99,13 @@ __device__ __forceinline__ bool project_point_ref(float x, float y, float z, con
     return true;
 }
 
+// ROWS: the capacity of the per-row arrays (kShortRows, or NSC_MAX_ELEVATION for taller images).
+template <int ROWS>
 __global__ void __launch_bounds__(kGThreads)
 anywidth_kernel(const __grid_constant__ AnyArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float* hist = reinterpret_cast<float*>(smem_raw);                  // T x n_bins
-    __shared__ int s_nvalid[NSC_MAX_ELEVATION], s_src[NSC_MAX_ELEVATION];
+    __shared__ int s_nvalid[ROWS], s_src[ROWS];
     __shared__ double s_red[kGThreads / 32];
     const int tid = threadIdx.x, E = a.E, W = a.W, T = a.T, F = a.F;
     const Scratch S(a.scratch + (size_t)blockIdx.x * a.scratch_per_cta, E, W, T, F);
@@ -247,7 +249,7 @@ int validate_any(const nsc_params* p) {
     if (!p) return NSC_ERR_NULL_POINTER;
     if (p->struct_size != (int32_t)sizeof(nsc_params)) return NSC_ERR_BAD_STRUCT;
     if (p->n_azimuth < 2 || p->n_azimuth > kMaxWidth) return NSC_ERR_BAD_PARAMS;
-    if (p->n_elevation < 1 || p->n_elevation > NSC_MAX_ELEVATION) return NSC_ERR_BAD_PARAMS;
+    if (p->n_elevation < 1 || p->n_elevation > max_rows(p)) return NSC_ERR_BAD_PARAMS;
     if (p->target_rows < 1 || p->target_rows > NSC_MAX_TARGET_ROWS) return NSC_ERR_BAD_PARAMS;
     if (p->n_bins < 1 || p->n_bins > p->n_azimuth / 2 + 1) return NSC_ERR_BAD_PARAMS;
     if ((long long)p->target_rows * p->n_bins > NSC_MAX_DESCRIPTOR) return NSC_ERR_BAD_PARAMS;
@@ -305,9 +307,10 @@ int run(AnyArgs& a, const nsc_params* p, int rows, const int32_t* h_lut, void* w
         if (e != cudaSuccess) return record_cuda(e);
     }
     const size_t smem = (size_t)a.T * a.n_bins * 4;
-    cudaError_t e = cudaFuncSetAttribute(anywidth_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const auto kernel = a.E > kShortRows ? anywidth_kernel<NSC_MAX_ELEVATION> : anywidth_kernel<kShortRows>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return record_cuda(e);
-    anywidth_kernel<<<grid, kGThreads, smem, s>>>(a);
+    kernel<<<grid, kGThreads, smem, s>>>(a);
     return record_cuda(cudaGetLastError());
 }
 
@@ -320,7 +323,7 @@ using namespace nsc;
 extern "C" {
 
 size_t nsc_anywidth_workspace_bytes(int n, int rows, const nsc_params* p) {
-    if (n < 0 || rows < 1 || rows > NSC_MAX_ELEVATION || validate_any(p) != NSC_OK) return 0;
+    if (n < 0 || validate_any(p) != NSC_OK || rows < 1 || rows > max_rows(p)) return 0;
     const int grid = n < kMaxGrid ? (n < 1 ? 1 : n) : kMaxGrid;
     return table_bytes(p) + Scratch::bytes(rows, p->n_azimuth, p->target_rows, p->n_azimuth / 2 + 1) * (size_t)grid;
 }
@@ -356,7 +359,7 @@ int nsc_anywidth_images(const float* d_images_in, int n_images, int rows, const 
     int st = validate_any(p);
     if (st != NSC_OK) return st;
     if (n_images < 0) return NSC_ERR_BAD_COUNT;
-    if (rows < 1 || rows > NSC_MAX_ELEVATION) return NSC_ERR_BAD_PARAMS;
+    if (rows < 1 || rows > max_rows(p)) return NSC_ERR_BAD_PARAMS;
     if (interp_method != -1 && interp_method != NSC_INTERP_LINEAR && interp_method != NSC_INTERP_NEAREST)
         return NSC_ERR_BAD_PARAMS;
     if (n_images == 0) return NSC_OK;

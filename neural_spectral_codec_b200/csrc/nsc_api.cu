@@ -174,7 +174,7 @@ int nsc_encode_range_images(const float* d_images, int n_images, int rows, const
     int st = make_device_params(p, h_lut, &dp);
     if (st != NSC_OK) return st;
     if (n_images < 0) return NSC_ERR_BAD_COUNT;
-    if (rows < 1 || rows > NSC_MAX_ELEVATION) return NSC_ERR_BAD_PARAMS;
+    if (rows < 1 || rows > max_rows(p)) return NSC_ERR_BAD_PARAMS;
     if (n_images == 0) return NSC_OK;
     if (!d_images || !d_out) return NSC_ERR_NULL_POINTER;
     return launch_encode_images(d_images, n_images, rows, dp, d_out, (cudaStream_t)stream);
@@ -205,7 +205,8 @@ int nsc_test_host_classify(const float* h_points, int point_stride, int64_t n_po
     for (int64_t i = 0; i < n_points; ++i) {
         const float* q = h_points + i * point_stride;
         uint32_t row_b = 0, col_b = 0;
-        const uint32_t key = classify(q[0], q[1], q[2], dp, dp.row_mode, row_b, col_b);
+        // the row search of the tall kernels: the same rows as the short one's for E <= 64
+        const uint32_t key = classify<NSC_MAX_ELEVATION>(q[0], q[1], q[2], dp, dp.row_mode, row_b, col_b);
         const bool keep = key != 0xffffffffu && !key_is_empty(key, dp);
         h_keep[i] = keep ? 1 : 0;
         h_row[i] = keep ? (int32_t)(row_b - kFloorBias) : -1;

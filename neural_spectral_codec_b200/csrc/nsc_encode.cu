@@ -1,13 +1,16 @@
 // Fused encode kernels: points -> min-range image (shared memory) -> interpolation -> spectrum
 // -> descriptor. Persistent CTAs pull whole scans from a work counter, so the range image, its
 // interpolation and the spectrum never leave shared memory: HBM traffic is the 16 B per point
-// and the descriptor. Three kernels share the per-point and the tail code:
+// and the descriptor. The kernels share the per-point and the tail code:
 //   encode_points_ws_kernel     the hot one (large batches of 16-byte points): one 1024-thread CTA
 //                               per SM, a TMA producer thread, 24 stream warps, 7 tail warps, two
 //                               images; see the comment above it
 //   encode_points_kernel        generic: 2 x 512-thread CTAs per SM, every warp streams and then runs
 //                               the tail (12-byte points, images too large to keep twice)
 //   encode_points_split_kernel  small batches: one thread-block cluster per scan
+//   encode_points_tall_kernel, encode_points_tall_split_kernel
+//                               the generic and the cluster kernel for images of 65..128 rows: one
+//                               image per SM, points straight into registers, pooled before the FFT
 #include <stdlib.h>
 
 #include <mutex>
@@ -24,6 +27,11 @@ namespace nsc {
 namespace {
 
 constexpr int kUnroll = 4;   // points in flight per thread (12-byte points, plain loads)
+#ifndef NSC_TALL_PTS
+#define NSC_TALL_PTS 12
+#endif
+constexpr int kTallPts = NSC_TALL_PTS;   // 16-byte points in flight per thread of a tall kernel (even)
+static_assert(kTallPts % 2 == 0, "the tall feed classifies points in pairs");
 
 // EncodeOutputs as the kernels read it: the peer pointers by value, and with rows_q the quantiser's
 // pairwise-sum plan for rows of D elements (nsc_quantize.cuh), built once per launch on the host.
@@ -164,21 +172,21 @@ __device__ __forceinline__ void scatter_min(uint32_t img_biased, uint32_t row_b,
         : "memory");
 }
 
-template <int ROWMODE>
+template <int ROWMODE, int ROWS = kShortRows>
 __device__ __forceinline__ void project_point(float x, float y, float z, const DeviceParams& dp,
                                               uint32_t img_biased, bool in_range = true) {
     uint32_t row_b, col_b;
-    uint32_t key = classify(x, y, z, dp, ROWMODE, row_b, col_b);
+    uint32_t key = classify<ROWS>(x, y, z, dp, ROWMODE, row_b, col_b);
     if (!in_range) key = 0xffffffffu;
     scatter_min(img_biased, row_b, col_b, key);
 }
 
 // Two points through the packed FP32 pipe (classify2, nsc_point.h); same bits as two project_point calls.
-template <int ROWMODE>
+template <int ROWMODE, int ROWS = kShortRows>
 __device__ __forceinline__ void project_pair(const float4& a, const float4& b, const DeviceParams& dp,
                                              uint32_t img_biased, bool in_a = true, bool in_b = true) {
     uint32_t ka, ra, ca, kb, rb, cb;
-    classify2(a.x, a.y, a.z, b.x, b.y, b.z, dp, ROWMODE, ka, ra, ca, kb, rb, cb);
+    classify2<ROWS>(a.x, a.y, a.z, b.x, b.y, b.z, dp, ROWMODE, ka, ra, ca, kb, rb, cb);
     if (!in_a) ka = 0xffffffffu;
     if (!in_b) kb = 0xffffffffu;
     scatter_min(img_biased, ra, ca, ka);
@@ -186,13 +194,28 @@ __device__ __forceinline__ void project_pair(const float4& a, const float4& b, c
 }
 
 // Point pass over points [beg, beg + n) of the concatenated buffer: every kept point lowers the
-// key of its pixel in the shared-memory min image. CTA-collective (no barrier inside).
-template <int STRIDE, int ROWMODE>
+// key of its pixel in the shared-memory min image. CTA-collective (no barrier inside). ROWS: the
+// row capacity of the kernel; the tall kernels (ROWS > kShortRows) keep no ring.
+template <int STRIDE, int ROWMODE, int ROWS = kShortRows>
 __device__ __forceinline__ void point_pass(const float* __restrict__ points, long long beg, int n,
                                            const DeviceParams& dp, uint32_t img_biased,
                                            unsigned char* ring) {
     const int tid = threadIdx.x;
-    if (STRIDE == 4) {
+    if (STRIDE == 4 && ROWS > kShortRows) {
+        // Tall kernels: the image leaves no room for a ring, so each thread keeps kTallPts
+        // 16-byte points in flight in registers (LDG.128, evict-first); points past the end are
+        // NaN, which never lowers a key (classify). 12 points: 1.13 x the rate of 8, 1.53 x that of 4
+        // (profiles/r3d_tall_image_cost.txt); 16 would not fit 128 registers.
+        const float4* gp = reinterpret_cast<const float4*>(points) + beg + tid;
+        const float4 nan4 = make_float4(NAN, NAN, NAN, NAN);
+        for (int base = 0; base < n; base += kThreads * kTallPts) {
+            float4 v[kTallPts];
+#pragma unroll
+            for (int u = 0; u < kTallPts; ++u) v[u] = base + u * kThreads + tid < n ? __ldcs(gp + base + u * kThreads) : nan4;
+#pragma unroll
+            for (int u = 0; u < kTallPts; u += 2) project_pair<ROWMODE, ROWS>(v[u], v[u + 1], dp, img_biased);
+        }
+    } else if (STRIDE == 4) {
         // Each thread streams its own points through a private kCpDepth-deep shared-memory
         // ring of 16-byte cp.async copies. No cross-thread barrier is needed: a thread only
         // reads what it copied itself. Stage `it` holds points it*kStagePoints +
@@ -264,7 +287,7 @@ __device__ __forceinline__ void point_pass(const float* __restrict__ points, lon
             }
 #pragma unroll
             for (int u = 0; u < kUnroll; ++u)
-                project_point<ROWMODE>(x[u], y[u], z[u], dp, img_biased);
+                project_point<ROWMODE, ROWS>(x[u], y[u], z[u], dp, img_biased);
         }
     }
 }
@@ -291,8 +314,9 @@ __device__ __forceinline__ void point_pass(const float* __restrict__ points, lon
 // interpolation, (optional) image output, spectrum, bins, normalisation, descriptor store.
 // `mark(p)` is called between the phases: 2, 3 and 4 here, 5..9 inside spectrum_and_bins (9: the
 // image is read for the last time). Returns false, right after the image output, when the launch
-// writes no descriptors.
-template <typename G, typename Mark>
+// writes no descriptors. ROWS > kShortRows (tall kernels): the image is pooled in place to its
+// first T rows before the spectrum (pool_rows_in_place).
+template <typename G, int ROWS = kShortRows, typename Mark>
 __device__ __forceinline__ bool finish_scan(const EncodeArgs& a, const DeviceParams& dp,
                                             const TailSmem& S, int scan, Mark mark) {
     const KernelOutputs& o = a.out;
@@ -311,19 +335,26 @@ __device__ __forceinline__ bool finish_scan(const EncodeArgs& a, const DevicePar
     }
     mark(2);
     if (!o.descriptors()) return false;
-    spectrum_and_bins(S, dp, dp.E, mark, G());
+    int rows = dp.E;
+    if (ROWS > kShortRows) {
+        pool_rows_in_place<G>(S, dp.E, dp.T);
+        rows = dp.T;
+    }
+    spectrum_and_bins(S, dp, rows, mark, G());
     mark(3);
     normalise_and_store(S, dp, o.row(scan, D), G());
     mark(4);
     return true;
 }
 
-template <int STRIDE, int ROWMODE>
-__global__ void __launch_bounds__(kThreads, kMinBlocks)
-encode_points_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant__ DeviceParams dp) {
+// The persistent loop of encode_points_kernel and encode_points_tall_kernel: every warp streams
+// the scan's points and then runs its tail.
+template <int STRIDE, int ROWMODE, int ROWS>
+__device__ __forceinline__ void persistent_scans(const EncodeArgs& a, const DeviceParams& dp) {
+    constexpr bool tall = ROWS > kShortRows;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ int s_scan;
-    const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes(STRIDE));
+    const SmemLayout L(dp.E, dp.T, dp.n_bins, tall ? 0 : ring_bytes(STRIDE), tall);
     const TailSmem S(smem_raw, L);
     uint32_t* img = reinterpret_cast<uint32_t*>(S.img);
     const uint32_t img_biased = smem_u32(img) - kFloorBias * (uint32_t)(kPitch * 4 + 4);
@@ -349,12 +380,27 @@ encode_points_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant
         const long long beg = a.offsets[scan] - a.origin;
         const int n = (int)(a.offsets[scan + 1] - a.offsets[scan]);
         NSC_PHASE(0);
-        point_pass<STRIDE, ROWMODE>(a.points, beg, n, dp, img_biased, smem_raw + L.ring_off);
+        point_pass<STRIDE, ROWMODE, ROWS>(a.points, beg, n, dp, img_biased, smem_raw + L.ring_off);
         __syncthreads();
         NSC_PHASE(1);
-        finish_scan<CtaGroup>(a, dp, S, scan, [&](int p) { NSC_PHASE(p); });
+        finish_scan<CtaGroup, ROWS>(a, dp, S, scan, [&](int p) { NSC_PHASE(p); });
     }
     if (tid == 0) wait_bulk_stores_done();      // descriptors leave shared memory before the CTA does
+}
+
+template <int STRIDE, int ROWMODE>
+__global__ void __launch_bounds__(kThreads, kMinBlocks)
+encode_points_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant__ DeviceParams dp) {
+    persistent_scans<STRIDE, ROWMODE, kShortRows>(a, dp);
+}
+
+// Images of more than 64 rows (up to NSC_MAX_ELEVATION): a 128 x 361 key image is 184 832 B, so
+// one CTA per SM holds one image and no ring; the points come straight from global memory into
+// registers (point_pass) and the tail pools the image before the spectrum (finish_scan).
+template <int STRIDE, int ROWMODE>
+__global__ void __launch_bounds__(kThreads, 1)
+encode_points_tall_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant__ DeviceParams dp) {
+    persistent_scans<STRIDE, ROWMODE, NSC_MAX_ELEVATION>(a, dp);
 }
 
 // ---- warp-specialised persistent kernel ---------------------------------------------------
@@ -671,14 +717,14 @@ encode_points_ws_kernel(const __grid_constant__ EncodeArgs a, const __grid_const
 // image; after a cluster barrier the leader min-reduces the other images through distributed
 // shared memory and runs the tail. Cuts the latency of a single 120 k-point scan from one SM's
 // worth of time to roughly 1/cluster_size of it plus the tail.
-template <int STRIDE, int ROWMODE>
-__global__ void __launch_bounds__(kThreads, 1)
-encode_points_split_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant__ DeviceParams dp) {
+template <int STRIDE, int ROWMODE, int ROWS>
+__device__ __forceinline__ void cluster_scan(const EncodeArgs& a, const DeviceParams& dp) {
+    constexpr bool tall = ROWS > kShortRows;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     const unsigned rank = cluster.block_rank(), csize = cluster.num_blocks();
-    const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes(STRIDE));
+    const SmemLayout L(dp.E, dp.T, dp.n_bins, tall ? 0 : ring_bytes(STRIDE), tall);
     const TailSmem S(smem_raw, L);
     uint32_t* img = reinterpret_cast<uint32_t*>(S.img);
     const uint32_t img_biased = smem_u32(img) - kFloorBias * (uint32_t)(kPitch * 4 + 4);
@@ -693,7 +739,7 @@ encode_points_split_kernel(const __grid_constant__ EncodeArgs a, const __grid_co
     const int n = (int)(a.offsets[scan + 1] - a.offsets[scan]);
     const int per = (n + (int)csize - 1) / (int)csize;
     const int lo = min(n, (int)rank * per), hi = min(n, lo + per);
-    point_pass<STRIDE, ROWMODE>(a.points, beg + lo, hi - lo, dp, img_biased, smem_raw + L.ring_off);
+    point_pass<STRIDE, ROWMODE, ROWS>(a.points, beg + lo, hi - lo, dp, img_biased, smem_raw + L.ring_off);
     cluster.sync();                           // every partial image is complete
     if (rank == 0) {
         for (int i = tid; i < n_pix; i += kThreads) {
@@ -706,9 +752,22 @@ encode_points_split_kernel(const __grid_constant__ EncodeArgs a, const __grid_co
     if (rank == 0) {
         __syncthreads();
         long long phase_t0 = 0;
-        finish_scan<CtaGroup>(a, dp, S, scan, [&](int p) { NSC_PHASE(p); });
+        finish_scan<CtaGroup, ROWS>(a, dp, S, scan, [&](int p) { NSC_PHASE(p); });
         if (tid == 0) wait_bulk_stores_done();
     }
+}
+
+template <int STRIDE, int ROWMODE>
+__global__ void __launch_bounds__(kThreads, 1)
+encode_points_split_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant__ DeviceParams dp) {
+    cluster_scan<STRIDE, ROWMODE, kShortRows>(a, dp);
+}
+
+// The same for images of more than 64 rows: every CTA of the cluster holds a whole tall image.
+template <int STRIDE, int ROWMODE>
+__global__ void __launch_bounds__(kThreads, 1)
+encode_points_tall_split_kernel(const __grid_constant__ EncodeArgs a, const __grid_constant__ DeviceParams dp) {
+    cluster_scan<STRIDE, ROWMODE, NSC_MAX_ELEVATION>(a, dp);
 }
 
 // Range images in, descriptors out: SpectralEncoder.forward / encode_range_image
@@ -731,6 +790,38 @@ encode_images_kernel(const float* __restrict__ images, int n_images, int rows,
         }
         __syncthreads();
         spectrum_and_bins(S, dp, rows);
+        RowDest dst;
+        dst.out = out + (long long)im * D;
+        normalise_and_store(S, dp, dst);
+    }
+    if (threadIdx.x == 0) wait_bulk_stores_done();
+}
+
+// The same for images of more than 64 rows: pooled to T rows while they are read from global
+// memory (pooled_value's arithmetic; forward() has no empty-row fill), so shared memory holds the
+// T-row image only.
+__global__ void __launch_bounds__(kThreads, kMinBlocks)
+encode_tall_images_kernel(const float* __restrict__ images, int n_images, int rows,
+                          const __grid_constant__ DeviceParams dp, float* __restrict__ out) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const int T = dp.T;
+    const SmemLayout L(T, T, dp.n_bins);
+    const TailSmem S(smem_raw, L);
+    const int D = T * dp.n_bins;
+    init_tail_tables(S, dp);
+    if (threadIdx.x < T) S.src[threadIdx.x] = threadIdx.x;
+    for (int im = blockIdx.x; im < n_images; im += gridDim.x) {
+        __syncthreads();
+        const float* src = images + (long long)im * rows * kAz;
+        for (int i = threadIdx.x; i < T * kAz; i += kThreads) {
+            const int t = i / kAz, c = i - t * kAz;
+            const int r0 = (t * rows) / T, r1 = ((t + 1) * rows + T - 1) / T;
+            float sum = 0.0f;
+            for (int r = r0; r < r1; ++r) sum += src[r * kAz + c];
+            S.img[t * kPitch + c] = sum / (float)(r1 - r0);
+        }
+        __syncthreads();
+        spectrum_and_bins(S, dp, T);
         RowDest dst;
         dst.out = out + (long long)im * D;
         normalise_and_store(S, dp, dst);
@@ -827,13 +918,16 @@ int configure(K kernel, int smem, const DeviceInfo& di, int* blocks_per_sm) {
 
 using PointKernel = void (*)(const EncodeArgs, const DeviceParams);
 
-// The instantiation of the cluster (split) or the generic point kernel for a point stride and a
-// row mode.
+// The instantiation of the cluster (split) or the generic point kernel, for images of up to 64
+// rows or taller ones, for a point stride and a row mode.
 #define NSC_POINT_KERNELS(K) {{K<3, kRowPoly>, K<3, kRowSearch>}, {K<4, kRowPoly>, K<4, kRowSearch>}}
-PointKernel point_kernel(bool split, int stride, int row_mode) {
+PointKernel point_kernel(bool split, bool tall, int stride, int row_mode) {
     static const PointKernel generic[2][2] = NSC_POINT_KERNELS(encode_points_kernel);
     static const PointKernel cluster[2][2] = NSC_POINT_KERNELS(encode_points_split_kernel);
-    return (split ? cluster : generic)[stride == 4 ? 1 : 0][row_mode == kRowPoly ? 0 : 1];
+    static const PointKernel generic_tall[2][2] = NSC_POINT_KERNELS(encode_points_tall_kernel);
+    static const PointKernel cluster_tall[2][2] = NSC_POINT_KERNELS(encode_points_tall_split_kernel);
+    const PointKernel(*k)[2] = split ? (tall ? cluster_tall : cluster) : (tall ? generic_tall : generic);
+    return k[stride == 4 ? 1 : 0][row_mode == kRowPoly ? 0 : 1];
 }
 #undef NSC_POINT_KERNELS
 
@@ -849,7 +943,7 @@ static size_t split_workspace(int n_split, int E) {
 }
 size_t workspace_bytes_for(int n_scans, int E) {
     (void)n_scans;
-    return split_workspace(kMaxSplitScans - 1, E);
+    return E > kShortRows ? kMinWorkspace : split_workspace(kMaxSplitScans - 1, E);   // tall kernels split no scan
 }
 size_t workspace_bytes_min() { return kMinWorkspace; }
 
@@ -896,7 +990,10 @@ int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutp
 #else
     constexpr bool env_split = true, env_ws = true, env_ts = true;
 #endif
-    const SmemLayout L(dp.E, dp.T, dp.n_bins, ring_bytes(in.stride));
+    // Images of more than 64 rows take the tall kernels (one image per SM, no ring, no
+    // warp-specialised variant): by the row count alone.
+    const bool tall = dp.E > kShortRows;
+    const SmemLayout L(dp.E, dp.T, dp.n_bins, tall ? 0 : ring_bytes(in.stride), tall);
     int csize = 1;
     if (env_split) {
         if (n_scans * 8 <= di.sms) csize = 8;
@@ -905,7 +1002,7 @@ int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutp
     }
     PointKernel kernel = nullptr;
     if (csize > 1) {
-        kernel = point_kernel(true, in.stride, dp.row_mode);
+        kernel = point_kernel(true, tall, in.stride, dp.row_mode);
         st = configure(kernel, L.total, di, nullptr);
         if (st != NSC_OK) return st;
         cudaLaunchConfig_t cfg = {};
@@ -925,7 +1022,7 @@ int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutp
     // Large batches of 16-byte points: the warp-specialised kernel, when two images, the FFT
     // scratch and the ring fit one SM's shared memory; other geometries take the generic kernel.
     const WsLayout W(dp.E, dp.T, dp.n_bins);
-    if (env_ws && in.stride == 4 && W.ok && W.total <= di.max_smem_optin) {
+    if (!tall && env_ws && in.stride == 4 && W.ok && W.total <= di.max_smem_optin) {
         kernel = dp.row_mode == kRowPoly ? encode_points_ws_kernel<kRowPoly> : encode_points_ws_kernel<kRowSearch>;
         st = configure(kernel, W.total, di, nullptr);
         if (st != NSC_OK) return st;
@@ -958,7 +1055,7 @@ int launch_encode(const PointBatch& in, const DeviceParams& dp, const EncodeOutp
         kernel<<<grid, kWsThreads, W.total, stream>>>(a, dp);
         return record_cuda(cudaGetLastError());
     }
-    kernel = point_kernel(false, in.stride, dp.row_mode);
+    kernel = point_kernel(false, tall, in.stride, dp.row_mode);
     int per_sm = 0;
     st = configure(kernel, L.total, di, &per_sm);
     if (st != NSC_OK) return st;
@@ -980,13 +1077,16 @@ int launch_encode_images(const float* d_images, int n_images, int rows, const De
     DeviceInfo di;
     int st = device_info(&di);
     if (st != NSC_OK) return st;
-    const SmemLayout L(rows, dp.T, dp.n_bins);
+    // more than 64 rows: pooled while loaded, so the kernel holds T <= 64 rows
+    const bool tall = rows > kShortRows;
+    const SmemLayout L(tall ? dp.T : rows, dp.T, dp.n_bins);
+    const auto kernel = tall ? encode_tall_images_kernel : encode_images_kernel;
     int per_sm = 0;
-    st = configure(encode_images_kernel, L.total, di, &per_sm);
+    st = configure(kernel, L.total, di, &per_sm);
     if (st != NSC_OK) return st;
     int grid = di.sms * per_sm;
     if (grid > n_images) grid = n_images;
-    encode_images_kernel<<<grid, kThreads, L.total, stream>>>(d_images, n_images, rows, dp, d_out);
+    kernel<<<grid, kThreads, L.total, stream>>>(d_images, n_images, rows, dp, d_out);
     return record_cuda(cudaGetLastError());
 }
 

@@ -15,6 +15,13 @@ constexpr uint32_t kInfBits = 0x7f800000u;
 constexpr int kColTerms = 7;            // odd polynomial for atan on [0,1] (azimuth)
 constexpr int kRowTerms = 5;            // odd polynomial for atan on the elevation FOV
 constexpr int kMaxSignals = 8;          // complex 360-point FFTs in flight per CTA (two rows each)
+// Row capacity of the encode kernels for images of up to 64 rows; taller images (up to
+// NSC_MAX_ELEVATION) take the tall kernels, whose row search reaches row NSC_MAX_ELEVATION - 1.
+constexpr int kShortRows = NSC_MAX_ELEVATION_SHORT;
+// The row envelope of a parameter block: NSC_MAX_ELEVATION with NSC_FLAG_TALL_IMAGES, else 64.
+inline int max_rows(const nsc_params* p) {
+    return (p->flags & NSC_FLAG_TALL_IMAGES) ? NSC_MAX_ELEVATION : NSC_MAX_ELEVATION_SHORT;
+}
 
 enum RowMode { kRowPoly = 0, kRowSearch = 1 };
 

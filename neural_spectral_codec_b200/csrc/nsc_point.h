@@ -156,8 +156,9 @@ NSC_HD uint32_t column_biased(float x, float y) {
     return floor_biased(r, 180.0f);
 }
 
-// Row + kFloorBias.
-template <typename P>
+// Row + kFloorBias. ROWS: the row capacity of the caller (a power of two >= E), which sets the
+// depth of the kRowSearch binary search.
+template <int ROWS = kShortRows, typename P>
 NSC_HD uint32_t row_biased(float z, float rho2, const P& dp, int row_mode) {
     if (row_mode == kRowPoly) {
         float u = z * rsqrt_fast(rho2);               // rho2 == 0 -> +-inf, clamped below
@@ -171,7 +172,7 @@ NSC_HD uint32_t row_biased(float z, float rho2, const P& dp, int row_mode) {
     const float q = z * fabsf(z);
     int row = 0;
 #pragma unroll
-    for (int step = NSC_MAX_ELEVATION / 2; step > 0; step >>= 1) {
+    for (int step = ROWS / 2; step > 0; step >>= 1) {
         const int k = row + step;
         if (k < dp.E && q >= dp.row_c[k] * rho2) row = k;
     }
@@ -183,14 +184,14 @@ NSC_HD uint32_t row_biased(float z, float rho2, const P& dp, int row_mode) {
 // the bits of s_hi (too far, +Inf, NaN) are NOT filtered here: they can only survive in a pixel
 // no in-range point hit, and the per-pixel conversion after the scatter maps them to "empty"
 // (key_is_empty). That moves the upper half of the range filter from 120 k points to 5 760 pixels.
-template <typename P>
+template <int ROWS = kShortRows, typename P>
 NSC_HD uint32_t classify(float x, float y, float z, const P& dp, int row_mode, uint32_t& row_b,
                          uint32_t& col_b) {
     const float xx = mul_rn(x, x), yy = mul_rn(y, y), zz = mul_rn(z, z);
     const float rho2 = add_rn(xx, yy);
     const float s = add_rn(rho2, zz);
     col_b = column_biased(x, y);
-    row_b = row_biased(z, rho2, dp, row_mode);
+    row_b = row_biased<ROWS>(z, rho2, dp, row_mode);
     return (s >= dp.s_lo) ? f2u(s) : 0xffffffffu;         // NaN compares false
 }
 
@@ -220,7 +221,7 @@ __device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
     return r;
 }
 
-template <typename P>
+template <int ROWS = kShortRows, typename P>
 __device__ __forceinline__ void classify2(float xa, float ya, float za, float xb, float yb, float zb,
                                           const P& dp, int row_mode, uint32_t& key_a, uint32_t& row_a,
                                           uint32_t& col_a, uint32_t& key_b, uint32_t& row_b,
@@ -272,8 +273,8 @@ __device__ __forceinline__ void classify2(float xa, float ya, float za, float xb
         row_a = floor_biased(va, 0.0f);
         row_b = floor_biased(vb, 0.0f);
     } else {
-        row_a = row_biased(za, rho2a, dp, row_mode);
-        row_b = row_biased(zb, rho2b, dp, row_mode);
+        row_a = row_biased<ROWS>(za, rho2a, dp, row_mode);
+        row_b = row_biased<ROWS>(zb, rho2b, dp, row_mode);
     }
 }
 #endif

@@ -49,25 +49,37 @@ constexpr int kCpRingBytes = kCpDepth * kCpPts * kThreads * 16;   // 65 536 B pe
 
 // Shared-memory carve-up, identical on host (size) and device (pointers). With a ring the two
 // FFT buffers alias it: the ring is idle (fully consumed) while the tail runs.
+// pooled: the layout of the tall kernels (rows > kShortRows), whose tail pools the image in place
+// to its first T rows (pool_rows_in_place) before the spectrum; both FFT buffers then lie in the
+// image's dead rows above them, and no ring is kept.
 struct SmemLayout {
     int img_off, tw_off, fa_off, fb_off, hist_off, mask_off, nvalid_off, src_off, red_off;
     int ring_off, bins_off, total;
     int n_sig;  // complex FFTs per batch
-    __host__ __device__ SmemLayout(int rows, int T, int n_bins, int ring_bytes = 0) {
+    __host__ __device__ SmemLayout(int rows, int T, int n_bins, int ring_bytes = 0, bool pooled = false) {
         const bool ring = ring_bytes > 0;
         int o = 0;
         auto take = [&o](int bytes) { int r = o; o += (bytes + 127) & ~127; return r; };
         n_sig = (T + 1) / 2 < kMaxSignals ? (T + 1) / 2 : kMaxSignals;
-        img_off = take(rows * kPitch * 4);
-        tw_off = take(kAz * 8);
-        // The second FFT buffer may reuse the image: once the (single) batch of signals has been
-        // loaded from the image into fa, the image is dead.
         const int sig_bytes = n_sig * kAz * 8;
-        const bool fb_on_img = (T + 1) / 2 <= kMaxSignals && rows * kPitch * 4 >= sig_bytes;
-        const int scratch = fb_on_img ? sig_bytes : 2 * sig_bytes;
-        ring_off = take(ring && ring_bytes > scratch ? ring_bytes : scratch);
-        fa_off = ring_off;
-        fb_off = fb_on_img ? img_off : ring_off + sig_bytes;
+        if (pooled) {
+            const int pooled_bytes = (T * kPitch * 4 + 127) & ~127;
+            const int img_bytes = rows * kPitch * 4;
+            img_off = take(img_bytes > pooled_bytes + 2 * sig_bytes ? img_bytes : pooled_bytes + 2 * sig_bytes);
+            tw_off = take(kAz * 8);
+            ring_off = fa_off = img_off + pooled_bytes;
+            fb_off = fa_off + sig_bytes;
+        } else {
+            img_off = take(rows * kPitch * 4);
+            tw_off = take(kAz * 8);
+            // The second FFT buffer may reuse the image: once the (single) batch of signals has
+            // been loaded from the image into fa, the image is dead.
+            const bool fb_on_img = (T + 1) / 2 <= kMaxSignals && rows * kPitch * 4 >= sig_bytes;
+            const int scratch = fb_on_img ? sig_bytes : 2 * sig_bytes;
+            ring_off = take(ring && ring_bytes > scratch ? ring_bytes : scratch);
+            fa_off = ring_off;
+            fb_off = fb_on_img ? img_off : ring_off + sig_bytes;
+        }
         hist_off = take(T * n_bins * 4);
         mask_off = take(rows * kMaskWords * 4);
         nvalid_off = take(rows * 4);
@@ -236,6 +248,26 @@ __device__ __forceinline__ float pooled_value(const TailSmem& S, int rows, int T
     float sum = 0.0f;
     for (int r = r0; r < r1; ++r) sum += S.img[S.src[r] * kPitch + n];
     return sum / (float)(r1 - r0);
+}
+
+// The tall kernels' pooling (rows > T): rows 0..T-1 of S.img become the pooled rows, with
+// pooled_value's arithmetic, and S.src the identity, so that spectrum_and_bins(S, dp, T) reads
+// them and the FFT buffers may take the rows above (SmemLayout's `pooled` layout). First the
+// empty-row fill is written out (an empty row takes its source row's values; sources are never
+// empty, so no copy reads a copied row), then every thread pools one column upwards: target row i
+// reads rows >= floor(i * rows / T) >= i, none of which a smaller target has overwritten.
+template <typename G>
+__device__ __forceinline__ void pool_rows_in_place(const TailSmem& S, int rows, int T) {
+    for (int i = G::tid(); i < rows * kAz; i += G::kSize) {
+        const int r = i / kAz, c = i - r * kAz;
+        if (S.src[r] != r) S.img[r * kPitch + c] = S.img[S.src[r] * kPitch + c];
+    }
+    G::sync();
+    for (int r = G::tid(); r < rows; r += G::kSize) S.src[r] = r;
+    G::sync();
+    for (int n = G::tid(); n < kAz; n += G::kSize)
+        for (int i = 0; i < T; ++i) S.img[i * kPitch + n] = pooled_value(S, rows, T, i, n);
+    G::sync();
 }
 
 // One Stockham pass of radix R over n_sig complex signals of length 360: one thread per

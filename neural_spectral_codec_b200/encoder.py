@@ -62,6 +62,7 @@ class RangeImageProjector:
 
     # -- helpers shared with SpectralEncoder ------------------------------------------------
     def _fill_params(self, p: _lib.NscParams) -> None:
+        p.flags = _lib.FLAG_TALL_IMAGES       # this package handles images of up to 128 rows
         p.n_elevation = int(self.n_elevation)
         p.n_azimuth = int(self.n_azimuth)
         p.min_range = float(self.min_range)
@@ -154,7 +155,7 @@ def _workspace(dev: torch.device, stream: int, p: "_lib.NscParams", n_scans: int
 def _anywidth_workspace(dev: torch.device, stream: int, p: "_lib.NscParams", n: int, rows: int) -> torch.Tensor:
     need = int(_lib.load().nsc_anywidth_workspace_bytes(n, rows, C.byref(p)))
     if need == 0:
-        raise ValueError("encoder geometry outside the supported envelope (rows <= 64, 2 <= n_azimuth <= 4096, "
+        raise ValueError("encoder geometry outside the supported envelope (rows <= 128, 2 <= n_azimuth <= 4096, "
                          "n_bins <= n_azimuth // 2 + 1)")
     key = (dev.index if dev.index is not None else torch.cuda.current_device(), stream, "anywidth")
     ws = _WORKSPACES.get(key)
@@ -545,6 +546,7 @@ def interpolate_range_image(range_image: Union[np.ndarray, torch.Tensor], method
         p = _lib.NscParams()
         lib.nsc_default_params(C.byref(p))
         p.n_azimuth, p.n_elevation, p.target_rows, p.n_bins = int(x.shape[2]), int(x.shape[1]), 1, 1
+        p.flags = _lib.FLAG_TALL_IMAGES
         if x.shape[0]:
             _anywidth_images(x, p, None, 1 if method == "nearest" else 0, None, out)
         if single:

@@ -1,6 +1,12 @@
 #!/usr/bin/env python
 """Per-phase cycle counts of the persistent encode kernel (tuning build:
-make -C neural_spectral_codec_b200/csrc VARIANT=phase DEFS=-DNSC_PHASE_TIMING, NSC_LIB=...)."""
+make -C neural_spectral_codec_b200/csrc VARIANT=phase DEFS=-DNSC_PHASE_TIMING, NSC_LIB=...).
+
+    python tools/phase_timing.py [shape] [n_elevation]      (default: hdl64 16)
+
+The generic and the tall kernels count phases; the warp-specialised one does not, so at 16 rows
+run it with the tuning variant's NSC_WS=0. For images of more than 64 rows the in-place pooling
+counts as part of "load signals"."""
 import ctypes as C
 import os
 import sys
@@ -11,8 +17,10 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from neural_spectral_codec_b200 import SpectralEncoder, _lib, synth  # noqa: E402
 
 shape = synth.SHAPES[sys.argv[1] if len(sys.argv) > 1 else "hdl64"]
+rows = int(sys.argv[2]) if len(sys.argv) > 2 else 16
 n = 1184                      # 4 scans per CTA
-enc = SpectralEncoder(n_elevation=16, target_elevation_bins=16).to("cuda")
+enc = SpectralEncoder(n_elevation=rows, target_elevation_bins=16,
+                      elevation_range=(shape.el_lo_deg, shape.el_hi_deg) if rows > 16 else (-24.8, 2.0)).to("cuda")
 pts, offs = synth.make_batch(shape, 0, n, device="cuda")
 out = torch.empty((n, 800), device="cuda")
 ws = torch.zeros(64, dtype=torch.int32, device="cuda")
