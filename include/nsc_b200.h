@@ -320,7 +320,8 @@ int nsc_wasserstein_cdf(const float* d_hists, int64_t n_rows, int n_bins, float 
  *   top_k          0 = distances only; else <= 1024: d_top_idx int64[n_queries * top_k] (-1
  *                  padded), d_top_dist float32 (ascending, +inf padded), d_top_count
  *                  int32[n_queries] = min(top_k, rows not excluded). Ties are broken by the
- *                  lower database index (deterministic).
+ *                  lower database index (deterministic). Larger top_k (up to the whole database):
+ *                  nsc_wasserstein_rank below, which returns the same results for top_k <= 1024.
  *   d_workspace    nsc_wasserstein_workspace_bytes(n_queries) bytes, ZERO before the first call
  *                  (every call leaves it zero where it matters). With it, top_k <= 128 is selected
  *                  by many CTAs per query from per-warp minima kept by the distance pass; NULL or
@@ -355,6 +356,37 @@ int nsc_wasserstein_query_u16(const float* d_query_hists, int n_queries, const u
                               const double* d_query_xyz, double min_spatial_distance,
                               float* d_distances, int top_k, int64_t* d_top_idx, float* d_top_dist,
                               int32_t* d_top_count, void* d_workspace, size_t workspace_bytes, void* stream);
+
+/* Any top_k, up to the whole database and beyond: the reference's TwoStageRetrieval._global_retrieval
+ * asks for every keyframe (top_k = len(keyframes), two_stage_retrieval.py:181-185).
+ * nsc_wasserstein_rank / nsc_wasserstein_rank_u16 take the arguments of nsc_wasserstein_query /
+ * nsc_wasserstein_query_u16 with a 64-bit top_k, run the same distance pass (d_distances bit-identical)
+ * and then rank each query's rows with a stable radix sort. Results, for every top_k:
+ *   - the order is that of the key (distance bit pattern as uint32, row index), ascending: equal
+ *     distances go to the lower row, +inf (excluded rows) and NaN last; the selection of
+ *     nsc_wasserstein_query follows the same rule;
+ *   - d_top_count[q] = min(top_k, finite distances of query q); entries at or past it are -1 / +inf,
+ *     including those past n_db when top_k > n_db;
+ *   - top_k = 0: distances only; n_queries = 0: nothing.
+ * Validation, before any CUDA call: n_queries < 0, n_db < 0 or >= 2^32, top_k < 0 -> NSC_ERR_BAD_COUNT;
+ * n_bins outside 1..1024 -> NSC_ERR_BAD_PARAMS; then the pointers of nsc_wasserstein_query ->
+ * NSC_ERR_NULL_POINTER; then, when top_k > 0, a workspace that is NULL or smaller than
+ * nsc_wasserstein_rank_workspace_bytes(n_queries, n_db) -> NSC_ERR_WORKSPACE.
+ * The workspace (O(n_queries * n_db): keys and rows twice plus per-tile counts) needs no
+ * initialisation and carries nothing between calls. nsc_wasserstein_rank_workspace_bytes returns 0
+ * for negative arguments and n_db >= 2^32, SIZE_MAX where the size does not fit a size_t. All work is
+ * queued on `stream`: no synchronisation, no allocation. */
+size_t nsc_wasserstein_rank_workspace_bytes(int n_queries, int64_t n_db);
+int nsc_wasserstein_rank(const float* d_query_hists, int n_queries, const float* d_db_cdfs,
+                         int64_t n_db, int n_bins, float epsilon, const double* d_db_xyz,
+                         const double* d_query_xyz, double min_spatial_distance,
+                         float* d_distances, int64_t top_k, int64_t* d_top_idx, float* d_top_dist,
+                         int32_t* d_top_count, void* d_workspace, size_t workspace_bytes, void* stream);
+int nsc_wasserstein_rank_u16(const float* d_query_hists, int n_queries, const uint16_t* d_db_cdf16,
+                             int64_t n_db, int n_bins, float epsilon, const double* d_db_xyz,
+                             const double* d_query_xyz, double min_spatial_distance,
+                             float* d_distances, int64_t top_k, int64_t* d_top_idx, float* d_top_dist,
+                             int32_t* d_top_count, void* d_workspace, size_t workspace_bytes, void* stream);
 
 /* ---- descriptor wire format (SURVEY.md 8(f), fourth "next" row) --------------------------- */
 /* Replaces HistogramQuantizer.quantize / dequantize (reference src/encoding/quantization.py

@@ -94,6 +94,11 @@ SYMBOLS = {
     "nsc_wasserstein_cdf_u16": (_I, [_VP, _I64, _I, _VP, _VP]),
     "nsc_wasserstein_query_u16": (_I, [_VP, _I, _VP, _I64, _I, C.c_float, _VP, _VP, C.c_double, _VP, _I,
                                        _VP, _VP, _VP, _VP, _SZ, _VP]),
+    "nsc_wasserstein_rank_workspace_bytes": (_SZ, [_I, _I64]),
+    "nsc_wasserstein_rank": (_I, [_VP, _I, _VP, _I64, _I, C.c_float, _VP, _VP, C.c_double, _VP, _I64,
+                                  _VP, _VP, _VP, _VP, _SZ, _VP]),
+    "nsc_wasserstein_rank_u16": (_I, [_VP, _I, _VP, _I64, _I, C.c_float, _VP, _VP, C.c_double, _VP, _I64,
+                                      _VP, _VP, _VP, _VP, _SZ, _VP]),
     "nsc_quantize_histograms": (_I, [_VP, _I64, _I, C.c_float, _VP, _VP]),
     "nsc_dequantize_histograms": (_I, [_VP, _I64, _I, C.c_float, _VP, _VP]),
     "nsc_test_pairwise_sum_plan": (_I, [_I, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),

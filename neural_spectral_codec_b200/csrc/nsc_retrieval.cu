@@ -15,6 +15,8 @@
 //                          resolved by that CTA with an exact 8-pass radix select of the 64-bit keys)
 //   topk_kernel            128 < k <= 1024: one CTA per query, per-thread-minimum bound + candidate
 //                          sort, 4-pass radix select as the last resort
+// and, for nsc_wasserstein_rank (any k), a stable segmented radix sort of each query's distances:
+// rank_hist_kernel, rank_scan_kernel, rank_scatter_kernel (see "rank" below).
 #include <math.h>
 
 #include "nsc_internal.h"
@@ -679,12 +681,245 @@ topk_kernel(const __grid_constant__ TopkArgs a) {
     if (tid == 0) a.top_count[q] = (int)k;
 }
 
+// ---- rank: every row of the database in order -----------------------------------------------
+// nsc_wasserstein_rank orders each query's distances with a stable LSD radix sort of the 32-bit
+// patterns, the row index riding along as payload (distances are >= 0, +inf or NaN, so unsigned
+// order is numeric order with NaN last). A tile of kRankTile keys never straddles two queries.
+// Every pass is three launches:
+//   rank_hist_kernel     digit counts of each tile
+//   rank_scan_kernel     one CTA per query: exclusive scan of its counts, digit-major, which gives
+//                        every (digit, tile) its first output position
+//   rank_scatter_kernel  stable rank inside the tile (per-warp digit counters, match_any within a
+//                        round of 32 keys), then the scatter of keys and rows
+// The first pass reads the keys straight from the distances (row = position); rows enter in index
+// order and every pass is stable, so equal distances stay in row order. The last pass writes only
+// the ranks below min(top_k, finite keys) into the outputs, its scan the padding and the count.
+#ifndef NSC_RANK_BITS
+#define NSC_RANK_BITS 8                // 8 or 11: DESIGN.md §7 has the measurement
+#endif
+constexpr int kRankBits = NSC_RANK_BITS;
+static_assert(kRankBits == 8 || kRankBits == 11, "digit width");
+constexpr int kRadix = 1 << kRankBits;
+constexpr int kRankPasses = (32 + kRankBits - 1) / kRankBits;
+constexpr int kRankThreads = 256;
+constexpr int kRankWarps = kRankThreads / 32;
+constexpr int kRankItems = 16;                          // keys per thread
+constexpr long long kRankTile = kRankThreads * kRankItems;
+constexpr int kScanThreads = 1024;
+constexpr int kScanItems = 8;
+constexpr unsigned kInfBits = 0x7f800000u;
+constexpr int kMaxGridY = 65535;                        // queries per launch
+
+struct RankArgs {
+    const unsigned* src_keys;   // Q x N; the first pass reads the distances' bits
+    const unsigned* src_rows;   // Q x N; null on the first pass (row = position)
+    unsigned* dst_keys;         // Q x N; unused on the last pass
+    unsigned* dst_rows;
+    unsigned* hist;             // Q x kRadix x n_tiles: counts, then first output positions
+    unsigned* finite;           // Q x n_tiles: finite keys per tile (first pass)
+    unsigned* n_finite;         // Q
+    long long n_db;
+    long long k;
+    long long* top_idx;         // Q x k
+    float* top_dist;
+    int* top_count;
+    int q0;                     // first query of the launch
+    int n_tiles;
+    int shift;
+    int first, last;
+};
+
+__global__ void __launch_bounds__(kRankThreads)
+rank_hist_kernel(const __grid_constant__ RankArgs a) {
+    __shared__ unsigned h[kRadix];
+    __shared__ unsigned s_fin;
+    const int lane = threadIdx.x & 31;
+    const long long q = a.q0 + (long long)blockIdx.y, lo = (long long)blockIdx.x * kRankTile;
+    const int n = (int)(a.n_db - lo < kRankTile ? a.n_db - lo : kRankTile);
+    for (int i = threadIdx.x; i < kRadix; i += kRankThreads) h[i] = 0;
+    if (threadIdx.x == 0) s_fin = 0;
+    const unsigned* keys = a.src_keys + q * a.n_db + lo;
+    unsigned key[kRankItems];
+#pragma unroll
+    for (int i = 0; i < kRankItems; ++i) {
+        const int e = i * kRankThreads + threadIdx.x;
+        key[i] = e < n ? keys[e] : 0u;
+    }
+    __syncthreads();
+    unsigned fin = 0;
+#pragma unroll
+    for (int i = 0; i < kRankItems; ++i) {
+        const bool act = i * kRankThreads + (int)threadIdx.x < n;
+        const unsigned amask = __ballot_sync(0xffffffffu, act);
+        if (act) {
+            const unsigned d = (key[i] >> a.shift) & (kRadix - 1);
+            const unsigned peers = __match_any_sync(amask, d);      // ties share digits: one atomic per digit
+            if (lane == __ffs(peers) - 1) atomicAdd(&h[d], (unsigned)__popc(peers));
+            fin += key[i] < kInfBits;
+        }
+    }
+    if (a.first) {
+        fin = __reduce_add_sync(0xffffffffu, fin);
+        if (lane == 0 && fin) atomicAdd(&s_fin, fin);
+    }
+    __syncthreads();
+    unsigned* out = a.hist + q * kRadix * a.n_tiles + blockIdx.x;
+    for (int d = threadIdx.x; d < kRadix; d += kRankThreads) out[(long long)d * a.n_tiles] = h[d];
+    if (a.first && threadIdx.x == 0) a.finite[q * a.n_tiles + blockIdx.x] = s_fin;
+}
+
+__global__ void __launch_bounds__(kScanThreads)
+rank_scan_kernel(const __grid_constant__ RankArgs a) {
+    __shared__ __align__(16) unsigned s[kScanThreads * kScanItems];
+    __shared__ unsigned warp_tot[32];
+    __shared__ unsigned s_total, s_fin;
+    const int tid = threadIdx.x;
+    const long long q = a.q0 + (long long)blockIdx.x;
+    const long long n = (long long)kRadix * a.n_tiles;
+    unsigned* h = a.hist + q * n;
+    unsigned carry = 0;
+    for (long long base = 0; base < n; base += kScanThreads * kScanItems) {
+        for (int i = tid; i < kScanThreads * kScanItems; i += kScanThreads) s[i] = base + i < n ? h[base + i] : 0u;
+        __syncthreads();
+        uint4* s4 = reinterpret_cast<uint4*>(s) + tid * (kScanItems / 4);
+        const uint4 v0 = s4[0], v1 = s4[1];
+        const unsigned v[kScanItems] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
+        unsigned sum = 0;
+#pragma unroll
+        for (int j = 0; j < kScanItems; ++j) sum += v[j];
+        unsigned run = block_excl_scan(sum, warp_tot, &s_total) + carry;     // ends with a barrier
+        unsigned o[kScanItems];
+#pragma unroll
+        for (int j = 0; j < kScanItems; ++j) { o[j] = run; run += v[j]; }
+        s4[0] = make_uint4(o[0], o[1], o[2], o[3]);
+        s4[1] = make_uint4(o[4], o[5], o[6], o[7]);
+        carry += s_total;
+        __syncthreads();
+        for (int i = tid; i < kScanThreads * kScanItems; i += kScanThreads)
+            if (base + i < n) h[base + i] = s[i];
+        __syncthreads();
+    }
+    if (a.first) {
+        unsigned f = 0;
+        for (int t = tid; t < a.n_tiles; t += kScanThreads) f += a.finite[q * a.n_tiles + t];
+        f = block_excl_scan(f, warp_tot, &s_total);
+        if (tid == 0) { s_fin = s_total; a.n_finite[q] = s_total; }
+        __syncthreads();
+    }
+    if (a.last) {
+        const long long nf = a.first ? s_fin : a.n_finite[q];
+        const long long c = a.k < nf ? a.k : nf;
+        for (long long r = c + tid; r < a.k; r += kScanThreads) {
+            a.top_idx[q * a.k + r] = -1;
+            a.top_dist[q * a.k + r] = INFINITY;
+        }
+        if (tid == 0) a.top_count[q] = (int)c;
+    }
+}
+
+__global__ void __launch_bounds__(kRankThreads)
+rank_scatter_kernel(const __grid_constant__ RankArgs a) {
+    extern __shared__ unsigned rank_cnt[];              // kRankWarps x kRadix
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long q = a.q0 + (long long)blockIdx.y, lo = (long long)blockIdx.x * kRankTile;
+    const int n = (int)(a.n_db - lo < kRankTile ? a.n_db - lo : kRankTile);
+    unsigned* wc = rank_cnt + warp * kRadix;
+    for (int i = lane; i < kRadix; i += 32) wc[i] = 0;
+    // warp w owns the tile's keys [w0, w0 + 32 * kRankItems), 32 consecutive ones per round
+    const int w0 = warp * 32 * kRankItems;
+    const unsigned* keys = a.src_keys + q * a.n_db + lo;
+    const unsigned* rows = a.src_rows ? a.src_rows + q * a.n_db + lo : nullptr;
+    unsigned key[kRankItems], row[kRankItems], pos[kRankItems];
+#pragma unroll
+    for (int i = 0; i < kRankItems; ++i) {
+        const int e = w0 + i * 32 + lane;
+        key[i] = e < n ? keys[e] : 0u;
+        row[i] = e < n ? (rows ? rows[e] : (unsigned)(lo + e)) : 0u;
+    }
+    __syncwarp();
+    // rank among the warp's keys of the same digit, in position order
+#pragma unroll
+    for (int i = 0; i < kRankItems; ++i) {
+        const bool act = w0 + i * 32 + lane < n;
+        const unsigned amask = __ballot_sync(0xffffffffu, act);
+        if (act) {
+            const unsigned d = (key[i] >> a.shift) & (kRadix - 1);
+            const unsigned peers = __match_any_sync(amask, d);
+            const int leader = __ffs(peers) - 1;
+            unsigned base = 0;
+            if (lane == leader) {
+                base = wc[d];
+                wc[d] = base + __popc(peers);
+            }
+            pos[i] = __shfl_sync(amask, base, leader) + __popc(peers & ((1u << lane) - 1));
+        }
+        __syncwarp();
+    }
+    __syncthreads();
+    // each warp's first output position per digit: the tile's (rank_scan_kernel), then the lower warps'
+    const unsigned* start = a.hist + q * kRadix * a.n_tiles + blockIdx.x;
+    for (int d = threadIdx.x; d < kRadix; d += kRankThreads) {
+        unsigned run = start[(long long)d * a.n_tiles];
+#pragma unroll
+        for (int w = 0; w < kRankWarps; ++w) {
+            const unsigned c = rank_cnt[w * kRadix + d];
+            rank_cnt[w * kRadix + d] = run;
+            run += c;
+        }
+    }
+    __syncthreads();
+    if (!a.last) {
+#pragma unroll
+        for (int i = 0; i < kRankItems; ++i)
+            if (w0 + i * 32 + lane < n) {
+                const long long p = q * a.n_db + wc[(key[i] >> a.shift) & (kRadix - 1)] + pos[i];
+                a.dst_keys[p] = key[i];
+                a.dst_rows[p] = row[i];
+            }
+    } else {
+        const long long nf = a.n_finite[q];
+        const long long c = a.k < nf ? a.k : nf;
+#pragma unroll
+        for (int i = 0; i < kRankItems; ++i)
+            if (w0 + i * 32 + lane < n) {
+                const long long p = (long long)wc[(key[i] >> a.shift) & (kRadix - 1)] + pos[i];
+                if (p < c) {
+                    a.top_idx[q * a.k + p] = row[i];
+                    a.top_dist[q * a.k + p] = __uint_as_float(key[i]);
+                }
+            }
+    }
+}
+
 int sm_count(int* sms) {
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return record_cuda(e);
     e = cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
     return e == cudaSuccess ? NSC_OK : record_cuda(e);
+}
+
+// Workspace of the rank, in 256-byte aligned regions: keys and rows twice (ping-pong), the tile
+// counts, the finite keys per tile and per query. size = SIZE_MAX where that does not fit a size_t.
+struct RankLayout {
+    size_t keys[2], rows[2], hist, finite, n_finite, size;
+};
+
+RankLayout rank_layout(long long n_queries, long long n_db) {
+    RankLayout l{};
+    const unsigned __int128 tiles = (n_db + kRankTile - 1) / kRankTile;
+    const unsigned __int128 sizes[7] = {(unsigned __int128)n_queries * n_db * 4, (unsigned __int128)n_queries * n_db * 4,
+                                        (unsigned __int128)n_queries * n_db * 4, (unsigned __int128)n_queries * n_db * 4,
+                                        (unsigned __int128)n_queries * kRadix * tiles * 4,
+                                        (unsigned __int128)n_queries * tiles * 4, (unsigned __int128)n_queries * 4};
+    size_t* at[7] = {&l.keys[0], &l.rows[0], &l.keys[1], &l.rows[1], &l.hist, &l.finite, &l.n_finite};
+    unsigned __int128 off = 0;
+    for (int i = 0; i < 7; ++i) {
+        *at[i] = (size_t)off;
+        off += (sizes[i] + 255) / 256 * 256;
+    }
+    l.size = off > (unsigned __int128)SIZE_MAX ? SIZE_MAX : (size_t)off;
+    return l;
 }
 
 }  // namespace
@@ -736,6 +971,11 @@ size_t nsc_wasserstein_workspace_bytes(int n_queries) {
     if (n_queries < 0) return 0;
     const size_t per_query = 16 + (size_t)kSelCap * 8 + (size_t)kMaxDistGrid * kRWarps * 8;
     return (size_t)n_queries * per_query + 256;
+}
+
+size_t nsc_wasserstein_rank_workspace_bytes(int n_queries, int64_t n_db) {
+    if (n_queries < 0 || n_db < 0 || n_db >= (1ll << 32)) return 0;
+    return rank_layout(n_queries, n_db).size;
 }
 
 }  // extern "C"
@@ -859,6 +1099,68 @@ int wasserstein_query(const float* d_query_hists, int n_queries, const T* d_db_c
     return NSC_OK;
 }
 
+// nsc_wasserstein_rank and nsc_wasserstein_rank_u16: the distance pass of wasserstein_query, then
+// the radix sort of every query's distances
+template <typename T>
+int wasserstein_rank(const float* d_query_hists, int n_queries, const T* d_db_cdfs, int64_t n_db, int n_bins,
+                     float epsilon, const double* d_db_xyz, const double* d_query_xyz, double min_spatial_distance,
+                     float* d_distances, int64_t top_k, int64_t* d_top_idx, float* d_top_dist, int32_t* d_top_count,
+                     void* d_workspace, size_t workspace_bytes, void* stream) {
+    if (n_queries < 0 || n_db < 0 || n_db >= (1ll << 32) || top_k < 0) return NSC_ERR_BAD_COUNT;
+    if (n_bins < 1 || n_bins > 32 * kMaxPerLane) return NSC_ERR_BAD_PARAMS;
+    if (n_queries == 0) return NSC_OK;
+    if (!d_query_hists || !d_distances) return NSC_ERR_NULL_POINTER;
+    if (n_db > 0 && !d_db_cdfs) return NSC_ERR_NULL_POINTER;
+    if (top_k > 0 && (!d_top_idx || !d_top_dist || !d_top_count)) return NSC_ERR_NULL_POINTER;
+    if ((d_db_xyz == nullptr) != (d_query_xyz == nullptr)) return NSC_ERR_NULL_POINTER;
+    const RankLayout l = rank_layout(n_queries, n_db);
+    if (top_k > 0 && (!d_workspace || workspace_bytes < l.size)) return NSC_ERR_WORKSPACE;
+    int st = wasserstein_query(d_query_hists, n_queries, d_db_cdfs, n_db, n_bins, epsilon, d_db_xyz, d_query_xyz,
+                               min_spatial_distance, d_distances, 0, nullptr, nullptr, nullptr, nullptr, 0, stream);
+    if (st != NSC_OK || top_k == 0) return st;
+    cudaStream_t s = (cudaStream_t)stream;
+    char* ws = static_cast<char*>(d_workspace);
+    const size_t scatter_smem = (size_t)kRankWarps * kRadix * 4;
+    if (scatter_smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(rank_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                   (int)scatter_smem);
+        if (e != cudaSuccess) return record_cuda(e);
+    }
+    RankArgs a{};
+    a.hist = reinterpret_cast<unsigned*>(ws + l.hist);
+    a.finite = reinterpret_cast<unsigned*>(ws + l.finite);
+    a.n_finite = reinterpret_cast<unsigned*>(ws + l.n_finite);
+    a.n_db = n_db;
+    a.k = top_k;
+    a.top_idx = (long long*)d_top_idx;
+    a.top_dist = d_top_dist;
+    a.top_count = d_top_count;
+    a.n_tiles = (int)((n_db + kRankTile - 1) / kRankTile);
+    // no rows (n_db = 0): one scan launch, which writes the padding and the counts
+    const int passes = n_db > 0 ? kRankPasses : 1;
+    for (int q0 = 0; q0 < n_queries; q0 += kMaxGridY) {
+        const int nq = n_queries - q0 < kMaxGridY ? n_queries - q0 : kMaxGridY;
+        a.q0 = q0;
+        for (int p = 0; p < passes; ++p) {
+            a.shift = p * kRankBits;
+            a.first = p == 0;
+            a.last = p == passes - 1;
+            a.src_keys = p == 0 ? reinterpret_cast<const unsigned*>(d_distances)
+                                : reinterpret_cast<const unsigned*>(ws + l.keys[(p - 1) & 1]);
+            a.src_rows = p == 0 ? nullptr : reinterpret_cast<const unsigned*>(ws + l.rows[(p - 1) & 1]);
+            a.dst_keys = reinterpret_cast<unsigned*>(ws + l.keys[p & 1]);
+            a.dst_rows = reinterpret_cast<unsigned*>(ws + l.rows[p & 1]);
+            const dim3 tiles(a.n_tiles, nq);
+            if (n_db > 0) rank_hist_kernel<<<tiles, kRankThreads, 0, s>>>(a);
+            rank_scan_kernel<<<nq, kScanThreads, 0, s>>>(a);
+            if (n_db > 0) rank_scatter_kernel<<<tiles, kRankThreads, scatter_smem, s>>>(a);
+            const cudaError_t e = cudaGetLastError();
+            if (e != cudaSuccess) return record_cuda(e);
+        }
+    }
+    return NSC_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -881,6 +1183,26 @@ int nsc_wasserstein_query_u16(const float* d_query_hists, int n_queries, const u
     return wasserstein_query(d_query_hists, n_queries, reinterpret_cast<const unsigned short*>(d_db_cdf16), n_db,
                              n_bins, epsilon, d_db_xyz, d_query_xyz, min_spatial_distance, d_distances, top_k,
                              d_top_idx, d_top_dist, d_top_count, d_workspace, workspace_bytes, stream);
+}
+
+int nsc_wasserstein_rank(const float* d_query_hists, int n_queries, const float* d_db_cdfs, int64_t n_db,
+                         int n_bins, float epsilon, const double* d_db_xyz, const double* d_query_xyz,
+                         double min_spatial_distance, float* d_distances, int64_t top_k, int64_t* d_top_idx,
+                         float* d_top_dist, int32_t* d_top_count, void* d_workspace, size_t workspace_bytes,
+                         void* stream) {
+    return wasserstein_rank(d_query_hists, n_queries, d_db_cdfs, n_db, n_bins, epsilon, d_db_xyz, d_query_xyz,
+                            min_spatial_distance, d_distances, top_k, d_top_idx, d_top_dist, d_top_count,
+                            d_workspace, workspace_bytes, stream);
+}
+
+int nsc_wasserstein_rank_u16(const float* d_query_hists, int n_queries, const uint16_t* d_db_cdf16, int64_t n_db,
+                             int n_bins, float epsilon, const double* d_db_xyz, const double* d_query_xyz,
+                             double min_spatial_distance, float* d_distances, int64_t top_k, int64_t* d_top_idx,
+                             float* d_top_dist, int32_t* d_top_count, void* d_workspace, size_t workspace_bytes,
+                             void* stream) {
+    return wasserstein_rank(d_query_hists, n_queries, reinterpret_cast<const unsigned short*>(d_db_cdf16), n_db,
+                            n_bins, epsilon, d_db_xyz, d_query_xyz, min_spatial_distance, d_distances, top_k,
+                            d_top_idx, d_top_dist, d_top_count, d_workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

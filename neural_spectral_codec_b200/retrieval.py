@@ -17,8 +17,14 @@ default stays float32, which keeps the unquantised distances. Rows and queries o
 into either database: uint16 rows are dequantised on the device, float rows going into a uint16
 database are quantised on the device, both with the retriever's ``epsilon``.
 
-All arithmetic runs in ``libnsc_b200.so`` (``nsc_wasserstein_cdf`` / ``nsc_wasserstein_query``);
-there is no CPU path.
+``query_batch`` accepts any ``top_k``, as the reference's ``query`` does: up to ``MAX_TOP_K`` = 1024
+the selection kernels of ``nsc_wasserstein_query`` pick the nearest rows; beyond that
+``nsc_wasserstein_rank`` orders the whole database with a stable radix sort on the device (the
+reference's ``_global_retrieval`` asks for every keyframe). Both give the order of (distance, lower
+row first).
+
+All arithmetic runs in ``libnsc_b200.so`` (``nsc_wasserstein_cdf`` / ``nsc_wasserstein_query`` /
+``nsc_wasserstein_rank``); there is no CPU path.
 """
 from __future__ import annotations
 
@@ -49,6 +55,7 @@ class WassersteinRetriever:
         self._cdfs: Optional[torch.Tensor] = None
         self._xyz: Optional[torch.Tensor] = None        # capacity x 3 float64 (NaN = unknown)
         self._ws: Optional[torch.Tensor] = None         # selection workspace (zero between calls)
+        self._rank_ws: Optional[torch.Tensor] = None    # rank workspace (k > MAX_TOP_K; needs no zeroing)
         self.database_size = 0
 
     # -- database ---------------------------------------------------------------------------
@@ -156,41 +163,38 @@ class WassersteinRetriever:
             q = self._convert(q, torch.empty(q.shape, dtype=torch.float32, device=self.device))
         q = q.contiguous()
         k = min(int(top_k), n)
-        # The select kernel holds its candidates in one CTA (k <= 1024). Larger k -- the reference's
-        # TwoStageRetrieval._global_retrieval asks for every keyframe, top_k = len(keyframes) -- takes
-        # the distance matrix of the same kernel and a stable device sort: the same (distance,
-        # lower index first) order.
-        k_kernel = k if k <= MAX_TOP_K else 0
         dist = torch.empty((nq, n), dtype=torch.float32, device=self.device)
         idx = torch.empty((nq, k), dtype=torch.int64, device=self.device)
         top = torch.empty((nq, k), dtype=torch.float32, device=self.device)
-        # every path below writes the counts, except the empty cases
-        cnt = (torch.empty if (n and nq and k_kernel) else torch.zeros)((nq,), dtype=torch.int32, device=self.device)
+        # every call below writes the counts, except the empty cases
+        cnt = (torch.empty if (n and nq and k) else torch.zeros)((nq,), dtype=torch.int32, device=self.device)
         if n and nq:
             use_xyz = query_positions is not None and spatial_filter_distance > 0
             qp = None
             if use_xyz:
                 qp = torch.as_tensor(query_positions, dtype=torch.float64).reshape(nq, 3).to(self.device).contiguous()
-            need = int(lib.nsc_wasserstein_workspace_bytes(nq))
-            if self._ws is None or self._ws.numel() < need:
-                self._ws = torch.zeros(need, dtype=torch.uint8, device=self.device)
-            name = "nsc_wasserstein_query_u16" if self.database_dtype == torch.uint16 else "nsc_wasserstein_query"
+            u16 = "_u16" if self.database_dtype == torch.uint16 else ""
+            if k <= MAX_TOP_K:
+                need = int(lib.nsc_wasserstein_workspace_bytes(nq))
+                if self._ws is None or self._ws.numel() < need:
+                    self._ws = torch.zeros(need, dtype=torch.uint8, device=self.device)
+                name, ws = "nsc_wasserstein_query" + u16, self._ws
+            else:
+                # the selection kernels hold k <= 1024 candidates per query; larger k (the reference's
+                # _global_retrieval asks for every keyframe) ranks the whole database
+                need = int(lib.nsc_wasserstein_rank_workspace_bytes(nq, n))
+                if self._rank_ws is None or self._rank_ws.numel() < need:
+                    self._rank_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+                name, ws = "nsc_wasserstein_rank" + u16, self._rank_ws
             with torch.cuda.device(self.device):
                 st = getattr(lib, name)(
                     q.data_ptr(), nq, self._cdfs.data_ptr(), n, q.shape[1], self.epsilon,
                     self._xyz.data_ptr() if use_xyz else None, qp.data_ptr() if use_xyz else None,
-                    float(spatial_filter_distance), dist.data_ptr(), k_kernel,
-                    idx.data_ptr() if k_kernel else None, top.data_ptr() if k_kernel else None,
-                    cnt.data_ptr() if k_kernel else None, self._ws.data_ptr(), self._ws.numel(),
+                    float(spatial_filter_distance), dist.data_ptr(), k,
+                    idx.data_ptr() if k else None, top.data_ptr() if k else None,
+                    cnt.data_ptr() if k else None, ws.data_ptr(), ws.numel(),
                     torch.cuda.current_stream(self.device).cuda_stream)
             _lib.check(st, name)
-            if k > MAX_TOP_K:
-                sd, si = torch.sort(dist, dim=1, stable=True)
-                top, idx = sd[:, :k].contiguous(), si[:, :k].contiguous()
-                cnt = torch.isfinite(dist).sum(1).clamp(max=k).to(torch.int32)
-                beyond = torch.arange(k, device=self.device).unsqueeze(0) >= cnt.unsqueeze(1)
-                idx[beyond] = -1
-                top[beyond] = float("inf")
         if return_distances:
             return idx, top, cnt, dist
         return idx, top, cnt
