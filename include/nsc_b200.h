@@ -208,10 +208,15 @@ int nsc_interpolate_range_images(const float* d_images_in, int n_images, int row
 /* ---- image widths other than 360 columns ----------------------------------------------------
  * The reference accepts any n_azimuth (spectral_encoder.py:35-47, range_image.py:102-127); every
  * shipped config uses 360, which the entry points above are specialised to (they refuse other
- * widths with NSC_ERR_BAD_PARAMS). These two cover 2 <= n_azimuth <= 4096 with one general kernel
- * (the reference's own operation order for the projection, a direct float64 DFT per row): same
- * results to the same tolerances, ~0.1-0.3 ms per scan instead of ~0.3 us. h_lut has
- * n_azimuth / 2 + 1 entries. Workspace: nsc_anywidth_workspace_bytes(n, rows, p).
+ * widths with NSC_ERR_BAD_PARAMS). These two cover 2 <= n_azimuth <= 4096 with two kernels and the
+ * same results to the same tolerances. A call with d_out set, a width whose prime factors are all at
+ * most 13 and an image that fits one block's shared memory (nsc_test_anywidth_path) runs a fused
+ * kernel: image, fp32 mixed-radix FFT and histogram in shared memory, ~1.5 us per scan on a whole
+ * B200 (about a fifth of the 360-column rate). Every other call runs a general kernel (the
+ * reference's own operation order for the projection, a direct float64 DFT per row), ~0.1-0.3 ms
+ * per scan per CTA. Both give bit-identical range images. h_lut has
+ * n_azimuth / 2 + 1 entries. Workspace: nsc_anywidth_workspace_bytes(n, rows, p), enough for both
+ * kernels, needs no initialisation.
  *   nsc_anywidth_points  encode_points / project [+ interpolate_range_image] for n_scans scans:
  *       d_out (descriptors, float32[n_scans * target_rows * n_bins]) and / or d_images
  *       (float32[n_scans * n_elevation * n_azimuth], the image named by `stage`); either may be NULL
@@ -410,6 +415,14 @@ int nsc_test_host_classify(const float* h_points, int point_stride, int64_t n_po
                            const nsc_params* p, int32_t* h_row, int32_t* h_col, uint8_t* h_keep);
 /* 0 = polynomial row assignment, 1 = threshold search (wide fields of view); < 0 = status. */
 int nsc_test_row_mode(const nsc_params* p);
+/* Which kernel nsc_anywidth_points / nsc_anywidth_images run for images of `rows` rows under p,
+ * with (want_descriptor != 0) or without a descriptor output: 1 = the fused shared-memory kernel,
+ * 0 = the general kernel, < 0 = status (the entry points' parameter checks). Host only. */
+int nsc_test_anywidth_path(const nsc_params* p, int rows, int want_descriptor);
+/* The fused kernel's W-point complex forward FFT (its plan and radix passes, twiddles in float32)
+ * run on the host: h_in and h_out hold W interleaved (re, im) float pairs. NSC_ERR_BAD_PARAMS for W
+ * outside 2..4096 or with a prime factor above 13. */
+int nsc_test_anywidth_fft(int W, const float* h_in, float* h_out);
 /* The summation plan the quantiser kernels follow for rows of n_bins elements (host only, no CUDA
  * call): leaves [leaf_start[l], leaf_start[l] + leaf_len[l]) for l < *n_leaves, each summed with
  * NumPy's 8 strided accumulators, then *n_adds additions in single-assignment form -- addition t

@@ -104,6 +104,8 @@ SYMBOLS = {
     "nsc_test_pairwise_sum_plan": (_I, [_I, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     "nsc_test_host_classify": (_I, [_VP, _I, _I64, _PP, _VP, _VP, _VP]),
     "nsc_test_row_mode": (_I, [_PP]),
+    "nsc_test_anywidth_path": (_I, [_PP, _I, _I]),
+    "nsc_test_anywidth_fft": (_I, [_I, _VP, _VP]),
 }
 
 _lib = None

@@ -2,9 +2,12 @@
 // (src/encoding/spectral_encoder.py:35-47, range_image.py:102-127); every shipped config uses 360,
 // which is what the fused kernels of nsc_encode.cu are specialised to (8*9*5 FFT plan, column
 // polynomial in units of 1 degree). This file keeps the class a drop-in for the other widths with
-// ONE general kernel that favours being obviously right over being fast:
+// two kernels behind nsc_anywidth_points / nsc_anywidth_images.
+//
+// The GENERAL kernel favours being obviously right over being fast, and serves every call:
 //   * projection with the reference's own float32 / float64 operation order (range_image.py:146-198)
-//     and CUDA's atan2f, per-pixel min by a 32-bit atomicMin on the bits of the range;
+//     and CUDA's atan2f, per-pixel min by a 32-bit atomicMin on the bits of the range
+//     (project_point_ref, nsc_anywidth.cuh);
 //   * hole interpolation ('linear' in float64 like np.interp, or 'nearest') and the empty-row fill
 //     (range_image.py:15-89) on a validity snapshot;
 //   * adaptive row pooling (spectral_encoder.py:171-176), a direct O(W^2) DFT per row in float64
@@ -12,11 +15,24 @@
 //     ascending frequency, L1 normalisation (spectral_encoder.py:180-202).
 // One CTA per scan / image, grid-stride; images and spectra live in a per-CTA global scratch
 // (L2-resident), the histogram in shared memory. ~0.1-0.3 ms per scan for W <= 1024.
+//
+// The FUSED kernel takes every call that computes descriptors when W has no prime factor above 13
+// and its shared-memory layout fits one block (choose_fused): the image, the FFT buffers, the
+// twiddles and the histogram live in shared memory, one 512-thread CTA per SM loops over the
+// scans. It projects with the same project_point_ref (shared-memory atomicMin), interpolates,
+// fills and pools with the general kernel's arithmetic (images and pooled rows bit-identical), and
+// takes the spectrum with an fp32 mixed-radix Stockham FFT, two pooled rows per complex transform,
+// bin sums straight from the spectrum and the general kernel's normalisation. The descriptors
+// agree with the general kernel's to the suite's tolerances.
 #include <math.h>
+#include <stdint.h>
+#include <stdlib.h>
 #include <string.h>
 
 #include <vector>
 
+#include "nsc_anywidth.cuh"
+#include "nsc_fft.cuh"
 #include "nsc_internal.h"
 
 namespace nsc {
@@ -25,26 +41,6 @@ namespace {
 
 constexpr int kGThreads = 256;
 constexpr int kMaxWidth = 4096;
-
-struct AnyArgs {
-    // input: points (CSR) or images
-    const float* points;
-    int stride;
-    const long long* offsets;
-    long long origin;
-    const float* images_in;    // n x rows x W, or null
-    int n;                     // scans or images
-    int E, W, T, F, n_bins;
-    int interpolate;           // 0 none, 1 linear, 2 nearest
-    float min_range, max_range, eps, uniform;
-    double el_min, el_max;
-    const int* bin_start;      // n_bins + 1 first frequencies (device)
-    float* out;                // n x T x n_bins, or null
-    float* images_out;         // n x E x W, or null
-    int stage;                 // NSC_STAGE_PROJECTED / NSC_STAGE_INTERPOLATED for images_out
-    unsigned char* scratch;    // per-CTA regions
-    size_t scratch_per_cta;
-};
 
 struct Scratch {
     float* img;          // E x W (key bits during the scatter)
@@ -74,30 +70,6 @@ struct Scratch {
         valid = base + o;
     }
 };
-
-// One point -> (pixel, range bits), range_image.py:146-198 in the reference's arithmetic:
-// float32 for range / azimuth / elevation / column, float64 for the row.
-__device__ __forceinline__ bool project_point_ref(float x, float y, float z, const AnyArgs& a, int& pix,
-                                                  unsigned& key) {
-    if (!(isfinite(x) && isfinite(y) && isfinite(z))) return false;                       // :151
-    const float x2 = fminf(fmaxf(__fmul_rn(x, x), 0.0f), 1e10f), y2 = fminf(fmaxf(__fmul_rn(y, y), 0.0f), 1e10f),
-                z2 = fminf(fmaxf(__fmul_rn(z, z), 0.0f), 1e10f);                          // :159-161
-    const float rho2 = __fadd_rn(x2, y2);
-    const float rng = __fsqrt_rn(__fadd_rn(rho2, z2));                                    // :162
-    if (!(rng >= a.min_range && rng <= a.max_range) || !isfinite(rng)) return false;      // :174
-    const float pi_f = 3.14159265358979323846f, two_pi_f = 6.28318530717958647692f;
-    float az = __fadd_rn(atan2f(y, x), pi_f);                                             // :166-167
-    if (az >= two_pi_f) az = __fsub_rn(az, two_pi_f);                                     // (az + pi) % 2 pi
-    const float el = atan2f(z, __fsqrt_rn(rho2));                                         // :170-171
-    const double frac = ((double)el - a.el_min) / (a.el_max - a.el_min);                  // :186 (float64)
-    double rowd = floor(frac * (double)a.E);
-    int row = rowd < 0.0 ? 0 : rowd > (double)(a.E - 1) ? a.E - 1 : (int)rowd;            // :187-191
-    const float cold = floorf(__fmul_rn(__fdiv_rn(az, two_pi_f), (float)a.W));            // :194
-    int col = cold < 0.0f ? 0 : cold > (float)(a.W - 1) ? a.W - 1 : (int)cold;            // :195-198
-    pix = row * a.W + col;
-    key = __float_as_uint(rng);
-    return true;
-}
 
 // ROWS: the capacity of the per-row arrays (kShortRows, or NSC_MAX_ELEVATION for taller images).
 template <int ROWS>
@@ -245,6 +217,404 @@ anywidth_kernel(const __grid_constant__ AnyArgs a) {
     }
 }
 
+// ================================================================================================
+// The fused kernel: the same stages with the image in shared memory and an fp32 FFT.
+//
+// A mixed-radix Stockham FFT of W points: pass p of radix R reads butterfly j's inputs
+// x[j + r * W / R], r < R, multiplies input r by exp(-2 pi i k r / (NS R)) with NS the product of
+// the earlier radices and k = j mod NS, takes an R-point DFT and writes output q to
+// y[(j / NS) * NS * R + k + q * NS]. Radices 8, 4, 2, 3, 5 have register butterflies
+// (nsc_fft.cuh); 7, 11 and 13 take the generic odd-prime butterfly. The pass code is
+// __host__ __device__ so that nsc_test_anywidth_fft runs it on the CPU.
+constexpr int kMaxPasses = 12;           // 4096 = 2^12
+
+struct FftPlan {
+    int n_pass;
+    int radix[kMaxPasses];
+};
+
+// Radices in pass order: 8s, then a 4 or a 2 for what remains of the power of two, then the odd
+// primes. False when W has a prime factor above 13.
+__host__ __device__ inline bool plan_fft(int W, FftPlan* p) {
+    p->n_pass = 0;
+    int w = W;
+    const int order[] = {8, 4, 2, 3, 5, 7, 11, 13};
+    for (int r : order)
+        while (w % r == 0 && p->n_pass < kMaxPasses) {
+            p->radix[p->n_pass++] = r;
+            w /= r;
+        }
+    return w == 1;
+}
+
+// exp(-2 pi i m / W) with m / W reduced exactly (as the general kernel's table), rounded to float2.
+__host__ __device__ inline float2 any_twiddle(int m, int W) {
+    double s, c;
+#ifdef __CUDA_ARCH__
+    sincospi(2.0 * (double)m / (double)W, &s, &c);
+#else
+    const double x = 2.0 * (double)m / (double)W;
+    s = sin(M_PI * x);
+    c = cos(M_PI * x);
+#endif
+    return make_float2((float)c, (float)-s);
+}
+
+// X[q] = sum_r a[r] w^(q r) for an odd prime R, w = exp(-2 pi i / R) = tw[W / R]: inputs paired as
+// t = a[r] + a[R-r], d = a[r] - a[R-r], outputs q and R - q from one cosine and one sine sum.
+template <int R>
+NSC_FFT_HD void dft_odd_prime_store(float2* a, const float2* tw, int m, float2* out, int ns) {
+    constexpr int H = (R - 1) / 2;
+    float2 x0 = a[0];
+#pragma unroll
+    for (int r = 1; r <= H; ++r) {
+        const float2 t = cadd(a[r], a[R - r]), d = csub(a[r], a[R - r]);
+        a[r] = t;
+        a[R - r] = d;
+        x0 = cadd(x0, t);
+    }
+    out[0] = x0;
+#pragma unroll 1
+    for (int q = 1; q <= H; ++q) {
+        float2 s = a[0], u = make_float2(0.0f, 0.0f);
+        int e = 0;                                            // q r mod R
+#pragma unroll
+        for (int r = 1; r <= H; ++r) {
+            e += q;
+            if (e >= R) e -= R;
+            const float2 w = tw[e * m];                       // (cos th, -sin th), th = 2 pi q r / R
+            s = make_float2(fmaf(a[r].x, w.x, s.x), fmaf(a[r].y, w.x, s.y));
+            u = make_float2(fmaf(-a[R - r].y, w.y, u.x), fmaf(a[R - r].x, w.y, u.y));   // -i d sin th
+        }
+        out[q * ns] = cadd(s, u);
+        out[(R - q) * ns] = csub(s, u);
+    }
+}
+
+template <int R>
+NSC_FFT_HD void any_butterfly(const float2* __restrict__ x, float2* __restrict__ y, const float2* __restrict__ tw,
+                              int W, int ns, int j) {
+    const int m = W / R;                      // butterflies per signal
+    const int blk = j / ns, k = j - blk * ns;
+    const int step = k * (m / ns);            // k * W / (ns * R)
+    float2 a[R];
+#pragma unroll
+    for (int r = 0; r < R; ++r) a[r] = x[j + r * m];
+    if (k) {
+#pragma unroll
+        for (int r = 1; r < R; ++r) a[r] = cmul(a[r], tw[r * step]);
+    }
+    float2* out = y + blk * ns * R + k;
+    if (R == 2) {
+        out[0] = cadd(a[0], a[1]);
+        out[ns] = csub(a[0], a[1]);
+        return;
+    }
+    if (R == 7 || R == 11 || R == 13) {
+        dft_odd_prime_store<R>(a, tw, m, out, ns);
+        return;
+    }
+    if (R == 3) dft3(a[0], a[1], a[2]);
+    else if (R == 4) dft4(a[0], a[1], a[2], a[3]);
+    else if (R == 5) dft5(a);
+    else dft8(a);
+#pragma unroll
+    for (int q = 0; q < R; ++q) out[q * ns] = a[q];
+}
+
+// Butterflies t0, t0 + step, ... of one pass over n_sig signals of W points each.
+template <int R>
+NSC_FFT_HD void any_pass(const float2* x, float2* y, const float2* tw, int W, int ns, int n_sig, int t0, int step) {
+    const int m = W / R;
+    for (int t = t0; t < n_sig * m; t += step) {
+        const int g = t / m, j = t - g * m;
+        any_butterfly<R>(x + g * W, y + g * W, tw, W, ns, j);
+    }
+}
+
+__host__ __device__ inline void fft_pass(int R, const float2* x, float2* y, const float2* tw, int W, int ns, int n_sig,
+                                         int t0, int step) {
+    switch (R) {
+        case 8: any_pass<8>(x, y, tw, W, ns, n_sig, t0, step); break;
+        case 4: any_pass<4>(x, y, tw, W, ns, n_sig, t0, step); break;
+        case 2: any_pass<2>(x, y, tw, W, ns, n_sig, t0, step); break;
+        case 3: any_pass<3>(x, y, tw, W, ns, n_sig, t0, step); break;
+        case 5: any_pass<5>(x, y, tw, W, ns, n_sig, t0, step); break;
+        case 7: any_pass<7>(x, y, tw, W, ns, n_sig, t0, step); break;
+        case 11: any_pass<11>(x, y, tw, W, ns, n_sig, t0, step); break;
+        default: any_pass<13>(x, y, tw, W, ns, n_sig, t0, step); break;
+    }
+}
+
+constexpr int kFThreads = 512;
+constexpr size_t kSmemOptIn = 227 * 1024;      // one block's opt-in shared memory on sm_100
+constexpr int kMaxFusedSignals = 8;            // row pairs transformed at once
+constexpr int kPtsInFlight = 4;                // point loads per thread before the first projection
+
+// Byte offsets of the fused kernel's shared memory.
+struct FusedLayout {
+    int n_sig;                  // complex signals (row pairs) per FFT batch
+    unsigned img;               // E x W range image (key bits during the scatter)
+    unsigned bits;              // E x ceil(W / 32) validity words (interpolation)
+    unsigned tw;                // W float2 twiddles
+    unsigned fa, fb;            // n_sig x W float2 each: the Stockham ping-pong
+    unsigned hist;              // T x n_bins bin sums
+    unsigned bstart;            // n_bins + 1 first frequencies
+    unsigned nvalid, src;       // E ints each: valid pixels per row, source row of the empty-row fill
+    unsigned red;               // kFThreads / 32 doubles
+    unsigned total;
+};
+
+inline FusedLayout fused_layout(int E, int W, int T, int n_bins, int n_sig) {
+    FusedLayout L;
+    size_t o = 0;
+    auto take = [&o](size_t bytes) {
+        const unsigned at = (unsigned)o;
+        o += (bytes + 15) & ~(size_t)15;
+        return at;
+    };
+    L.n_sig = n_sig;
+    L.red = take((kFThreads / 32) * 8);
+    L.img = take((size_t)E * W * 4);
+    L.bits = take((size_t)E * ((W + 31) / 32) * 4);
+    L.tw = take((size_t)W * 8);
+    L.fa = take((size_t)n_sig * W * 8);
+    L.fb = take((size_t)n_sig * W * 8);
+    L.hist = take((size_t)T * n_bins * 4);
+    L.bstart = take(((size_t)n_bins + 1) * 4);
+    L.nvalid = take((size_t)E * 4);
+    L.src = take((size_t)E * 4);
+    L.total = (unsigned)o;
+    return L;
+}
+
+// The choice between the kernels, from the arguments alone: the fused kernel needs a descriptor
+// to compute, a width whose prime factors are at most 13 and a layout with one row pair
+// that fits one block's shared memory (as many row pairs per batch as fit, up to
+// kMaxFusedSignals). Tuning builds (-DNSC_TUNING) take NSC_ANYWIDTH=0 to force the general kernel.
+bool choose_fused(const nsc_params* p, int rows, bool want_descriptor, FusedLayout* L, FftPlan* plan) {
+#ifdef NSC_TUNING
+    static const bool env_fused = [] { const char* e = getenv("NSC_ANYWIDTH"); return !(e && e[0] == '0'); }();
+    if (!env_fused) return false;
+#endif
+    if (!want_descriptor || !plan_fft(p->n_azimuth, plan)) return false;
+    const int T = p->target_rows, n_sig_total = (T + 1) / 2;
+    for (int s = n_sig_total < kMaxFusedSignals ? n_sig_total : kMaxFusedSignals; s >= 1; --s) {
+        *L = fused_layout(rows, p->n_azimuth, T, p->n_bins, s);
+        if (L->total <= kSmemOptIn) return true;
+    }
+    return false;
+}
+
+struct FusedArgs {
+    AnyArgs a;
+    FusedLayout L;
+    FftPlan plan;
+};
+
+// One scan's points into the key image: kPtsInFlight loads per thread in flight, then the
+// projections and shared-memory atomicMin on the range bits. VEC4: stride 4 from a 16-byte
+// aligned base, one float4 per point.
+template <bool VEC4>
+__device__ __forceinline__ void scatter_points(const AnyArgs& a, int item, unsigned* keys) {
+    const long long beg = a.offsets[item] - a.origin;
+    const int n = (int)(a.offsets[item + 1] - a.offsets[item]);
+    const float* p = a.points + beg * a.stride;
+    for (int i0 = threadIdx.x; i0 < n; i0 += kPtsInFlight * kFThreads) {
+        float x[kPtsInFlight], y[kPtsInFlight], z[kPtsInFlight];
+#pragma unroll
+        for (int u = 0; u < kPtsInFlight; ++u) {
+            const int i = i0 + u * kFThreads;
+            if (i < n) {
+                if (VEC4) {
+                    const float4 v = reinterpret_cast<const float4*>(p)[i];
+                    x[u] = v.x, y[u] = v.y, z[u] = v.z;
+                } else {
+                    const float* q = p + (size_t)i * a.stride;
+                    x[u] = q[0], y[u] = q[1], z[u] = q[2];
+                }
+            }
+        }
+#pragma unroll
+        for (int u = 0; u < kPtsInFlight; ++u) {
+            int pix;
+            unsigned key;
+            if (i0 + u * kFThreads < n && project_point_ref(x[u], y[u], z[u], a, pix, key)) atomicMin(keys + pix, key);
+        }
+    }
+}
+
+// The general kernel's pooling arithmetic (row t of the pooled image at column x).
+__device__ __forceinline__ float pooled_at(const float* img, const int* src, int E, int T, int W, int t, int x) {
+    if (E == T) return img[src[t] * W + x];
+    const int r0 = (t * E) / T, r1 = ((t + 1) * E + T - 1) / T;
+    float sum = 0.0f;
+    for (int r = r0; r < r1; ++r) sum += img[src[r] * W + x];
+    return sum / (float)(r1 - r0);
+}
+
+// Nearest set bit strictly left / right of column x in a circular row of W bits with at least one
+// set bit other than x's: the column the general kernel's pixel-by-pixel walk stops at.
+__device__ __forceinline__ int valid_left(const unsigned* row, int W, int x) {
+    int c = x == 0 ? W - 1 : x - 1;
+    for (;;) {
+        const unsigned v = row[c >> 5] & (0xffffffffu >> (31 - (c & 31)));
+        if (v) return (c & ~31) + 31 - __clz(v);
+        c = (c & ~31) - 1;
+        if (c < 0) c = W - 1;
+    }
+}
+__device__ __forceinline__ int valid_right(const unsigned* row, int W, int x) {
+    int c = x == W - 1 ? 0 : x + 1;
+    for (;;) {
+        const unsigned v = row[c >> 5] & (0xffffffffu << (c & 31));
+        if (v) return (c & ~31) + __ffs(v) - 1;
+        c = (c & ~31) + 32;
+        if (c >= W) c = 0;
+    }
+}
+
+template <bool VEC4>
+__global__ void __launch_bounds__(kFThreads, 1)
+anywidth_fused_kernel(const __grid_constant__ FusedArgs f) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const AnyArgs& a = f.a;
+    const FusedLayout& L = f.L;
+    float* img = reinterpret_cast<float*>(smem_raw + L.img);
+    unsigned* keys = reinterpret_cast<unsigned*>(img);
+    unsigned* bits = reinterpret_cast<unsigned*>(smem_raw + L.bits);
+    float2* tw = reinterpret_cast<float2*>(smem_raw + L.tw);
+    float2* fa = reinterpret_cast<float2*>(smem_raw + L.fa);
+    float2* fb = reinterpret_cast<float2*>(smem_raw + L.fb);
+    float* hist = reinterpret_cast<float*>(smem_raw + L.hist);
+    int* bstart = reinterpret_cast<int*>(smem_raw + L.bstart);
+    int* s_nvalid = reinterpret_cast<int*>(smem_raw + L.nvalid);
+    int* s_src = reinterpret_cast<int*>(smem_raw + L.src);
+    double* s_red = reinterpret_cast<double*>(smem_raw + L.red);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int E = a.E, W = a.W, T = a.T, nb = a.n_bins, D = T * nb, EW = E * W;
+    const int words = (W + 31) >> 5;
+    for (int m = tid; m < W; m += kFThreads) tw[m] = any_twiddle(m, W);
+    for (int b = tid; b <= nb; b += kFThreads) bstart[b] = a.bin_start[b];
+    for (int item = blockIdx.x; item < a.n; item += gridDim.x) {
+        __syncthreads();
+        // ---- the range image
+        if (a.images_in) {
+            const float* src = a.images_in + (size_t)item * EW;
+            for (int i = tid; i < EW; i += kFThreads) img[i] = src[i];
+        } else {
+            for (int i = tid; i < EW; i += kFThreads) keys[i] = kInfBits;
+            __syncthreads();
+            scatter_points<VEC4>(a, item, keys);
+            __syncthreads();
+            for (int i = tid; i < EW; i += kFThreads) {                                // empty -> 0
+                const unsigned k = keys[i];
+                img[i] = k == kInfBits ? 0.0f : __uint_as_float(k);
+            }
+        }
+        if (tid < E) { s_nvalid[tid] = 0; s_src[tid] = tid; }
+        __syncthreads();
+        if (a.images_out && a.stage == NSC_STAGE_PROJECTED)
+            for (int i = tid; i < EW; i += kFThreads) a.images_out[(size_t)item * EW + i] = img[i];
+        // ---- hole interpolation + empty-row fill: the general kernel's arithmetic on a bit snapshot
+        if (a.interpolate) {
+            for (int w = warp; w < E * words; w += kFThreads / 32) {
+                const int r = w / words, x = (w - r * words) * 32 + lane;
+                const unsigned v = __ballot_sync(0xffffffffu, x < W && img[r * W + x] > 0.0f);
+                if (lane == 0) {
+                    bits[w] = v;
+                    if (v) atomicAdd(&s_nvalid[r], __popc(v));
+                }
+            }
+            __syncthreads();
+            for (int i = tid; i < EW; i += kFThreads) {
+                const int r = i / W, x = i - r * W;
+                const int cnt = s_nvalid[r];
+                const unsigned* vr = bits + r * words;
+                if (cnt == 0 || cnt == W || ((vr[x >> 5] >> (x & 31)) & 1u)) continue;
+                const int il = valid_left(vr, W, x), ir = valid_right(vr, W, x);
+                const int dl = x - il + (il > x ? W : 0), dr = ir - x + (ir < x ? W : 0);
+                const float* row = img + r * W;
+                if (a.interpolate == 2) {
+                    img[i] = row[dl < dr || (dl == dr && il < ir) ? il : ir];
+                } else {
+                    const double fl = (double)row[il], fr = (double)row[ir];
+                    const double slope = __ddiv_rn(__dsub_rn(fr, fl), (double)(dl + dr));
+                    img[i] = __double2float_rn(__dadd_rn(__dmul_rn(slope, (double)dl), fl));
+                }
+            }
+            __syncthreads();
+            if (tid < E && s_nvalid[tid] == 0) {
+                int k = tid - 1;
+                while (k >= 0 && s_nvalid[k] == 0) --k;
+                if (k < 0) {
+                    k = tid + 1;
+                    while (k < E && s_nvalid[k] == 0) ++k;
+                }
+                if (k >= 0 && k < E) s_src[tid] = k;
+            }
+            __syncthreads();
+        }
+        if (a.images_out && a.stage == NSC_STAGE_INTERPOLATED)
+            for (int i = tid; i < EW; i += kFThreads) {
+                const int r = i / W, x = i - r * W;
+                a.images_out[(size_t)item * EW + i] = img[s_src[r] * W + x];
+            }
+        // ---- pooled rows 2g, 2g + 1 -> one complex FFT -> split by conjugate symmetry -> bin sums
+        const int n_sig_total = (T + 1) / 2;
+        for (int g0 = 0; g0 < n_sig_total; g0 += L.n_sig) {
+            const int n_sig = min(L.n_sig, n_sig_total - g0);
+            for (int t = tid; t < n_sig * W; t += kFThreads) {
+                const int g = t / W, x = t - g * W;
+                const int ra = 2 * (g0 + g), rb = ra + 1;
+                fa[t] = make_float2(pooled_at(img, s_src, E, T, W, ra, x),
+                                    rb < T ? pooled_at(img, s_src, E, T, W, rb, x) : 0.0f);
+            }
+            __syncthreads();
+            float2 *x = fa, *y = fb;
+            for (int p = 0, ns = 1; p < f.plan.n_pass; ++p) {
+                const int R = f.plan.radix[p];
+                fft_pass(R, x, y, tw, W, ns, n_sig, tid, kFThreads);
+                __syncthreads();
+                float2* t = x;
+                x = y;
+                y = t;
+                ns *= R;
+            }
+            // Z = FFT(a + i b): |A[k]| = |Z[k] + conj Z[-k]| / 2, |B[k]| = |Z[k] - conj Z[-k]| / 2,
+            // summed over each bin's frequencies in ascending k as they are computed
+            for (int i = tid; i < n_sig * 2 * nb; i += kFThreads) {
+                const int g = i / (2 * nb), rem = i - g * 2 * nb, h = rem >= nb, b = rem - h * nb;
+                const int row = 2 * (g0 + g) + h;
+                if (row >= T) continue;
+                const float2* z = x + g * W;
+                float s = 0.0f;
+                for (int k = bstart[b], k1 = bstart[b + 1]; k < k1; ++k) {
+                    const float2 p = z[k], m = z[k == 0 ? 0 : W - k];
+                    const float re = h ? p.y + m.y : p.x + m.x, im = h ? p.x - m.x : p.y - m.y;
+                    s += 0.5f * __fsqrt_rn(fmaf(re, re, im * im));
+                }
+                hist[row * nb + b] = s;
+            }
+            __syncthreads();
+        }
+        // ---- normalisation: the general kernel's rule (float64 total, __fdiv_rn by total + eps)
+        double acc = 0.0;
+        for (int i = tid; i < D; i += kFThreads) acc += (double)hist[i];
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, d);
+        if (lane == 0) s_red[warp] = acc;
+        __syncthreads();
+        double tot = 0.0;
+        for (int w = 0; w < kFThreads / 32; ++w) tot += s_red[w];
+        const float total = (float)tot;
+        const bool ok = total > a.eps;
+        const float denom = __fadd_rn(total, a.eps);
+        for (int i = tid; i < D; i += kFThreads)
+            a.out[(size_t)item * D + i] = ok ? __fdiv_rn(hist[i], denom) : a.uniform;
+    }
+}
+
 int validate_any(const nsc_params* p) {
     if (!p) return NSC_ERR_NULL_POINTER;
     if (p->struct_size != (int32_t)sizeof(nsc_params)) return NSC_ERR_BAD_STRUCT;
@@ -259,12 +629,13 @@ int validate_any(const nsc_params* p) {
     return NSC_OK;
 }
 
-int grid_for(int n, int* grid) {
+int grid_for(int n, int* grid, int* sms_out = nullptr) {
     int dev = 0, sms = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (e != cudaSuccess) return record_cuda(e);
     *grid = n < 2 * sms ? n : 2 * sms;
+    if (sms_out) *sms_out = sms;
     return NSC_OK;
 }
 constexpr int kMaxGrid = 1024;     // bounds the workspace without asking the device
@@ -283,8 +654,8 @@ int run(AnyArgs& a, const nsc_params* p, int rows, const int32_t* h_lut, void* w
     a.uniform = 1.0f / (float)(a.T * a.n_bins);
     a.el_min = p->el_min_rad;
     a.el_max = p->el_max_rad;
-    int grid = 0;
-    int st = grid_for(a.n, &grid);
+    int grid = 0, sms = 0;
+    int st = grid_for(a.n, &grid, &sms);
     if (st != NSC_OK) return st;
     if (grid > kMaxGrid) grid = kMaxGrid;
     const size_t per = Scratch::bytes(a.E, a.W, a.T, a.F);
@@ -306,6 +677,20 @@ int run(AnyArgs& a, const nsc_params* p, int rows, const int32_t* h_lut, void* w
         cudaError_t e = cudaMemcpyAsync(ws, start.data(), start.size() * 4, cudaMemcpyHostToDevice, s);
         if (e != cudaSuccess) return record_cuda(e);
     }
+    FusedArgs f;
+    if (choose_fused(p, rows, a.out != nullptr, &f.L, &f.plan)) {
+        // as many CTAs as fit on every SM, each looping over scans / images
+        f.a = a;
+        const bool vec4 = a.points && a.stride == 4 && ((uintptr_t)a.points & 15) == 0;
+        const auto kernel = vec4 ? anywidth_fused_kernel<true> : anywidth_fused_kernel<false>;
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)f.L.total);
+        int per_sm = 0;
+        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kFThreads, f.L.total);
+        if (e != cudaSuccess) return record_cuda(e);
+        const long long fgrid = (long long)sms * (per_sm > 0 ? per_sm : 1);
+        kernel<<<(int)(a.n < fgrid ? a.n : fgrid), kFThreads, f.L.total, s>>>(f);
+        return record_cuda(cudaGetLastError());
+    }
     const size_t smem = (size_t)a.T * a.n_bins * 4;
     const auto kernel = a.E > kShortRows ? anywidth_kernel<NSC_MAX_ELEVATION> : anywidth_kernel<kShortRows>;
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -326,6 +711,34 @@ size_t nsc_anywidth_workspace_bytes(int n, int rows, const nsc_params* p) {
     if (n < 0 || validate_any(p) != NSC_OK || rows < 1 || rows > max_rows(p)) return 0;
     const int grid = n < kMaxGrid ? (n < 1 ? 1 : n) : kMaxGrid;
     return table_bytes(p) + Scratch::bytes(rows, p->n_azimuth, p->target_rows, p->n_azimuth / 2 + 1) * (size_t)grid;
+}
+
+int nsc_test_anywidth_path(const nsc_params* p, int rows, int want_descriptor) {
+    const int st = validate_any(p);
+    if (st != NSC_OK) return st;
+    if (rows < 1 || rows > max_rows(p)) return NSC_ERR_BAD_PARAMS;
+    FusedLayout L;
+    FftPlan plan;
+    return choose_fused(p, rows, want_descriptor != 0, &L, &plan) ? 1 : 0;
+}
+
+int nsc_test_anywidth_fft(int W, const float* h_in, float* h_out) {
+    FftPlan plan;
+    if (W < 2 || W > kMaxWidth || !plan_fft(W, &plan)) return NSC_ERR_BAD_PARAMS;
+    if (!h_in || !h_out) return NSC_ERR_NULL_POINTER;
+    std::vector<float2> tw(W), x(W), y(W);
+    for (int m = 0; m < W; ++m) tw[m] = any_twiddle(m, W);
+    for (int i = 0; i < W; ++i) x[i] = make_float2(h_in[2 * i], h_in[2 * i + 1]);
+    for (int p = 0, ns = 1; p < plan.n_pass; ++p) {
+        fft_pass(plan.radix[p], x.data(), y.data(), tw.data(), W, ns, 1, 0, 1);
+        x.swap(y);
+        ns *= plan.radix[p];
+    }
+    for (int i = 0; i < W; ++i) {
+        h_out[2 * i] = x[i].x;
+        h_out[2 * i + 1] = x[i].y;
+    }
+    return NSC_OK;
 }
 
 int nsc_anywidth_points(const float* d_points, int point_stride, const int64_t* d_offsets, int64_t point_origin,

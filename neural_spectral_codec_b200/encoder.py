@@ -166,7 +166,9 @@ def _anywidth_workspace(dev: torch.device, stream: int, p: "_lib.NscParams", n: 
 
 
 def _anywidth_points(points, offsets, n_scans, stride, p, lut, out, images, stage):
-    """Widths other than 360: the general kernel (``nsc_anywidth_points``)."""
+    """Widths other than 360 (``nsc_anywidth_points``): the fused shared-memory kernel for
+    descriptors at widths whose prime factors are at most 13 and images that fit one block's
+    shared memory, the general kernel otherwise (and for images alone)."""
     dev = points.device
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
@@ -319,8 +321,8 @@ class SpectralEncoder(nn.Module):
         ``dtype=torch.uint16`` returns the rows in the wire format instead: the integers
         ``HistogramQuantizer(output_dim).quantize`` gives for the float32 rows (epsilon 1e-8, each
         row summing to 65535), quantised in the same kernel launch. ``out``, if given, has ``dtype``.
-        Image widths other than 360 have no fused kernel: there the general kernel writes float32
-        rows and ``nsc_quantize_histograms`` quantises them -- the same integers, two launches.
+        Image widths other than 360 have no uint16 epilogue: there ``nsc_anywidth_points`` writes
+        float32 rows and ``nsc_quantize_histograms`` quantises them -- the same integers, two launches.
         """
         lib = _lib.load()
         if dtype not in (torch.float32, torch.uint16):
@@ -434,7 +436,7 @@ class SpectralEncoder(nn.Module):
             raise ValueError(f"out must be contiguous {dtype.name} (B, output_dim)")
         if n_scans == 0:
             return out
-        if self.n_azimuth != _lib.N_AZIMUTH:     # other widths: the general kernel, one device batch
+        if self.n_azimuth != _lib.N_AZIMUTH:     # other widths: nsc_anywidth_points, one device batch
             host = pts if arrs is None else (np.concatenate(arrs) if len(arrs) else np.zeros((0, 4), np.float32))
             d = self.encode_points_batch(torch.from_numpy(np.ascontiguousarray(host)).to(dev), torch.from_numpy(offs),
                                          dtype=torch.uint16 if u16 else torch.float32)
@@ -542,7 +544,7 @@ def interpolate_range_image(range_image: Union[np.ndarray, torch.Tensor], method
         x = x.to(device)
     x = x.to(torch.float32).contiguous()
     out = torch.empty_like(x)
-    if x.shape[2] != _lib.N_AZIMUTH:             # other widths: the general kernel
+    if x.shape[2] != _lib.N_AZIMUTH:             # other widths: the general kernel (images only)
         p = _lib.NscParams()
         lib.nsc_default_params(C.byref(p))
         p.n_azimuth, p.n_elevation, p.target_rows, p.n_bins = int(x.shape[2]), int(x.shape[1]), 1, 1
