@@ -220,6 +220,12 @@ int nsc_interpolate_range_images(const float* d_images_in, int n_images, int row
  *   nsc_anywidth_points  encode_points / project [+ interpolate_range_image] for n_scans scans:
  *       d_out (descriptors, float32[n_scans * target_rows * n_bins]) and / or d_images
  *       (float32[n_scans * n_elevation * n_azimuth], the image named by `stage`); either may be NULL
+ *   nsc_anywidth_points_u16  nsc_anywidth_points straight to the wire format of nsc_encode_batch_u16:
+ *       d_out uint16[n_scans * target_rows * n_bins], each row the integers nsc_quantize_histograms
+ *       (q_epsilon) gives for the float32 row nsc_anywidth_points writes for the same call (empty and
+ *       fully filtered scans included), quantised in the same kernel's epilogue. No images. The call
+ *       runs the kernel the float32 call runs, with the same workspace; arguments are validated in
+ *       nsc_anywidth_points' order, with the same status codes
  *   nsc_anywidth_images  forward / encode_range_image (interp_method = -1: no interpolation, as the
  *       reference's forward) and interpolate_range_image (d_out NULL, d_images_out set,
  *       interp_method NSC_INTERP_LINEAR | NSC_INTERP_NEAREST) on images already on the device */
@@ -227,11 +233,22 @@ size_t nsc_anywidth_workspace_bytes(int n, int rows, const nsc_params* p);
 int nsc_anywidth_points(const float* d_points, int point_stride, const int64_t* d_offsets, int64_t point_origin,
                         int n_scans, const nsc_params* p, const int32_t* h_lut, float* d_out, float* d_images,
                         int stage, void* d_workspace, size_t workspace_bytes, void* stream);
+int nsc_anywidth_points_u16(const float* d_points, int point_stride, const int64_t* d_offsets, int64_t point_origin,
+                            int n_scans, const nsc_params* p, const int32_t* h_lut, float q_epsilon, uint16_t* d_out,
+                            void* d_workspace, size_t workspace_bytes, void* stream);
 int nsc_anywidth_images(const float* d_images_in, int n_images, int rows, const nsc_params* p, const int32_t* h_lut,
                         int interp_method, float* d_out, float* d_images_out, void* d_workspace,
                         size_t workspace_bytes, void* stream);
 
 /* ---- host-buffer pipeline (the end-to-end call: H2D, encode, D2H inside) -------------- */
+/* Every encode entry point of the pipeline accepts every image width the entry points above
+ * accept: n_azimuth = 360 runs the kernels of nsc_encode_batch / nsc_encode_batch_u16 and is
+ * validated as they validate; any other n_azimuth (2..4096) runs those of nsc_anywidth_points /
+ * nsc_anywidth_points_u16 and is validated by their rules (h_lut then has n_azimuth / 2 + 1
+ * entries). The rows are those the device entry points give for the same scans, however the scans
+ * are chunked. At other widths each buffer also keeps the workspace of those kernels (for the
+ * general kernel, per-CTA scratch of up to a few MB times the CTAs of one chunk): it is
+ * allocated by the first call that needs it and grown by a later call that needs more. */
 typedef struct nsc_pipeline nsc_pipeline;
 
 /* Creates a pipeline that stages at most max_chunk_points points per chunk through

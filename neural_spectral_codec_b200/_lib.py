@@ -77,6 +77,7 @@ SYMBOLS = {
     "nsc_interpolate_range_images": (_I, [_VP, _I, _I, _I, _VP, _VP]),
     "nsc_anywidth_workspace_bytes": (_SZ, [_I, _I, _PP]),
     "nsc_anywidth_points": (_I, [_VP, _I, _VP, _I64, _I, _PP, _VP, _VP, _VP, _I, _VP, _SZ, _VP]),
+    "nsc_anywidth_points_u16": (_I, [_VP, _I, _VP, _I64, _I, _PP, _VP, C.c_float, _VP, _VP, _SZ, _VP]),
     "nsc_anywidth_images": (_I, [_VP, _I, _I, _PP, _VP, _I, _VP, _VP, _VP, _SZ, _VP]),
     "nsc_pipeline_create": (_I, [_I64, _I, _I, C.POINTER(_VP)]),
     "nsc_pipeline_destroy": (None, [_VP]),

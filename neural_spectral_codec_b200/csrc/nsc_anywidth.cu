@@ -34,6 +34,7 @@
 #include "nsc_anywidth.cuh"
 #include "nsc_fft.cuh"
 #include "nsc_internal.h"
+#include "nsc_quantize.cuh"
 
 namespace nsc {
 
@@ -71,10 +72,73 @@ struct Scratch {
     }
 };
 
+// The uint16 rows of nsc_anywidth_points_u16 (the kernels' Q instantiations): the quantiser's epsilon
+// and NumPy's pairwise-sum plan for D = T * n_bins, built on the host once per launch.
+struct QuantOut {
+    unsigned short* out;       // n x T x n_bins
+    float eps;
+    SumPlan plan;
+};
+
+// The uint16 epilogue of both kernels: the normalised row -- the float32 values the float path
+// stores -- goes through HistogramQuantizer.quantize as nsc_quantize_histograms would take it from
+// global memory (NumPy-order row sum, one division, half-to-even rounding, the rounding error added
+// to the first largest bin), the arithmetic of quantise_and_store (nsc_tail.cuh) with the CTA's own
+// barriers. hist: the D bin sums, normalised in place and then replaced by the integers; slot:
+// kSumSlots floats for warp 0's pairwise sum; part: 2 x NT / 32 words. Both lie in shared memory
+// that is dead at this point; the caller's next writes to them follow its barrier at the top of the
+// next scan. Every thread has read the float path's partials before the first barrier here.
+// Not inlined: it runs once per scan, and inlined into the general kernel it made that kernel spill.
+template <int NT>
+__device__ __noinline__ void quantise_row(float* hist, int D, bool ok, float denom, float uniform,
+                                             const QuantOut& q, float* slot, unsigned* part, unsigned short* out) {
+    constexpr int kWarps = NT / 32;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    for (int i = tid; i < D; i += NT) hist[i] = ok ? __fdiv_rn(hist[i], denom) : uniform;
+    __syncthreads();
+    if (warp == 0) numpy_sum(hist, q.plan, slot, lane);
+    __syncthreads();
+    const float sum = slot[q.plan.result_slot];
+    const bool norm = sum > q.eps;                                 // quantization.py:144-146
+    const float qden = __fadd_rn(sum, q.eps);
+    const bool hoisted = norm && moderate(qden);                   // __fdiv_rn's bits (RowDivisor)
+    const RowDivisor div(hoisted ? qden : 1.0f);
+    unsigned qsum = 0, best = 0;                                   // best: (q << 16) | (0xffff - index)
+    for (int i = tid; i < D; i += NT) {
+        const float h = hist[i];
+        const int v = quantise_value(norm ? (hoisted ? div(h) : __fdiv_rn(h, qden)) : h);
+        hist[i] = __int_as_float(v);
+        qsum += (unsigned)v;
+        best = max(best, ((unsigned)v << 16) | (0xffffu - (unsigned)i));
+    }
+    qsum = __reduce_add_sync(0xffffffffu, qsum);
+    best = __reduce_max_sync(0xffffffffu, best);
+    if (lane == 0) {
+        part[warp] = qsum;
+        part[kWarps + warp] = best;
+    }
+    __syncthreads();
+    qsum = 0;
+    best = 0;
+    for (int w = 0; w < kWarps; ++w) {
+        qsum += part[w];
+        best = max(best, part[kWarps + w]);
+    }
+    int fix_idx = -1, fix_val = 0;                                 // quantization.py:154-167
+    if ((int)qsum > 0 && qsum != 65535u) {
+        fix_idx = 0xffff - (int)(best & 0xffffu);
+        const int v = (int)(best >> 16) + (65535 - (int)qsum);
+        fix_val = v < 0 ? 0 : (v > 65535 ? 65535 : v);
+    }
+    for (int i = tid; i < D; i += NT) out[i] = (unsigned short)(i == fix_idx ? fix_val : __float_as_int(hist[i]));
+}
+
 // ROWS: the capacity of the per-row arrays (kShortRows, or NSC_MAX_ELEVATION for taller images).
-template <int ROWS>
+// Q: uint16 rows to q.out (and no images) instead of float32 rows to a.out; the dynamic shared
+// memory then holds kSumSlots more floats after the histogram.
+template <int ROWS, bool Q>
 __global__ void __launch_bounds__(kGThreads)
-anywidth_kernel(const __grid_constant__ AnyArgs a) {
+anywidth_kernel(const __grid_constant__ AnyArgs a, const __grid_constant__ QuantOut q) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float* hist = reinterpret_cast<float*>(smem_raw);                  // T x n_bins
     __shared__ int s_nvalid[ROWS], s_src[ROWS];
@@ -161,7 +225,7 @@ anywidth_kernel(const __grid_constant__ AnyArgs a) {
                 const int r = i / W, x = i - r * W;
                 a.images_out[(size_t)item * E * W + i] = S.img[(size_t)s_src[r] * W + x];
             }
-        if (!a.out) continue;
+        if (!Q && !a.out) continue;
         // ---- row pooling (adaptive_avg_pool2d over rows, spectral_encoder.py:171-176)
         for (int i = tid; i < T * W; i += kGThreads) {
             const int t = i / W, x = i - t * W;
@@ -212,8 +276,12 @@ anywidth_kernel(const __grid_constant__ AnyArgs a) {
         const float total = (float)tot;
         const bool ok = total > a.eps;
         const float denom = __fadd_rn(total, a.eps);
-        for (int i = tid; i < D; i += kGThreads)
-            a.out[(size_t)item * D + i] = ok ? __fdiv_rn(hist[i], denom) : a.uniform;
+        if (Q)
+            quantise_row<kGThreads>(hist, D, ok, denom, a.uniform, q, hist + D, reinterpret_cast<unsigned*>(s_red),
+                                    q.out + (size_t)item * D);
+        else
+            for (int i = tid; i < D; i += kGThreads)
+                a.out[(size_t)item * D + i] = ok ? __fdiv_rn(hist[i], denom) : a.uniform;
     }
 }
 
@@ -410,6 +478,7 @@ struct FusedArgs {
     AnyArgs a;
     FusedLayout L;
     FftPlan plan;
+    QuantOut q;                 // the Q instantiation's output
 };
 
 // One scan's points into the key image: kPtsInFlight loads per thread in flight, then the
@@ -474,7 +543,10 @@ __device__ __forceinline__ int valid_right(const unsigned* row, int W, int x) {
     }
 }
 
-template <bool VEC4>
+// Q: uint16 rows to f.q.out instead of float32 rows to a.out. The epilogue's pairwise-sum slots go
+// in fa, dead once the bin sums are in hist: a row of D <= T (W / 2 + 1) elements, T <= 64, needs at
+// most 2 ceil(D / 57) - 1 slots (leaves of more than 57 elements), fewer bytes than fa's W x 8.
+template <bool VEC4, bool Q>
 __global__ void __launch_bounds__(kFThreads, 1)
 anywidth_fused_kernel(const __grid_constant__ FusedArgs f) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -610,8 +682,12 @@ anywidth_fused_kernel(const __grid_constant__ FusedArgs f) {
         const float total = (float)tot;
         const bool ok = total > a.eps;
         const float denom = __fadd_rn(total, a.eps);
-        for (int i = tid; i < D; i += kFThreads)
-            a.out[(size_t)item * D + i] = ok ? __fdiv_rn(hist[i], denom) : a.uniform;
+        if (Q)
+            quantise_row<kFThreads>(hist, D, ok, denom, a.uniform, f.q, reinterpret_cast<float*>(fa),
+                                    reinterpret_cast<unsigned*>(s_red), f.q.out + (size_t)item * D);
+        else
+            for (int i = tid; i < D; i += kFThreads)
+                a.out[(size_t)item * D + i] = ok ? __fdiv_rn(hist[i], denom) : a.uniform;
     }
 }
 
@@ -642,7 +718,25 @@ constexpr int kMaxGrid = 1024;     // bounds the workspace without asking the de
 
 size_t table_bytes(const nsc_params* p) { return (((size_t)p->n_bins + 1) * 4 + 255) & ~(size_t)255; }
 
-int run(AnyArgs& a, const nsc_params* p, int rows, const int32_t* h_lut, void* ws, size_t ws_bytes, cudaStream_t s) {
+// The first frequency of every bin from the host table (n_azimuth / 2 + 1 entries), into start if
+// given: NSC_ERR_BAD_LUT for a table that decreases or leaves [0, n_bins).
+int bin_starts(const nsc_params* p, const int32_t* h_lut, int* start) {
+    const int F = p->n_azimuth / 2 + 1;
+    int prev = 0, b = 0;
+    for (int k = 0; k < F; ++k) {
+        if (h_lut[k] < prev || h_lut[k] >= p->n_bins) return NSC_ERR_BAD_LUT;
+        prev = h_lut[k];
+        if (start)
+            while (b <= h_lut[k]) start[b++] = k;
+    }
+    if (start)
+        while (b <= p->n_bins) start[b++] = F;
+    return NSC_OK;
+}
+
+// q: the uint16 rows of nsc_anywidth_points_u16 (a.out null), or null.
+int run(AnyArgs& a, const nsc_params* p, int rows, const int32_t* h_lut, QuantOut* q, void* ws, size_t ws_bytes,
+        cudaStream_t s) {
     a.E = rows;
     a.W = p->n_azimuth;
     a.T = p->target_rows;
@@ -663,26 +757,32 @@ int run(AnyArgs& a, const nsc_params* p, int rows, const int32_t* h_lut, void* w
     a.scratch = (unsigned char*)ws + table_bytes(p);
     a.scratch_per_cta = per;
     a.bin_start = (const int*)ws;
-    if (a.out) {
+    const bool want = a.out || q;
+    if (want) {
         if (!h_lut) return NSC_ERR_NULL_POINTER;
         std::vector<int> start(a.n_bins + 1);
-        int prev = 0, b = 0;
-        for (int k = 0; k < a.F; ++k) {
-            if (h_lut[k] < prev || h_lut[k] >= a.n_bins) return NSC_ERR_BAD_LUT;
-            prev = h_lut[k];
-            while (b <= h_lut[k]) start[b++] = k;
-        }
-        while (b <= a.n_bins) start[b++] = a.F;
+        const int st_lut = bin_starts(p, h_lut, start.data());
+        if (st_lut != NSC_OK) return st_lut;
         // pageable source: the runtime stages it before returning, so the vector may go away
         cudaError_t e = cudaMemcpyAsync(ws, start.data(), start.size() * 4, cudaMemcpyHostToDevice, s);
         if (e != cudaSuccess) return record_cuda(e);
     }
+    QuantOut qo;
+    memset(&qo, 0, sizeof(qo));
+    if (q) {
+        qo = *q;
+        st = build_plan(a.T * a.n_bins, &qo.plan);        // D <= NSC_MAX_DESCRIPTOR: always fits
+        if (st != NSC_OK) return st;
+    }
+    // the same kernel for both output types: the uint16 rows quantise the floats the float call writes
     FusedArgs f;
-    if (choose_fused(p, rows, a.out != nullptr, &f.L, &f.plan)) {
+    if (choose_fused(p, rows, want, &f.L, &f.plan)) {
         // as many CTAs as fit on every SM, each looping over scans / images
         f.a = a;
+        f.q = qo;
         const bool vec4 = a.points && a.stride == 4 && ((uintptr_t)a.points & 15) == 0;
-        const auto kernel = vec4 ? anywidth_fused_kernel<true> : anywidth_fused_kernel<false>;
+        const auto kernel = q ? (vec4 ? anywidth_fused_kernel<true, true> : anywidth_fused_kernel<false, true>)
+                              : (vec4 ? anywidth_fused_kernel<true, false> : anywidth_fused_kernel<false, false>);
         cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)f.L.total);
         int per_sm = 0;
         if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kFThreads, f.L.total);
@@ -691,15 +791,24 @@ int run(AnyArgs& a, const nsc_params* p, int rows, const int32_t* h_lut, void* w
         kernel<<<(int)(a.n < fgrid ? a.n : fgrid), kFThreads, f.L.total, s>>>(f);
         return record_cuda(cudaGetLastError());
     }
-    const size_t smem = (size_t)a.T * a.n_bins * 4;
-    const auto kernel = a.E > kShortRows ? anywidth_kernel<NSC_MAX_ELEVATION> : anywidth_kernel<kShortRows>;
+    const size_t smem = ((size_t)a.T * a.n_bins + (q ? kSumSlots : 0)) * 4;
+    const auto kernel = q ? (a.E > kShortRows ? anywidth_kernel<NSC_MAX_ELEVATION, true> : anywidth_kernel<kShortRows, true>)
+                          : (a.E > kShortRows ? anywidth_kernel<NSC_MAX_ELEVATION, false>
+                                              : anywidth_kernel<kShortRows, false>);
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return record_cuda(e);
-    kernel<<<grid, kGThreads, smem, s>>>(a);
+    kernel<<<grid, kGThreads, smem, s>>>(a, qo);
     return record_cuda(cudaGetLastError());
 }
 
 }  // namespace
+
+int check_anywidth(const nsc_params* p, const int32_t* h_lut) {
+    const int st = validate_any(p);
+    if (st != NSC_OK) return st;
+    if (!h_lut) return NSC_ERR_NULL_POINTER;
+    return bin_starts(p, h_lut, nullptr);
+}
 
 }  // namespace nsc
 
@@ -763,7 +872,31 @@ int nsc_anywidth_points(const float* d_points, int point_stride, const int64_t* 
     a.out = d_out;
     a.images_out = d_images;
     a.stage = stage;
-    return run(a, p, p->n_elevation, h_lut, d_workspace, workspace_bytes, (cudaStream_t)stream);
+    return run(a, p, p->n_elevation, h_lut, nullptr, d_workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int nsc_anywidth_points_u16(const float* d_points, int point_stride, const int64_t* d_offsets, int64_t point_origin,
+                            int n_scans, const nsc_params* p, const int32_t* h_lut, float q_epsilon, uint16_t* d_out,
+                            void* d_workspace, size_t workspace_bytes, void* stream) {
+    int st = validate_any(p);
+    if (st != NSC_OK) return st;
+    if (n_scans < 0) return NSC_ERR_BAD_COUNT;
+    if (point_stride != 3 && point_stride != 4) return NSC_ERR_BAD_STRIDE;
+    if (n_scans == 0) return NSC_OK;
+    if (!d_offsets || !d_out) return NSC_ERR_NULL_POINTER;
+    AnyArgs a;
+    memset(&a, 0, sizeof(a));
+    a.points = d_points;
+    a.stride = point_stride;
+    a.offsets = (const long long*)d_offsets;
+    a.origin = point_origin;
+    a.n = n_scans;
+    a.interpolate = p->interpolate_empty != 0 ? 1 : 0;
+    a.stage = NSC_STAGE_INTERPOLATED;
+    QuantOut q;
+    q.out = d_out;
+    q.eps = q_epsilon;
+    return run(a, p, p->n_elevation, h_lut, &q, d_workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int nsc_anywidth_images(const float* d_images_in, int n_images, int rows, const nsc_params* p, const int32_t* h_lut,
@@ -785,7 +918,7 @@ int nsc_anywidth_images(const float* d_images_in, int n_images, int rows, const 
     a.out = d_out;
     a.images_out = d_images_out;
     a.stage = NSC_STAGE_INTERPOLATED;
-    return run(a, p, rows, h_lut, d_workspace, workspace_bytes, (cudaStream_t)stream);
+    return run(a, p, rows, h_lut, nullptr, d_workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

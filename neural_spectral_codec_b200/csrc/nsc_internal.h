@@ -85,4 +85,7 @@ int launch_interpolate(const float* d_in, int n_images, int rows, int nearest, f
 size_t workspace_bytes_for(int n_scans, int E);   // recommended: room to split the last wave's scans
 size_t workspace_bytes_min();                      // enough for every launch (no splitting)
 
+// The parameter and freq->bin table checks of nsc_anywidth_points, in its order (nsc_anywidth.cu)
+int check_anywidth(const nsc_params* p, const int32_t* h_lut);
+
 }  // namespace nsc

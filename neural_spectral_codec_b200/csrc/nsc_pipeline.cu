@@ -1,6 +1,7 @@
 // Host-buffer pipeline of libnsc_b200.so (nsc_pipeline_*, declared in include/nsc_b200.h): scans in
 // host memory go to the device in chunks through per-slot buffers and streams, are encoded there,
-// and their rows come back, the copies of one chunk overlapping the kernel of another.
+// and their rows come back, the copies of one chunk overlapping the kernel of another. Width 360
+// runs the kernels of nsc_encode.cu, every other width those of nsc_anywidth.cu.
 #include <string.h>
 
 #include <atomic>
@@ -114,6 +115,7 @@ static const int kMaxDescriptor = NSC_MAX_DESCRIPTOR;
 struct nsc_pipeline {
     int device;
     int n_buffers;
+    int sms;
     int64_t max_chunk_points;
     // A slot's buffers may be reused only when it is not busy. busy: `done` was recorded after the
     // last enqueued work that reads or writes these buffers, on whichever stream that work went
@@ -125,6 +127,8 @@ struct nsc_pipeline {
         long long* d_offsets;
         float* d_out;
         unsigned* d_ws;
+        void* d_any_ws;        // workspace of the other widths' kernels, lazy, grown on demand
+        size_t any_ws_bytes;
         float* h_stage;        // pinned staging of one chunk (list path, single scans), lazy
         long long* h_offsets;  // pinned chunk offsets, lazy
         float* h_out;          // pinned chunk descriptors (list path), lazy
@@ -164,12 +168,55 @@ static cudaError_t ensure_pinned(const nsc_pipeline* pl, Slot& s, bool need_out)
     return e;
 }
 
+// What a call encodes with: at 360 columns the kernels of nsc_encode.cu with `dp`, at any other
+// width those of nsc_anywidth.cu with p and h_lut.
+struct Encoder {
+    const nsc_params* p;
+    const int32_t* h_lut;
+    bool any_width;
+    DeviceParams dp;
+};
+
+// The parameter and table checks of the entry point each width's kernels have: nsc_encode_batch's
+// at 360 columns (and for a null or foreign parameter block), nsc_anywidth_points' at the others.
+static int prepare(const nsc_params* p, const int32_t* h_lut, Encoder* enc) {
+    enc->p = p;
+    enc->h_lut = h_lut;
+    enc->any_width = p && p->struct_size == (int32_t)sizeof(nsc_params) && p->n_azimuth != NSC_N_AZIMUTH;
+    return enc->any_width ? check_anywidth(p, h_lut) : make_device_params(p, h_lut, &enc->dp);
+}
+
+// The one encode launch of every entry point: scans `in` of the slot's buffers, rows to out.rows or
+// out.rows_q, on `stream`. The other widths' workspace (the bin table and the general kernel's
+// per-CTA scratch for the grid of this launch) is allocated on first use and grown when a later call
+// needs more; the caller has waited for the slot, so nothing in flight still uses it.
+static int encode(const nsc_pipeline* pl, Slot& s, const Encoder& enc, const PointBatch& in,
+                  const EncodeOutputs& out, cudaStream_t stream) {
+    if (!enc.any_width) return launch_encode(in, enc.dp, out, s.d_ws, 256, stream);
+    const int grid = in.n_scans < 2 * pl->sms ? in.n_scans : 2 * pl->sms;
+    const size_t need = nsc_anywidth_workspace_bytes(grid, enc.p->n_elevation, enc.p);
+    if (s.any_ws_bytes < need) {
+        if (s.d_any_ws) cudaFree(s.d_any_ws);
+        s.d_any_ws = nullptr;
+        s.any_ws_bytes = 0;
+        const cudaError_t e = cudaMalloc(&s.d_any_ws, need);
+        if (e != cudaSuccess) return record_cuda(e);
+        s.any_ws_bytes = need;
+    }
+    const int64_t* offsets = (const int64_t*)in.offsets;
+    if (out.rows_q)
+        return nsc_anywidth_points_u16(in.points, in.stride, offsets, in.origin, in.n_scans, enc.p, enc.h_lut,
+                                       out.q_eps, out.rows_q, s.d_any_ws, s.any_ws_bytes, stream);
+    return nsc_anywidth_points(in.points, in.stride, offsets, in.origin, in.n_scans, enc.p, enc.h_lut, out.rows,
+                               nullptr, NSC_STAGE_INTERPOLATED, s.d_any_ws, s.any_ws_bytes, stream);
+}
+
 // The checks both batch entry points make first, in this order. NSC_OK with n_scans == 0 means
 // there is nothing to do.
 static int check_batch(const nsc_pipeline* pl, const nsc_params* p, const int32_t* h_lut, int n_scans,
-                       int stride, const void* h_points, const void* h_index, const void* h_out, DeviceParams* dp) {
+                       int stride, const void* h_points, const void* h_index, const void* h_out, Encoder* enc) {
     if (!pl) return NSC_ERR_NULL_POINTER;
-    const int st = make_device_params(p, h_lut, dp);
+    const int st = prepare(p, h_lut, enc);
     if (st != NSC_OK) return st;
     if (n_scans < 0) return NSC_ERR_BAD_COUNT;
     if (stride != 3 && stride != 4) return NSC_ERR_BAD_STRIDE;
@@ -182,9 +229,9 @@ static int check_batch(const nsc_pipeline* pl, const nsc_params* p, const int32_
 // `origin`) on slot.stream, and their rows come back on that stream straight into h_out or, with
 // `bounce`, through the slot's pinned h_out. Returns when every slot is free and h_out complete.
 template <class ChunkEnd, class Put>
-static int run_chunks(nsc_pipeline* pl, int n_scans, int stride, const DeviceParams& dp, void* h_out,
+static int run_chunks(nsc_pipeline* pl, int n_scans, int stride, const Encoder& enc, void* h_out,
                       size_t out_bytes, float q_eps, bool bounce, ChunkEnd chunk_end, Put put) {
-    const size_t row_bytes = (size_t)dp.T * dp.n_bins * out_bytes;
+    const size_t row_bytes = (size_t)enc.p->target_rows * enc.p->n_bins * out_bytes;
     EncodeOutputs out;
     out.q_eps = q_eps;
     // bounced rows of THIS call still in a slot's h_out; a slot that another call left busy has none
@@ -208,7 +255,7 @@ static int run_chunks(nsc_pipeline* pl, int n_scans, int stride, const DevicePar
         if (out_bytes == 4) out.rows = s.d_out;
         else out.rows_q = reinterpret_cast<unsigned short*>(s.d_out);
         if (st == NSC_OK)
-            st = launch_encode({s.d_points, stride, s.d_offsets, origin, ns}, dp, out, s.d_ws, 256, s.stream);
+            st = encode(pl, s, enc, {s.d_points, stride, s.d_offsets, origin, ns}, out, s.stream);
         if (st == NSC_OK)
             st = record_cuda(cudaMemcpyAsync(bounce ? (void*)s.h_out : (char*)h_out + first * row_bytes, s.d_out,
                                              ns * row_bytes, cudaMemcpyDeviceToHost, s.stream));
@@ -229,8 +276,8 @@ static int run_chunks(nsc_pipeline* pl, int n_scans, int stride, const DevicePar
 static int pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_stride, int64_t n_points,
                            const int64_t* h_offsets, int n_scans, const nsc_params* p, const int32_t* h_lut,
                            void* h_out, size_t out_bytes, float q_eps) {
-    DeviceParams dp;
-    const int st = check_batch(pl, p, h_lut, n_scans, point_stride, h_points, h_offsets, h_out, &dp);
+    Encoder enc;
+    const int st = check_batch(pl, p, h_lut, n_scans, point_stride, h_points, h_offsets, h_out, &enc);
     if (st != NSC_OK || n_scans == 0) return st;
     if (n_points < 0) return NSC_ERR_BAD_COUNT;
     if (h_offsets[0] < 0 || h_offsets[n_scans] > n_points) return NSC_ERR_BAD_OFFSETS;
@@ -258,7 +305,7 @@ static int pipeline_encode(nsc_pipeline* pl, const float* h_points, int point_st
                                 cudaMemcpyHostToDevice, s.stream);
         return e;
     };
-    return run_chunks(pl, n_scans, point_stride, dp, h_out, out_bytes, q_eps, false, chunk_end, put);
+    return run_chunks(pl, n_scans, point_stride, enc, h_out, out_bytes, q_eps, false, chunk_end, put);
 }
 
 // Copies scans [first, last) into the pinned staging buffer with a few host threads (a single
@@ -296,8 +343,8 @@ static void stage_scans(float* dst, const float* const* h_scans, const int64_t* 
 static int pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, const int64_t* h_counts,
                                  int point_stride, int n_scans, const nsc_params* p, const int32_t* h_lut,
                                  void* h_out, size_t out_bytes, float q_eps) {
-    DeviceParams dp;
-    const int st = check_batch(pl, p, h_lut, n_scans, point_stride, h_scans, h_counts, h_out, &dp);
+    Encoder enc;
+    const int st = check_batch(pl, p, h_lut, n_scans, point_stride, h_scans, h_counts, h_out, &enc);
     if (st != NSC_OK || n_scans == 0) return st;
     for (int i = 0; i < n_scans; ++i) {
         if (h_counts[i] < 0) return NSC_ERR_BAD_OFFSETS;
@@ -327,7 +374,7 @@ static int pipeline_encode_scans(nsc_pipeline* pl, const float* const* h_scans, 
                                 s.stream);
         return e;
     };
-    return run_chunks(pl, n_scans, point_stride, dp, h_out, out_bytes, q_eps, true, chunk_end, put);
+    return run_chunks(pl, n_scans, point_stride, enc, h_out, out_bytes, q_eps, true, chunk_end, put);
 }
 
 extern "C" {
@@ -342,6 +389,7 @@ void nsc_pipeline_destroy(nsc_pipeline* pl) {
         if (s.d_offsets) cudaFree(s.d_offsets);
         if (s.d_out) cudaFree(s.d_out);
         if (s.d_ws) cudaFree(s.d_ws);
+        if (s.d_any_ws) cudaFree(s.d_any_ws);
         if (s.h_stage) cudaFreeHost(s.h_stage);
         if (s.h_offsets) cudaFreeHost(s.h_offsets);
         if (s.h_out) cudaFreeHost(s.h_out);
@@ -363,6 +411,11 @@ int nsc_pipeline_create(int64_t max_chunk_points, int n_buffers, int device, nsc
     pl->device = device;
     pl->n_buffers = n_buffers;
     pl->max_chunk_points = max_chunk_points;
+    const cudaError_t e_sms = cudaDeviceGetAttribute(&pl->sms, cudaDevAttrMultiProcessorCount, device);
+    if (e_sms != cudaSuccess) {
+        nsc_pipeline_destroy(pl);
+        return record_cuda(e_sms);
+    }
     for (int i = 0; i < n_buffers; ++i) {
         Slot& s = pl->slot[i];
         cudaError_t e;
@@ -413,8 +466,8 @@ int nsc_pipeline_encode_scans_u16(nsc_pipeline* pl, const float* const* h_scans,
 int nsc_pipeline_encode_scan(nsc_pipeline* pl, const float* h_points, int point_stride, int64_t n_points,
                              const nsc_params* p, const int32_t* h_lut, float* d_out, void* stream) {
     if (!pl) return NSC_ERR_NULL_POINTER;
-    DeviceParams dp;
-    int st = make_device_params(p, h_lut, &dp);
+    Encoder enc;
+    int st = prepare(p, h_lut, &enc);
     if (st != NSC_OK) return st;
     if (point_stride != 3 && point_stride != 4) return NSC_ERR_BAD_STRIDE;
     if (n_points < 0) return NSC_ERR_BAD_COUNT;
@@ -441,7 +494,7 @@ int nsc_pipeline_encode_scan(nsc_pipeline* pl, const float* h_points, int point_
     if (st == NSC_OK) {
         EncodeOutputs out;
         out.rows = d_out;
-        st = launch_encode({s.d_points, point_stride, s.d_offsets, 0, 1}, dp, out, s.d_ws, 256, cs);
+        st = encode(pl, s, enc, {s.d_points, point_stride, s.d_offsets, 0, 1}, out, cs);
     }
     e = mark(s, cs);
     return st != NSC_OK ? st : record_cuda(e);

@@ -152,11 +152,17 @@ def _workspace(dev: torch.device, stream: int, p: "_lib.NscParams", n_scans: int
     return ws
 
 
-def _anywidth_workspace(dev: torch.device, stream: int, p: "_lib.NscParams", n: int, rows: int) -> torch.Tensor:
+def _anywidth_need(p: "_lib.NscParams", n: int, rows: int) -> int:
+    """Workspace bytes of the kernels for widths other than 360; ValueError outside their envelope."""
     need = int(_lib.load().nsc_anywidth_workspace_bytes(n, rows, C.byref(p)))
     if need == 0:
         raise ValueError("encoder geometry outside the supported envelope (rows <= 128, 2 <= n_azimuth <= 4096, "
                          "n_bins <= n_azimuth // 2 + 1)")
+    return need
+
+
+def _anywidth_workspace(dev: torch.device, stream: int, p: "_lib.NscParams", n: int, rows: int) -> torch.Tensor:
+    need = _anywidth_need(p, n, rows)
     key = (dev.index if dev.index is not None else torch.cuda.current_device(), stream, "anywidth")
     ws = _WORKSPACES.get(key)
     if ws is None or ws.numel() * 4 < need:
@@ -168,16 +174,23 @@ def _anywidth_workspace(dev: torch.device, stream: int, p: "_lib.NscParams", n: 
 def _anywidth_points(points, offsets, n_scans, stride, p, lut, out, images, stage):
     """Widths other than 360 (``nsc_anywidth_points``): the fused shared-memory kernel for
     descriptors at widths whose prime factors are at most 13 and images that fit one block's
-    shared memory, the general kernel otherwise (and for images alone)."""
+    shared memory, the general kernel otherwise (and for images alone). A uint16 ``out`` takes
+    ``nsc_anywidth_points_u16`` (same kernel, quantised in its epilogue; no images)."""
     dev = points.device
+    u16 = out is not None and out.dtype == torch.uint16
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
         ws = _anywidth_workspace(dev, stream, p, n_scans, p.n_elevation)
-        st = _lib.load().nsc_anywidth_points(
-            points.data_ptr(), stride, offsets.data_ptr(), 0, n_scans, C.byref(p),
-            lut.ctypes.data if lut is not None else None, out.data_ptr() if out is not None else None,
-            images.data_ptr() if images is not None else None, stage, ws.data_ptr(), ws.numel() * 4, stream)
-    _lib.check(st, "nsc_anywidth_points")
+        if u16:
+            st = _lib.load().nsc_anywidth_points_u16(
+                points.data_ptr(), stride, offsets.data_ptr(), 0, n_scans, C.byref(p), lut.ctypes.data,
+                _lib.QUANT_EPSILON, out.data_ptr(), ws.data_ptr(), ws.numel() * 4, stream)
+        else:
+            st = _lib.load().nsc_anywidth_points(
+                points.data_ptr(), stride, offsets.data_ptr(), 0, n_scans, C.byref(p),
+                lut.ctypes.data if lut is not None else None, out.data_ptr() if out is not None else None,
+                images.data_ptr() if images is not None else None, stage, ws.data_ptr(), ws.numel() * 4, stream)
+    _lib.check(st, "nsc_anywidth_points_u16" if u16 else "nsc_anywidth_points")
 
 
 def _anywidth_images(x, p, lut, method, out, images_out):
@@ -190,15 +203,6 @@ def _anywidth_images(x, p, lut, method, out, images_out):
             out.data_ptr() if out is not None else None, images_out.data_ptr() if images_out is not None else None,
             ws.data_ptr(), ws.numel() * 4, stream)
     _lib.check(st, "nsc_anywidth_images")
-
-
-def _quantize_rows(rows: torch.Tensor, out: torch.Tensor) -> None:
-    """float32 descriptor rows -> ``out`` in the wire format (``nsc_quantize_histograms``, the
-    reference quantiser's default epsilon): the second launch of widths without a fused kernel."""
-    with torch.cuda.device(rows.device):
-        st = _lib.load().nsc_quantize_histograms(rows.data_ptr(), rows.shape[0], rows.shape[1], _lib.QUANT_EPSILON,
-                                                 out.data_ptr(), torch.cuda.current_stream(rows.device).cuda_stream)
-    _lib.check(st, "nsc_quantize_histograms")
 
 
 def _check_batch(points: torch.Tensor, offsets: torch.Tensor):
@@ -320,9 +324,8 @@ class SpectralEncoder(nn.Module):
 
         ``dtype=torch.uint16`` returns the rows in the wire format instead: the integers
         ``HistogramQuantizer(output_dim).quantize`` gives for the float32 rows (epsilon 1e-8, each
-        row summing to 65535), quantised in the same kernel launch. ``out``, if given, has ``dtype``.
-        Image widths other than 360 have no uint16 epilogue: there ``nsc_anywidth_points`` writes
-        float32 rows and ``nsc_quantize_histograms`` quantises them -- the same integers, two launches.
+        row summing to 65535), quantised in the same kernel launch at every image width. ``out``, if
+        given, has ``dtype``.
         """
         lib = _lib.load()
         if dtype not in (torch.float32, torch.uint16):
@@ -337,10 +340,7 @@ class SpectralEncoder(nn.Module):
         p = self._params()
         lut = self.freq_to_bin()
         if self.n_azimuth != _lib.N_AZIMUTH:
-            rows = out if dtype == torch.float32 else torch.empty(out.shape, dtype=torch.float32, device=dev)
-            _anywidth_points(points, offsets, n_scans, stride, p, lut, rows, None, _lib.STAGE_INTERPOLATED)
-            if dtype == torch.uint16 and n_scans:
-                _quantize_rows(rows, out)
+            _anywidth_points(points, offsets, n_scans, stride, p, lut, out, None, _lib.STAGE_INTERPOLATED)
             return out
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
@@ -368,11 +368,8 @@ class SpectralEncoder(nn.Module):
             if pts.shape[1] > 4:
                 pts = pts[:, :3]
             offs = torch.tensor([0, pts.shape[0]], dtype=torch.int64).to(dev)
-        elif self.n_azimuth == _lib.N_AZIMUTH:
-            return self._encode_host_scan(_as_f32_points(points), dev)
-        else:
-            pts, offs = _host_scan_to_device(points, dev)
-        return self.encode_points_batch(pts, offs)[0]
+            return self.encode_points_batch(pts, offs)[0]
+        return self._encode_host_scan(_as_f32_points(points), dev)
 
     def _encode_host_scan(self, a: np.ndarray, dev: torch.device) -> torch.Tensor:
         """One pageable numpy scan -> descriptor on the device through ``nsc_pipeline_encode_scan``
@@ -382,6 +379,8 @@ class SpectralEncoder(nn.Module):
         pl = self._cached_pipeline("scan", (index, cap, 3), lambda k: k[0] == index and k[1] >= cap)
         out = torch.empty((self.output_dim,), dtype=torch.float32, device=dev)
         p = self._params()
+        if self.n_azimuth != _lib.N_AZIMUTH:
+            _anywidth_need(p, 1, p.n_elevation)
         lut = self.freq_to_bin()
         st = _lib.load().nsc_pipeline_encode_scan(pl, a.ctypes.data, a.shape[1], a.shape[0], C.byref(p),
                                                   lut.ctypes.data, out.data_ptr(),
@@ -436,17 +435,13 @@ class SpectralEncoder(nn.Module):
             raise ValueError(f"out must be contiguous {dtype.name} (B, output_dim)")
         if n_scans == 0:
             return out
-        if self.n_azimuth != _lib.N_AZIMUTH:     # other widths: nsc_anywidth_points, one device batch
-            host = pts if arrs is None else (np.concatenate(arrs) if len(arrs) else np.zeros((0, 4), np.float32))
-            d = self.encode_points_batch(torch.from_numpy(np.ascontiguousarray(host)).to(dev), torch.from_numpy(offs),
-                                         dtype=torch.uint16 if u16 else torch.float32)
-            out[...] = d.cpu().numpy()
-            return out
         biggest = int(np.diff(offs).max())
         chunk = max(int(max_chunk_points), biggest)
         key = (dev.index if dev.index is not None else torch.cuda.current_device(), chunk, n_buffers)
         pl = self._cached_pipeline("batch", key, key.__eq__)
         p = self._params()
+        if self.n_azimuth != _lib.N_AZIMUTH:
+            _anywidth_need(p, 1, p.n_elevation)
         lut = self.freq_to_bin()
         if arrs is not None:   # separate host arrays: gathered into pinned staging inside the library
             ptrs = (C.c_void_p * n_scans)(*[a.ctypes.data for a in arrs])
